@@ -4,7 +4,9 @@
 Workload (BASELINE.json configs[1]): synthetic head outputs, batch 64 per GPU @608x608 (grids 76/38/19), 80 classes,
 val setting conf 1e-4 / nms 0.4.  A "step" is one pass of the hot path over one batch.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (N>1 under torchrun, one rank per GPU)
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]
+                                                                  our arm (N>1 under torchrun, one rank per GPU); DIR receives
+                                                                  the detections of the last timed step as .npy files
   python bench.py --impl reference [--gpus N] --steps K ...       CPU arm on the host cores (rank 0 only): the UNMODIFIED
                                                                   reference from baseline/_ref when it is installed, else the
                                                                   oracle's C port of it
@@ -189,12 +191,14 @@ def run_reference(args, rank, world):
             cpu_port(min(n_img, 8), threads)
         t_all = 0.0
         for s in range(args.steps):
-            _, dt, _, _ = cpu_port(n_img, threads, seed=s)
+            _, dt, out, _ = cpu_port(n_img, threads, seed=s)
             t_all += dt
         kind = "port"
         sample = "%d images/step of the same synthetic workload, oracle C port of YOLOLayer x3 + cat + postprocess, OpenMP over " \
                  "images (baseline/_ref is not installed)" % n_img
     value = n_img * args.steps / t_all
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * t_all / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -222,6 +226,30 @@ def rows_equal(got, want):
         if g.shape != w.shape or not np.array_equal(np.ascontiguousarray(g).view(np.uint32), np.ascontiguousarray(w).view(np.uint32)):
             return False
     return True
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, per_image):
+    """Writes what a caller of the timed path receives for one step, the per-image lists of [K_i, 7] rows, as
+    counts.npy (float64 [n_images], rows per image) and detections.npy (float32 [R, 7], the rows of every image in image order).
+    Above 64 MB in all, detections.npy keeps a fixed, seeded sample of the rows and detections_index.npy (float64 [n]) gives
+    their positions in the full [R, 7] array."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = np.array([0 if r is None else r.shape[0] for r in per_image], np.float64)
+    rows = [r.detach().cpu().numpy() if hasattr(r, "detach") else np.asarray(r) for r in per_image if r is not None]
+    rows = np.concatenate(rows, 0).astype(np.float32) if rows else np.zeros((0, 7), np.float32)
+    np.save(os.path.join(out_dir, "counts.npy"), counts)
+    cap = (DUMP_BYTES - counts.nbytes - 3 * 4096) // (rows.itemsize * 7 + 8)     # 4 KB per file for the .npy headers
+    idx_path = os.path.join(out_dir, "detections_index.npy")
+    if rows.shape[0] > cap:
+        idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], cap, replace=False))
+        np.save(idx_path, idx.astype(np.float64))
+        rows = rows[idx]
+    elif os.path.exists(idx_path):
+        os.remove(idx_path)
+    np.save(os.path.join(out_dir, "detections.npy"), rows)
 
 
 def time_events(torch, fn, iters, warm=3):
@@ -324,8 +352,10 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--cpu-sample", type=int, default=64, help="images timed for the CPU baseline (0 = skip)")
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="repeat the CPU sample until this much time is spent")
-    ap.add_argument("--min-seconds", type=float, default=0.25, help="the K-step timed region is repeated until this much device "
-                                                                    "time is covered; the line reports the median round")
+    ap.add_argument("--min-seconds", type=float, default=0.25, help="the warm-up continues until this much device time is covered, "
+                                                                    "so that the K timed steps run at sustained clocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the detections of the last timed step to DIR as .npy "
+                                                                        "files (see dump_outputs)")
     ap.add_argument("--no-extras", action="store_true", help="skip the other configs' numbers")
     ap.add_argument("--inflight", type=int, default=0, help="0 = automatic (3 on one GPU, 2 with the exchange at N>1).  ""steps in flight: each step's chain is a CUDA graph; step i runs on stream "
                                                             "i %% inflight with its own workspace and output rows, so the latency-bound "
@@ -449,45 +479,50 @@ def main():
             return (state["i"] - 1) % NP
         return None
 
-    # clocks are sampled from here through the timed rounds and the per-kernel timing below
-    begin()
-    for _ in range(args.warmup):
-        step()
-    drain()
-    barrier()
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-
-    def timed_round():
-        state["i"] = 0
-        barrier()
-        ev0.record()
+    def warm(n):
         begin()
-        for _ in range(args.steps):
+        for _ in range(n):
             step()
-        last = drain()
-        ev1.record()
+        drain()
         barrier()
-        sec = ev0.elapsed_time(ev1) / 1e3
-        if world > 1:
-            t = torch.tensor([sec], device=dev)
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            sec = float(t.item())
-        return sec, last
 
-    sec0, last_slot = timed_round()
-    # a timed region of K steps is a few milliseconds: repeat it (same K) until min_seconds of device time are covered, so that
-    # the clocks are sampled under sustained load; the line reports the median round
-    n_rounds = int(min(200, max(1, math.ceil(args.min_seconds / max(sec0, 1e-6)))))
+    # clocks are sampled from here through the timed steps and the per-kernel timing below
+    warm(args.warmup)
+    # K timed steps are a few milliseconds: the warm-up goes on until min_seconds of device time are covered, so that they run at
+    # the clocks of sustained load.  The ranks agree on the count (at N>1 every step is matched by the exchange).
+    n_sustain = 0
+    if args.min_seconds > 0:
+        t0 = time.perf_counter()
+        warm(16)
+        per_step = (time.perf_counter() - t0) / 16
+        n_sustain = int(min(20000, math.ceil(args.min_seconds / max(per_step, 1e-7))))
+        if world > 1:
+            t = torch.tensor([n_sustain], device=dev)
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+            n_sustain = int(t.item())
+        warm(n_sustain)
+        n_sustain += 16
+
+    # ---- the timed region: exactly K steps ---------------------------------------------------------------------------------
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    state["i"] = 0
+    barrier()
+    ev0.record()
+    begin()
+    for _ in range(args.steps):
+        step()
+    last_slot = drain()
+    ev1.record()
+    barrier()
+    sec = ev0.elapsed_time(ev1) / 1e3
     if world > 1:
-        t = torch.tensor([n_rounds], device=dev)
+        t = torch.tensor([sec], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        n_rounds = int(t.item())
-    rounds = [sec0]
-    for _ in range(n_rounds - 1):
-        s_, last_slot = timed_round()
-        rounds.append(s_)
-    sec = float(np.median(rounds))
+        sec = float(t.item())
     value = world * B * args.steps / sec
+    if args.dump_outputs and rank == 0:
+        # what the caller of the timed path receives for the last step: this GPU's images, or at N>1 every rank's after the exchange
+        dump_outputs(args.dump_outputs, ex.results(last_slot) if world > 1 else hps[(args.steps - 1) % NP].results())
 
     # ---- one step alone (serial replays of one graph): the latency of a step, next to the pipelined throughput above --------
     for _ in range(3):
@@ -715,10 +750,10 @@ def main():
                                     "; at N>1 every step also pushes its kept rows into every rank's window (the final exchange) on a side "
                                     "stream, and the last exchange is delivered inside the timed region" if world > 1 else ""),
                        "steps_in_flight": NP, "one_step_alone_ms": 1e3 * sec_serial / args.steps,
-                       "timed_rounds": len(rounds), "round_ms_min_median_max": [1e3 * min(rounds), 1e3 * sec, 1e3 * max(rounds)],
+                       "sustained_warmup_steps": n_sustain,
                        "rows_per_step": rows_per_step,
                        "parallelism": "images sharded by rank, no collective inside decode/filter/NMS; final exchange by peer stores"},
-            "gpu_launches": (hp.launches_per_run + (3 if world > 1 else 0)) * args.steps * len(rounds),
+            "gpu_launches": (hp.launches_per_run + (3 if world > 1 else 0)) * args.steps,
             "e2e": e2e,
             "roofline": {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                          "traffic": traffic,

@@ -1,13 +1,16 @@
-"""GPU: the UNMODIFIED reference (zjykzj/YOLOv4, installed into baseline/_ref by tools/install_reference.sh; git-ignored, it
-travels to the GPU box with the snapshot) with and without yolov4_b200.patch_reference(), on the same GPU and the same inputs.
+"""GPU: the B200 path at the drop-in boundary of the reference (zjykzj/YOLOv4), after yolov4_b200.patch_reference().
 
-  eval   yolo.model.yolov4.YOLOv4 (yolov4.py:270-324), random init with non-degenerate BN: decoded [B,M,85] within 1e-5 relative
-         (north_star's tolerance); postprocess (utils.py:92-223) on the SAME decoded tensor: identical lists, bit for bit
-  train  the reference's criterion (yololoss.py:373-443) on the patched model: loss within 1e-5, gradient within 2e-5, both with
+Every test runs in two forms.  The golden form always runs: the patched boundary symbols against outputs of the UNMODIFIED
+reference stored under tests/golden/ by tests/golden/make_golden.py (postprocess.npz: the reference's decoded [2, 1008, 85] tensor
+of seeded 128x128 head outputs and the rows of its postprocess; loss.npz: raw head tensors, labels, the reference's loss and its
+autograd gradient with respect to the raw tensors).  The live form runs where the reference is installed into baseline/_ref
+(tools/install_reference.sh; git-ignored): the reference model with and without the patch, on the same GPU and the same inputs.
+
+  eval   decoded [B,M,85] within 1e-5 relative (north_star's tolerance); postprocess (utils.py:92-223) on the SAME decoded tensor:
+         identical lists, bit for bit (live: yolo.model.yolov4.YOLOv4, yolov4.py:270-324, random init with non-degenerate BN)
+  train  the reference's criterion (yololoss.py:373-443) on the patched layers: loss within 1e-5, gradient within 2e-5, both with
          the reference's own forward on top of the B200 YOLOLayer / build_target (its in-place mask multiplies must not break
          autograd) and with the rebound forward
-
-Nothing here reads /root/reference.  Skipped when baseline/_ref is absent.
 """
 import os
 import sys
@@ -17,11 +20,13 @@ import pytest
 import torch
 from torch import nn
 
+from test_cabi_cpu import _stand_in_reference
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.path.join(ROOT, "baseline", "_ref")
+HAVE_REF = os.path.isdir(os.path.join(REF, "yolo"))
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "yolo")), reason="baseline/_ref (the installed reference) is absent")]
+pytestmark = pytest.mark.gpu
 
 IMG = 128           # grids 16 / 8 / 4: the reference's Python postprocess stays fast
 
@@ -68,7 +73,7 @@ def _calibrate(model, x):
     return model
 
 
-def test_eval_model_and_postprocess_patched_vs_unpatched(ref):
+def _live_eval(ref):
     import yolov4_b200 as yb
     dev = torch.device("cuda")
     m4, cfg = ref["m4"], ref["cfg"]
@@ -110,8 +115,7 @@ def test_eval_model_and_postprocess_patched_vs_unpatched(ref):
     assert n_rows > 50, "the test input must produce detections"
 
 
-@pytest.mark.parametrize("loss_forward", [False, True])
-def test_train_loss_and_gradient_patched_vs_unpatched(ref, loss_forward):
+def _live_train(ref, loss_forward):
     import yolov4_b200 as yb
     from yolov4_b200.synth import synth_labels
     dev = torch.device("cuda")
@@ -151,3 +155,109 @@ def test_train_loss_and_gradient_patched_vs_unpatched(ref, loss_forward):
         scale = float(a.abs().max())
         assert scale > 0
         assert float((a - b).abs().max()) <= 2e-5 * scale, (float((a - b).abs().max()), scale)
+
+
+# ------------------------------------------------------------------------------------------------ golden form
+def _patched_boundary(monkeypatch, loss_forward=True):
+    """patch_reference() over stand-ins of the reference's module layout: the calls below go through the rebound symbols."""
+    import yolov4_b200 as yb
+    _stand_in_reference(monkeypatch)
+    done = yb.patch_reference(loss_forward=loss_forward)
+    assert "yolo.model.yololayer.YOLOLayer" in done and "yolo.util.utils.postprocess" in done
+    return sys.modules["yolo.model.yololayer"], sys.modules["yolo.util.utils"], sys.modules["yolo.model.yololoss"]
+
+
+def _golden_eval(golden_dir, monkeypatch):
+    import yolov4_b200 as yb
+    from yolov4_b200.synth import synth_head_outputs
+    ml, mu, _ = _patched_boundary(monkeypatch)
+    g = np.load(os.path.join(golden_dir, "postprocess.npz"))
+    # the head outputs the reference decoded in make_golden.gen_postprocess (the same seeded generator and arguments)
+    raws = [r.cuda() for r in synth_head_outputs(2, IMG, 80, seed=3, fg_prob=0.04, clustered=True)]
+    cfg = {"ANCHORS": yb.ANCHORS_PX, "ANCHOR_MASK": yb.ANCHOR_MASK, "N_CLASSES": 80}
+    with torch.no_grad():
+        out_b = torch.cat([ml.YOLOLayer(cfg, l, device="cuda").eval()(raws[l]) for l in range(3)], 1)
+    assert out_b.shape == (2, 3 * (16 * 16 + 8 * 8 + 4 * 4), 85)
+    a, b = g["pred"].astype(np.float64), out_b.cpu().numpy().astype(np.float64)
+    assert np.isfinite(a).all() and np.isfinite(b).all()
+    tiny = np.abs(a) < 1e-30            # sigmoid outputs below the fp32 normal range are compared absolutely (test_oracle_golden)
+    assert np.abs(b[tiny]).max(initial=0.0) < 1e-30
+    rel = np.abs(a - b)[~tiny] / np.abs(a[~tiny])
+    assert rel.max() <= 1e-5, rel.max()                                       # north_star: decoded values within 1e-5 relative
+    pred = torch.from_numpy(g["pred"]).cuda()                                 # the reference's own decoded tensor
+    n_rows, i = 0, 0
+    while f"s{i}_conf" in g:
+        got = mu.postprocess(pred, 80, float(g[f"s{i}_conf"]), float(g[f"s{i}_nms"]))
+        counts, rows = g[f"s{i}_counts"], g[f"s{i}_rows"]
+        assert len(got) == len(counts)
+        o = 0
+        for gi, n in zip(got, counts):
+            assert (gi is None) == (n == 0), (i, n)
+            if n:
+                assert gi.shape == (n, 7)
+                assert np.array_equal(gi.cpu().numpy().view(np.uint32), rows[o:o + n].view(np.uint32)), (i, o)
+            o += n
+        n_rows += o
+        i += 1
+    assert i == 5 and n_rows > 50, "the test input must produce detections"
+
+
+def _reference_forward_in_place(crit, outputs, labels):
+    """The reference's YOLOLoss.forward (yololoss.py:373-443) in its own form, on top of the criterion's build_target: the mask
+    products are taken in place on the layer's output (yololoss.py:402-408), then the four sums.  Written out here because the
+    golden form runs without the reference's code; loss.npz holds the reference's value and gradient it must reproduce."""
+    bce, l2 = nn.BCELoss(reduction="sum"), nn.MSELoss(reduction="sum")
+    total = 0
+    for od in outputs:
+        output = od["output"]
+        target, obj_mask, tgt_mask, tgt_scale = crit.build_target(output, od["pred"], int(od["layer_no"]), labels)
+        sel = np.r_[0:4, 5:output.shape[-1]]
+        output[..., 4] *= obj_mask
+        output[..., sel] *= tgt_mask
+        output[..., 2:4] *= tgt_scale
+        target[..., 4] *= obj_mask
+        target[..., sel] *= tgt_mask
+        target[..., 2:4] *= tgt_scale
+        bce_w = nn.BCELoss(weight=tgt_scale * tgt_scale, reduction="sum")
+        total = total + bce_w(output[..., :2], target[..., :2]) + l2(output[..., 2:4], target[..., 2:4]) / 2 + \
+            bce(output[..., 4], target[..., 4]) + bce(output[..., 5:], target[..., 5:])
+    return total
+
+
+def _golden_train(golden_dir, monkeypatch, loss_forward):
+    import yolov4_b200 as yb
+    ml, _, mlo = _patched_boundary(monkeypatch, loss_forward=loss_forward)
+    assert mlo.YOLOLoss.build_target is yb.YOLOLoss.build_target
+    assert (mlo.YOLOLoss.forward is yb.YOLOLoss.forward) == loss_forward
+    g = np.load(os.path.join(golden_dir, "loss.npz"))
+    cfg = {"ANCHORS": yb.ANCHORS_PX, "ANCHOR_MASK": yb.ANCHOR_MASK, "N_CLASSES": int(g["C"])}
+    leaves = [torch.from_numpy(g[f"raw{l}"]).cuda().requires_grad_(True) for l in range(3)]
+    labels = torch.from_numpy(g["labels"]).double()                            # as the loader collates them
+    # in the model the layers see a conv output, not a leaf (make_golden.gen_loss does the same)
+    outs = [ml.YOLOLayer(cfg, l, device="cuda").train()(leaves[l] * 1.0) for l in range(3)]
+    crit = yb.YOLOLoss(cfg, ignore_thresh=0.7, device="cuda")
+    loss = crit(outs, {"padded_labels": labels}) if loss_forward else _reference_forward_in_place(crit, outs, labels)
+    loss.backward()
+    want = float(g["loss"])
+    assert abs(loss.item() - want) <= 1e-5 * abs(want), (loss.item(), want)
+    for l in range(3):
+        a, b = torch.from_numpy(g[f"grad{l}"]).double(), leaves[l].grad.cpu().double()
+        scale = float(a.abs().max())
+        assert scale > 0
+        assert float((a - b).abs().max()) <= 2e-5 * scale, (l, float((a - b).abs().max()), scale)
+
+
+# ------------------------------------------------------------------------------------------------ tests
+def test_eval_model_and_postprocess_patched_vs_unpatched(golden_dir, monkeypatch, request):
+    _golden_eval(golden_dir, monkeypatch)
+    if HAVE_REF:
+        monkeypatch.undo()
+        _live_eval(request.getfixturevalue("ref"))
+
+
+@pytest.mark.parametrize("loss_forward", [False, True])
+def test_train_loss_and_gradient_patched_vs_unpatched(golden_dir, monkeypatch, request, loss_forward):
+    _golden_train(golden_dir, monkeypatch, loss_forward)
+    if HAVE_REF:
+        monkeypatch.undo()
+        _live_train(request.getfixturevalue("ref"), loss_forward)
