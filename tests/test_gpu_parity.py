@@ -190,7 +190,7 @@ def test_postprocess_dense_vs_oracle_608(seed, clustered, conf, nmst):
 
 
 def test_fused_vs_oracle_detect_416_and_odd_shapes():
-    for img, C, B in ((416, 80, 3), (96, 4, 5), (64, 20, 1)):
+    for img, C, B in ((416, 80, 3), (96, 4, 5), (64, 20, 1), (96, 20, 4)):
         raws = synth_head_outputs(B, img, C, seed=img, device="cuda", fg_prob=0.05, clustered=True)
         want = orc.detect([r.cpu().numpy() for r in raws], C, 0.01, 0.45, nthreads=8)
         got = yb.detect_raw(raws, C, 0.01, 0.45)
@@ -630,10 +630,10 @@ def test_fullsize_608_build_target_vs_reference_golden(golden_dir, layer):
 
 
 # ------------------------------------------------------------------------------------------------ non-default forms (read at load)
-@pytest.mark.parametrize("env", [{"YL_FLAG": "ldg"}, {"YL_FILTER": "fused"}, {"YL_DENSE": "groups"}, {"YL_PDL": "0"}])
+@pytest.mark.parametrize("env", [{"YL_FLAG": "ldg"}, {"YL_PDL": "0"}])
 def test_alternative_kernel_forms_bit_exact_in_a_fresh_process(env):
-    """The front-end forms selected by environment switches when the library loads (k_flag_raw, the fused TMA kernel, the round-1
-    dense kernel, no programmatic dependent launch) produce the oracle's bits too.  A fresh process per form."""
+    """The forms selected by environment switches when the library loads (k_flag_raw as the streaming flag kernel at every
+    threshold, no programmatic dependent launch) produce the oracle's bits too.  A fresh process per form."""
     import subprocess
     import sys
     code = r'''

@@ -1,4 +1,4 @@
-"""Times the dense front end alone (yl_post_reset + yl_filter_dense) at the BASELINE size; YL_DENSE=groups selects the round-1 form."""
+"""Times the dense front end alone (yl_post_reset + yl_filter_dense) at the BASELINE size."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import yolov4_b200 as yb
@@ -25,4 +25,4 @@ for conf in (1e-4, 0.2):
     for _ in range(20): run()
     e1.record(); torch.cuda.synchronize()
     t = e0.elapsed_time(e1) / 20 * 1e3
-    print("%s conf %g: %.1f us (reset + filter)  %.0f GB/s" % (os.environ.get("YL_DENSE", "rows"), conf, t, dense.numel() * 4 / t / 1e3))
+    print("conf %g: %.1f us (reset + filter)  %.0f GB/s" % (conf, t, dense.numel() * 4 / t / 1e3))

@@ -8,7 +8,7 @@ mkdir -p $out
 timeout 300 python tools/kernel_times.py > $out/kernel_times_plain.log 2>&1 || { echo "kernel_times.py failed without ncu"; tail -5 $out/kernel_times_plain.log; exit 1; }
 # launch list of the whole program (durations only)
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -k regex:^k_ --csv --log-file $out/launches_all_kernel_families.csv python tools/kernel_times.py > /dev/null 2>&1
-for k in k_flag_raw k_emit_flagged k_segment_nms_bins k_gather_rows k_decode_dense k_decode_train k_decode_train_bwd k_filter_dense k_target_objmask k_target_scatter k_loss_match k_loss_obj; do
+for k in k_flag_raw k_emit_flagged k_segment_nms_bins k_gather_rows k_decode_dense k_decode_train k_decode_train_bwd k_filter_dense_rows k_target_objmask k_target_scatter k_loss_match k_loss_obj; do
   skip=1
   timeout 600 ncu --set full --clock-control none --import-source on -k regex:^$k -s $skip -c 1 -o $out/$k python tools/kernel_times.py > $out/$k.log 2>&1
   if [ -f $out/$k.ncu-rep ]; then

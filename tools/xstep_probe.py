@@ -1,6 +1,5 @@
 """Cross-step pipelining probe: two independent postprocessors (own inputs, workspaces, CUDA graphs) replayed alternately
-on one stream (serial) or on two streams (step i+1's streaming flag kernel next to step i's emit / NMS / gather).
-YL_FLAG_SMEM caps the flag kernel's CTAs per SM (set in the environment before the library loads)."""
+on one stream (serial) or on two streams (step i+1's streaming flag kernel next to step i's emit / NMS / gather)."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import yolov4_b200 as yb
@@ -28,4 +27,4 @@ for name, prios in (("serial", None), ("%d streams" % NHP, (0,) * NHP)):
     for s in streams: torch.cuda.current_stream().wait_stream(s)
     ev1.record(); torch.cuda.synchronize()
     t = ev0.elapsed_time(ev1) * 1e3 / N
-    print("%s flag_smem=%s %-18s %.1f us/step %.0f img/s" % (os.environ.get("TAG", ""), os.environ.get("YL_FLAG_SMEM", "0"), name, t, B / t * 1e6), flush=True)
+    print("%s %-18s %.1f us/step %.0f img/s" % (os.environ.get("TAG", ""), name, t, B / t * 1e6), flush=True)

@@ -53,7 +53,7 @@ def is_stale():
 
 
 def build_lib(force=False, verbose=False, extra=(), out=None, only=None):
-    """extra: additional nvcc flags (e.g. -DYL_WS_STAGES=3 for tuning builds); out: alternative output path;
+    """extra: additional nvcc flags (e.g. -DYL_FT_STAGES=4 for tuning builds); out: alternative output path;
     only: basenames of the sources the extra flags apply to (the other objects are those of the default build)."""
     if out is None and not force and not is_stale():
         return LIB

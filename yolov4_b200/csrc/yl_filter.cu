@@ -1,8 +1,11 @@
 // yl_filter.cu -- front ends of the postprocess pipeline: confidence filter -> candidate segments.
 //
-//   k_filter_raw    fused YOLOLayer eval decode (yololayer.py:88-166) + xywh->xyxy (utils.py:117-126) + conf filter
-//                   with multi-label expansion (utils.py:139-184), single pass over the raw head tensor.
-//   k_filter_dense  the same filter over an already decoded [B,M,5+C] tensor (the literal postprocess() input).
+//   yl_filter_raw    fused YOLOLayer eval decode (yololayer.py:88-166) + xywh->xyxy (utils.py:117-126) + conf filter
+//                    with multi-label expansion (utils.py:139-184) straight from the raw head tensors, in two kernels:
+//                    a streaming flag pass (k_flag_tma, or k_flag_raw) and an exact pass over the flagged pairs
+//                    (k_emit_flagged).
+//   yl_filter_dense  the same filter over an already decoded [B,M,5+C] tensor (the literal postprocess() input):
+//                    k_filter_dense_rows, or k_filter_dense_unaligned for a base that is not 16-byte aligned.
 //
 // Both append one self-contained 32-byte record per surviving (box,class) pair to the (image,class) segment
 // cand[((b*C+c)*cap_seg + slot)*2 + {0,1}] = {score bits, box row, cls_conf bits, obj_conf bits}, {x1, y1, x2, y2}.
@@ -45,8 +48,8 @@ struct RawLayer {
     int row_off;           // rows of the lower scales in the concatenated [M] axis (yolov4.py:324)
     int tiles;             // CTAs along x for this scale
     int vec;               // 4 = 128-bit loads, 1 = scalar loads (planes not 16-byte aligned, e.g. 19x19)
-    int tma;               // streamed with TMA by k_filter_raw_tma (else register-staged loads)
-    int tile_boxes;        // boxes per warp tile in k_filter_raw_tma (128 TMA, 32 scalar)
+    int tma;               // streamed with TMA by k_flag_tma (else register-staged loads)
+    int tile_boxes;        // boxes per tile (k_flag_tma: 128 TMA, 32 scalar; grid kernels: K1_THREADS * vec)
     float stride;
     float aw[3], ah[3];    // masked anchors in grid units (yololayer.py:73-76)
 };
@@ -312,9 +315,9 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
     if (qb) emit_batch<VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb);
 }
 
-// One tile = K1_THREADS*VEC consecutive boxes of one (image, anchor).  Phase 1 streams the class planes with one
-// compare per logit; phase 2 resolves the ~1% flagged pairs warp-cooperatively (all lanes, all loads in flight
-// together) instead of serially in the lane that owns the box.
+// One tile = K1_THREADS*VEC consecutive boxes of one (image, anchor).  Phase 1 (the flag kernels) streams the class
+// planes with one compare per logit; phase 2 (k_emit_flagged, whose shared memory this is) resolves the ~1% flagged
+// pairs warp-cooperatively (all lanes, all loads in flight together) instead of serially in the lane that owns the box.
 struct LdgSmem {
     EmitWarp e[K1_WARPS];
     float sobj[K1_WARPS][128];
@@ -403,24 +406,9 @@ __device__ __forceinline__ void ldg_stream(const RawParams &P, const RawLayer &L
         }
 }
 
-template <int VEC, int NW>
-__device__ __forceinline__ void filter_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba, LdgSmem &sm)
-{
-    const int p0 = (tile * K1_THREADS + threadIdx.x) * VEC;
-    const bool inb = p0 < Ly.F2;                                     // F2 % VEC == 0, so a vector is all in or all out
-    float obj[VEC], lth[VEC];
-    unsigned bits[VEC][NW];
-    ldg_stream<VEC, NW>(P, Ly, ba, p0, inb, obj, lth, bits);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int v = 0; v < VEC; ++v) sm.sobj[warp][lane * VEC + v] = obj[v];
-    emit_pairs<VEC, NW>(P, Ly, ba, (tile * K1_THREADS + warp * 32) * VEC, lth, bits, sm.e[warp], sm.sobj[warp]);
-}
-
-
 // ---------------------------------------------------------------------------------------------------------------
-// Split form (default): the streaming kernel does nothing but load, compare and store 16 bytes per box (flag words +
-// sigmoid(objectness)), so it runs at the memory system's pace; k_emit_flagged then resolves the flagged pairs.
+// The streaming kernel does nothing but load, compare and store 16 bytes per box (flag words + sigmoid(objectness)),
+// so it runs at the memory system's pace; k_emit_flagged then resolves the flagged pairs.
 // ---------------------------------------------------------------------------------------------------------------
 template <int VEC, int NW>
 __device__ __forceinline__ void flag_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba)
@@ -527,37 +515,14 @@ k_emit_flagged(const __grid_constant__ RawParams P)
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// TMA form of the streaming pass (scales whose planes are 16-byte aligned: 76/38 @608, 52/26 @416).
-//
-// Every warp is an independent pipeline over "warp tiles" (128 consecutive boxes of one (image, anchor) x all
-// planes), fetched from a global atomic counter.  Lane 0 issues cp.async.bulk copies (SASS UBLKCP) of
-// [WT_KC class planes x 512 B] into the warp's private ring of shared-memory stages; each stage has a
-// transaction mbarrier the warp waits on.  A stage is refilled as soon as the warp has read it, and the ring keeps
-// running into the NEXT tile, so the next tile's first chunks (and its objectness plane) land while the warp
-// resolves the current tile's flagged pairs.  Bytes in flight are set by shared memory (12 warps x 12 KB per SM),
-// not by registers, and no warp ever waits for another.  Only the planes the pass needs are streamed: objectness
-// and the classes; tx,ty,tw,th are fetched on demand for the few boxes that produce a candidate.
+// Bulk and tensor-map (TMA) copies into shared memory, each completing on a transaction mbarrier the consumer waits on:
+// the class-plane rings of k_flag_tma and the row batches of k_filter_dense_rows.
 // ---------------------------------------------------------------------------------------------------------------
 #ifndef YL_WT_KC
 #define YL_WT_KC 8
 #endif
-#ifndef YL_WT_STAGES
-#define YL_WT_STAGES 2
-#endif
-constexpr int WT_KC = YL_WT_KC;            // class planes per stage
-constexpr int WT_STAGES = YL_WT_STAGES;
+constexpr int WT_KC = YL_WT_KC;            // class planes per TMA box (one ring stage of k_flag_tma)
 constexpr int WT_BOX = 128;                // boxes per warp tile (32 lanes x float4)
-
-struct alignas(128) WtWarp {
-    float stage[WT_STAGES][WT_KC][WT_BOX];     // 12 KB
-    float objp[2][WT_BOX];                     // objectness plane of the current / the next tile
-    unsigned long long full[WT_STAGES], obj_full[2];
-    float sobj1[32];                           // sigmoid(objectness) of a scalar (non-TMA) warp tile
-    EmitWarp em;
-};
-struct WtSmem {
-    WtWarp w[K1_WARPS];
-};
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(unsigned long long *bar, unsigned count)
@@ -598,163 +563,6 @@ struct WtTile {
     int row0;              // plane row of class 0 in the scale's 2-D view: ba*(5+C) + 5
     int tma;
 };
-
-// P.layer[] holds only the TMA-capable scales; layer[l].tiles = ceil(F2 / WT_BOX) warp tiles per (image, anchor).
-// Tile queue order: TMA tiles with the scalar tiles spread evenly among them (one scalar tile after every `every`
-// TMA tiles), so the latency-bound scalar tiles overlap the streaming ones instead of forming a tail.
-__device__ __forceinline__ WtTile wt_tile(const RawParams &P, int t, int n_tiles, int nba)
-{
-    WtTile T;
-    T.np = 0; T.src = nullptr; T.layer = 0; T.ba = 0; T.p0 = 0; T.row0 = 0; T.tma = 0;
-    if (t >= n_tiles) return T;
-    int n_tma = 0;
-    for (int l = 0; l < P.n_layers; ++l) n_tma += P.layer[l].tma ? P.layer[l].tiles * nba : 0;
-    const int n_sc = n_tiles - n_tma;
-    if (n_sc > 0 && n_tma >= n_sc) {
-        // queue position -> tile index (TMA tiles are indices [0, n_tma), scalar tiles [n_tma, n_tiles))
-        const int every = n_tma / n_sc, G = every + 1;
-        if (t < n_sc * G) {
-            const int g = t / G, r = t - g * G;
-            t = (r < every) ? g * every + r : n_tma + g;
-        } else {
-            t = n_sc * every + (t - n_sc * G);                       // the n_tma % n_sc TMA tiles left over
-        }
-    }
-    int l = 0;
-    while (l < P.n_layers - 1 && t >= P.layer[l].tiles * nba) { t -= P.layer[l].tiles * nba; ++l; }
-    const int tp = P.layer[l].tiles;
-    const int bal = t / tp, tx = t - bal * tp;
-    T.layer = l;
-    T.ba = P.img_first * 3 + bal;
-    T.p0 = tx * P.layer[l].tile_boxes;
-    T.np = min(P.layer[l].tile_boxes, P.layer[l].F2 - T.p0);
-    T.tma = P.layer[l].tma;
-    T.src = P.layer[l].raw + ((size_t)T.ba * (5 + P.C)) * P.layer[l].F2 + T.p0;
-    T.row0 = T.ba * (5 + P.C) + 5;
-    return T;
-}
-
-template <int NW>
-__global__ void __launch_bounds__(K1_THREADS)
-k_filter_raw_tma(const __grid_constant__ RawParams P, const __grid_constant__ TmaMaps maps, int nba, int n_tiles,
-                 unsigned *__restrict__ tile_counter)
-{
-    extern __shared__ __align__(128) unsigned char wt_smem_raw[];
-    WtSmem &S = *reinterpret_cast<WtSmem *>(wt_smem_raw);
-    const unsigned FULL = 0xFFFFFFFFu;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    WtWarp &W = S.w[warp];
-    const int C = P.C;
-    const int n_cc = (C + WT_KC - 1) / WT_KC;                        // class chunks per tile
-
-    if (lane == 0) {
-        for (int s = 0; s < WT_STAGES; ++s) mbar_init(&W.full[s], 1);
-        mbar_init(&W.obj_full[0], 1);
-        mbar_init(&W.obj_full[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-
-    // lane 0 issues one class chunk of tile T into ring stage s
-    auto issue_chunk = [&](const WtTile &T, int c, int s) {
-        mbar_expect_tx(&W.full[s], WT_KC * WT_BOX * 4u);             // full box, zero fill included
-        tma_load_2d(&W.stage[s][0][0], &maps.m[T.layer], T.p0, T.row0 + c * WT_KC, &W.full[s]);
-    };
-    auto issue_obj = [&](const WtTile &T, int slot) {
-        const unsigned bytes = (unsigned)T.np * 4u;
-        mbar_expect_tx(&W.obj_full[slot], bytes);
-        bulk_g2s(&W.objp[slot][0], T.src + 4 * (size_t)P.layer[T.layer].F2, bytes, &W.obj_full[slot]);
-    };
-    auto fetch_tile = [&]() {
-        int t = 0;
-        if (lane == 0) t = (int)atomicAdd(tile_counter, 1u);
-        return wt_tile(P, __shfl_sync(FULL, t, 0), n_tiles, nba);
-    };
-
-    WtTile cur = fetch_tile();
-    if (cur.np == 0) return;
-    if (lane == 0 && cur.tma) {
-        issue_obj(cur, 0);
-        for (int c = 0; c < WT_STAGES && c < n_cc; ++c) issue_chunk(cur, c, c);
-    }
-    int s = 0;                       // ring stage of the next chunk to consume
-    unsigned ph = 0u;                // phase bit per ring stage
-    unsigned it = 0u;                // tiles processed by this warp (objectness slot = it & 1, phase = (it >> 1) & 1)
-
-    while (cur.np != 0) {
-        WtTile nxt = fetch_tile();
-        const RawLayer &Ly = P.layer[cur.layer];
-        if (!cur.tma) {
-            // scalar tile (planes not 16-byte aligned, e.g. the 19x19 scale): register-staged loads, 32 boxes per warp
-            float obj1[1], lth1[1];
-            unsigned bits1[1][NW];
-            // a TMA tile may follow: start its objectness plane and first chunks now, they land while this tile runs
-            if (lane == 0 && nxt.np != 0 && nxt.tma) {
-                issue_obj(nxt, it & 1);
-                for (int c = 0; c < WT_STAGES && c < n_cc; ++c) issue_chunk(nxt, c, (s + c) % WT_STAGES);
-            }
-            ldg_stream<1, NW>(P, Ly, cur.ba, cur.p0 + lane, lane < cur.np, obj1, lth1, bits1);
-            W.sobj1[lane] = obj1[0];
-            emit_pairs<1, NW>(P, Ly, cur.ba, cur.p0, lth1, bits1, W.em, W.sobj1);
-            cur = nxt;
-            continue;
-        }
-        if (!nxt.tma) nxt.np = -nxt.np;                          // no prefetch into a scalar tile (restored below)
-        if (lane == 0 && nxt.np > 0) issue_obj(nxt, (it + 1) & 1);
-        const bool inb = lane * 4 < cur.np;
-        float obj[4], lth[4];
-        {
-            mbar_wait(&W.obj_full[it & 1], (it >> 1) & 1u);
-            const float4 to = *reinterpret_cast<const float4 *>(&W.objp[it & 1][lane * 4]);
-            const float tv[4] = {to.x, to.y, to.z, to.w};
-#pragma unroll
-            for (int v = 0; v < 4; ++v) {
-                obj[v] = inb ? spec_sigmoidf(tv[v]) : 0.0f;
-                lth[v] = inb ? class_logit_bound(obj[v], P.thr) : kInf;
-            }
-        }
-        unsigned bits[4][NW];
-#pragma unroll
-        for (int w = 0; w < NW; ++w) {
-            unsigned m0 = 0u, m1 = 0u, m2 = 0u, m3 = 0u;
-#pragma unroll 1
-            for (int cc = 0; cc < 32 / WT_KC; ++cc) {
-                const int c = w * (32 / WT_KC) + cc;                 // class chunk index
-                if (c >= n_cc) break;                                // warp-uniform
-                mbar_wait(&W.full[s], (ph >> s) & 1u);
-                const int kn = min(WT_KC, C - c * WT_KC);
-                const float *sp = &W.stage[s][0][lane * 4];
-                unsigned a0 = 0u, a1 = 0u, a2 = 0u, a3 = 0u;
-#pragma unroll
-                for (int k = 0; k < WT_KC; ++k)
-                    if (k < kn) {
-                        const float4 tv = *reinterpret_cast<const float4 *>(sp + k * WT_BOX);
-                        flag_or(a0, tv.x, lth[0], 1u << k);
-                        flag_or(a1, tv.y, lth[1], 1u << k);
-                        flag_or(a2, tv.z, lth[2], 1u << k);
-                        flag_or(a3, tv.w, lth[3], 1u << k);
-                    }
-                const int sh = cc * WT_KC;
-                m0 |= a0 << sh; m1 |= a1 << sh; m2 |= a2 << sh; m3 |= a3 << sh;
-                __syncwarp();                                        // every lane has read the stage
-                if (lane == 0) {
-                    const int cn = c + WT_STAGES;                    // the chunk that takes this stage next
-                    if (cn < n_cc) issue_chunk(cur, cn, s);
-                    else if (nxt.np > 0 && cn - n_cc < n_cc) issue_chunk(nxt, cn - n_cc, s);
-                }
-                ph ^= 1u << s;
-                s = (s + 1 == WT_STAGES) ? 0 : s + 1;
-            }
-            bits[0][w] = m0; bits[1][w] = m1; bits[2][w] = m2; bits[3][w] = m3;
-        }
-        // sigmoid(objectness) replaces the logits in the tile's objectness slot: the exact pass reads it per box slot
-        *reinterpret_cast<float4 *>(&W.objp[it & 1][lane * 4]) = make_float4(obj[0], obj[1], obj[2], obj[3]);
-        emit_pairs<4, NW>(P, Ly, cur.ba, cur.p0, lth, bits, W.em, W.objp[it & 1]);
-        if (nxt.np < 0) nxt.np = -nxt.np;
-        cur = nxt;
-        ++it;
-    }
-}
 
 // ---------------------------------------------------------------------------------------------------------------
 // TMA form of the streaming FLAG pass (YL_FLAG=tma): the same output as k_flag_raw (flag words + sigmoid(objectness), 16 B per
@@ -968,28 +776,10 @@ k_flag_tma(const __grid_constant__ RawParams P, const __grid_constant__ TmaMaps 
     }
 }
 
-// grid = (sum of tiles over the scales, img_count*3): one launch covers all scales of an image group.
-template <int NW>
-__global__ void __launch_bounds__(K1_THREADS)
-k_filter_raw(const __grid_constant__ RawParams P)
-{
-    __shared__ LdgSmem sm;
-    const int ba = P.img_first * 3 + blockIdx.y;
-    int tile = blockIdx.x;
-    int l = 0;
-    while (l < P.n_layers - 1 && tile >= P.layer[l].tiles) { tile -= P.layer[l].tiles; ++l; }
-    if (P.layer[l].vec == 4) filter_tile<4, NW>(P, P.layer[l], tile, ba, sm);
-    else filter_tile<1, NW>(P, P.layer[l], tile, ba, sm);
-}
-
-// Dense front end: rows of 5+C contiguous floats.  Four consecutive rows are exactly (5+C) float4s, and a group of
-// four rows that starts at a row index divisible by four is 16-byte aligned, so a warp streams two such groups per
-// round with 128-bit loads (all of them in flight before the first use), parks them in shared memory and then walks the
-// eight rows: NaN-propagating row pre-filter, per-class test, one record per surviving pair.
+// Dense front end: rows of 5+C contiguous floats (cx, cy, w, h, obj, classes): NaN-propagating row pre-filter, per-class
+// test, one record per surviving pair.
 constexpr int KD_THREADS = 256;
-constexpr int KD_WARPS = KD_THREADS / 32;
 constexpr int KD_MAXJ = (5 + YL_MAX_CLASSES + 31) / 32;
-constexpr int KD_GROUPS = 2;                                // 4-row groups per warp and round
 
 // One decoded row held one element per lane and slot: e[j] = row[32 j + lane].
 template <int NJ>
@@ -1052,104 +842,12 @@ __device__ __forceinline__ void dense_row(const float (&e)[NJ], int nch, int C, 
         }
 }
 
-template <int NJ>
-__global__ void __launch_bounds__(KD_THREADS)
-k_filter_dense(const float *__restrict__ pred, long M, int C, int num_classes, float thr, int cap_seg,
-               long row_first, long row_end, long rows_total,
-               uint4 *__restrict__ cand, unsigned *__restrict__ seg_count)
-{
-    __shared__ __align__(16) float stage[KD_WARPS][KD_GROUPS * 4 * 32 * NJ];   // the round's 8 rows back to back: row rr at rr*nch
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const long wid = ((long)blockIdx.x * KD_THREADS + threadIdx.x) >> 5;
-    const long nwarps = ((long)gridDim.x * KD_THREADS) >> 5;
-    const int nch = 5 + C;
-    const long g_first = row_first >> 2, g_end = (row_end + 3) >> 2;          // 4-row groups that touch [row_first, row_end)
-    const long total4 = rows_total * nch / 4;                                 // whole float4s of the tensor (rows_total*nch*4 bytes)
-    const float4 *p4 = reinterpret_cast<const float4 *>(pred);
-    float4 v[KD_GROUPS][NJ];
-    auto load_round = [&](long g0) {
-        if (g0 + KD_GROUPS <= g_end && (g0 + KD_GROUPS) * nch <= total4) {
-            // the whole round lies inside the tensor (every round but the last few): no per-load bounds arithmetic
-            const float4 *src = p4 + g0 * nch + lane;
-#pragma unroll
-            for (int q = 0; q < KD_GROUPS; ++q)
-#pragma unroll
-                for (int j = 0; j < NJ; ++j)
-                    if (32 * j + lane < nch) v[q][j] = ldg_stream4(reinterpret_cast<const float *>(src + q * nch + 32 * j));
-            return;
-        }
-#pragma unroll
-        for (int q = 0; q < KD_GROUPS; ++q) {
-            const long base4 = (g0 + q) * nch;                                // group g = float4s [g*nch, (g+1)*nch)
-#pragma unroll
-            for (int j = 0; j < NJ; ++j) {
-                const int i = 32 * j + lane;
-                v[q][j] = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (i < nch && g0 + q < g_end) {
-                    if (base4 + i < total4) {
-                        v[q][j] = ldg_stream4(reinterpret_cast<const float *>(p4 + base4 + i));
-                    } else if (base4 + i == total4) {
-                        // the tensor ends inside this float4 (rows_total * (5+C) not a multiple of 4): scalar loads
-                        const long rem = rows_total * nch - 4 * total4;
-                        const float *src = pred + 4 * total4;
-                        if (rem > 0) v[q][j].x = src[0];
-                        if (rem > 1) v[q][j].y = src[1];
-                        if (rem > 2) v[q][j].z = src[2];
-                    }
-                }
-            }
-        }
-    };
-    // per-lane threshold of the fast row test: slot j holds channel 32 j + lane; only the first num_classes class channels
-    // can make a row interesting, every other slot gets +inf (never passes; what it reads is in-bounds scratch)
-    float thr_j[NJ];
-#pragma unroll
-    for (int j = 0; j < NJ; ++j) {
-        const int idx = 32 * j + lane;
-        thr_j[j] = (idx >= 5 && idx < 5 + num_classes) ? thr : kInf;
-    }
-    long g0 = g_first + wid * KD_GROUPS;
-    if (g0 < g_end) load_round(g0);
-    while (g0 < g_end) {
-#pragma unroll
-        for (int q = 0; q < KD_GROUPS; ++q)
-#pragma unroll
-            for (int j = 0; j < NJ; ++j) {
-                const int i = 32 * j + lane;
-                if (i < nch) reinterpret_cast<float4 *>(stage[warp])[q * nch + i] = v[q][j];
-            }
-        __syncwarp();
-        const long gn = g0 + nwarps * KD_GROUPS;
-        if (gn < g_end) load_round(gn);                                       // the next round is in flight while this one is walked
-        const long r0 = g0 * 4;
-        const int rr_lo = (int)max(0L, row_first - r0), rr_hi = (int)min((long)(4 * KD_GROUPS), row_end - r0);
-        const float *st = stage[warp] + rr_lo * nch + lane;
-#pragma unroll 1
-        for (int rr = rr_lo; rr < rr_hi; ++rr, st += nch) {                   // rows of this round inside [row_first, row_end)
-            // ~92 % of the rows end here: with obj >= 0 a row produces something only if one of its first num_classes
-            // classes passes the per-class test (see dense_row); NaN / negative objectness always take the full path
-            float e[NJ];
-#pragma unroll
-            for (int j = 0; j < NJ; ++j) e[j] = st[32 * j];
-            const float obj = st[4 - lane];
-            bool hit = false;
-#pragma unroll
-            for (int j = 0; j < NJ; ++j) hit |= (__fmul_rn(e[j], obj) >= thr_j[j]);
-            if (obj >= 0.0f && !__any_sync(0xFFFFFFFFu, hit)) continue;      // warp-uniform
-            dense_row<NJ>(e, nch, C, num_classes, thr, cap_seg, r0 + rr, M, cand, seg_count);
-        }
-        __syncwarp();                                                         // all lanes have read the stage
-        g0 = gn;
-    }
-}
-
-// Row-per-lane form of the dense front end (default).  A warp takes 32 consecutive rows -- 32 * (5+C) * 4 contiguous bytes, 16-byte
-// aligned when the first row index is a multiple of four -- as ONE bulk copy into its private shared-memory buffer (UBLKCP,
-// transaction mbarrier; the next batch is in flight while this one is walked), and every lane then walks ITS OWN row: the
+// Row-per-lane form of the dense front end (16-byte aligned base).  A warp takes 32 consecutive rows -- 32 * (5+C) * 4 contiguous
+// bytes, 16-byte aligned when the first row index is a multiple of four -- as ONE bulk copy into its private shared-memory buffer
+// (UBLKCP, transaction mbarrier; the next batch is in flight while this one is walked), and every lane then walks ITS OWN row: the
 // reference's row filter is literally `obj * max_c cls >= conf` (utils.py:139-148), i.e. one NaN-propagating max chain
 // (FMNMX3.NAN, a class pitch of 5+C = 85 words is conflict-free) and one multiply-compare per row and lane, a quarter of the
-// instructions of the warp-per-row walk above, which spends a vote per row.  The ~8 % of rows that pass go through dense_row()
-// with all lanes, as before.
+// instructions of a warp-per-row walk, which spends a vote per row.  The ~8 % of rows that pass are emitted with all lanes.
 constexpr int KR_ROWS = 32;
 
 __device__ __forceinline__ float max_nan(float a, float b)
@@ -1305,19 +1003,11 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32
                                     const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// YL_NO_TMA=1 forces the register-staged LDG kernel for every scale (A/B measurements).
-static const bool g_use_tma = !(getenv("YL_NO_TMA") && getenv("YL_NO_TMA")[0] == '1');
-// YL_FILTER selects the front-end form: "split" (default: streaming flag kernel + emit kernel) or "fused" (one kernel streams
-// and emits: the TMA pipeline where planes are 16-byte aligned, register-staged otherwise; measured slower, kept for A/B).
-static const bool g_split = !(getenv("YL_FILTER") && strcmp(getenv("YL_FILTER"), "fused") == 0);
-// YL_FLAG selects the streaming kernel of the split form: "tma" (default; k_flag_tma: one persistent CTA per SM, TMA rings in shared
+// YL_FLAG selects the streaming flag kernel: "tma" (default; k_flag_tma: one persistent CTA per SM, TMA rings in shared
 // memory, 40 % of the register file and 107 KB of shared memory -- the form that lets the emit / NMS / gather CTAs of the PREVIOUS
 // steps run next to it when several steps are in flight) or "ldg" (k_flag_raw: register-staged loads, a few per cent faster alone
 // -- 81 us against 86 -- but it fills the register file, so nothing overlaps it).
 static const bool g_flag_tma = getenv("YL_FLAG") ? strcmp(getenv("YL_FLAG"), "tma") == 0 : true;
-// YL_FLAG_SMEM=<bytes, at most 48 KB>: dynamic shared memory requested (and not used) by k_flag_raw, which caps its CTAs per
-// SM so that CTAs of other kernels can be co-resident (cross-step pipelining experiments, tools/xstep_probe.py).
-static const int g_flag_smem = getenv("YL_FLAG_SMEM") ? atoi(getenv("YL_FLAG_SMEM")) : 0;
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda).
 static int encode_plane_map(CUtensorMap *map, const float *raw, int F2, long rows, int box_rows = WT_KC)
 {
@@ -1392,7 +1082,7 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
     const int n_cc = (C + WT_KC - 1) / WT_KC;
     // the TMA flag kernel streams every plane of every box; with a high threshold the register-staged kernel's objectness-first
     // mode skips most class planes instead
-    const bool flag_tma = g_split && g_flag_tma && !base.sparse;
+    const bool flag_tma = g_flag_tma && !base.sparse;
     for (int l = 0; l < n_layers; ++l) {
         RawLayer &Ly = lay[l];
         Ly.raw = raw[l]; Ly.Fw = F[l]; Ly.F2 = F[l] * F[l]; Ly.row_off = row_off;
@@ -1405,51 +1095,52 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
         }
         // 128-bit loads / bulk copies need 16-byte aligned planes: F^2 % 4 == 0 and an aligned base (19x19, 13x13 fall back)
         Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 16 == 0)) ? 4 : 1;
-        Ly.tma = (Ly.vec == 4 && g_use_tma && n_cc >= (flag_tma ? FT_STAGES : WT_STAGES)) ? 1 : 0;
+        Ly.tma = (Ly.vec == 4 && n_cc >= FT_STAGES) ? 1 : 0;              // k_flag_tma's ring needs FT_STAGES class chunks
         Ly.tile_boxes = 0; Ly.tiles = 0;
         n_tma += Ly.tma;
         row_off += 3 * Ly.F2;
     }
-    // Pt: persistent TMA kernels (warp tiles of 128 boxes, 32 for the scalar scales; TMA scales first).  Pl: the grid kernels
-    // (k_flag_raw / k_emit_flagged / k_filter_raw: CTA tiles of K1_THREADS * vec boxes).
-    const bool persistent = n_tma > 0 && (flag_tma || !g_split);
+    // Pt: k_flag_tma (warp tiles of 128 boxes, 32 for the scalar scales; TMA scales first).  Pl: k_flag_raw / k_emit_flagged
+    // (CTA tiles of K1_THREADS * vec boxes).
+    const bool persistent = flag_tma && n_tma > 0;
     RawParams Pt = base, Pl = base;
-    int tiles_tma = 0, tiles_ldg = 0;
-    for (int pass = 0; pass < 2; ++pass)
-        for (int l = 0; l < n_layers; ++l) {
-            RawLayer Ly = lay[l];
-            if (persistent && (pass == 0) == (Ly.tma == 1)) {
-                Ly.tile_boxes = Ly.tma ? WT_BOX : 32;
+    if (persistent)
+        for (int tma = 1; tma >= 0; --tma)
+            for (int l = 0; l < n_layers; ++l) {
+                if (lay[l].tma != tma) continue;
+                RawLayer Ly = lay[l];
+                Ly.tile_boxes = tma ? WT_BOX : 32;
                 Ly.tiles = (Ly.F2 + Ly.tile_boxes - 1) / Ly.tile_boxes;
-                tiles_tma += Ly.tiles;
                 Pt.layer[Pt.n_layers++] = Ly;
             }
-            if (pass == 0 && (g_split || !persistent)) {
-                Ly.tma = 0;
-                Ly.tile_boxes = K1_THREADS * Ly.vec;
-                Ly.tiles = (Ly.F2 / Ly.vec + K1_THREADS - 1) / K1_THREADS;
-                tiles_ldg += Ly.tiles;
-                Pl.layer[Pl.n_layers++] = Ly;
-            }
-        }
+    int tiles_ldg = 0;
+    for (int l = 0; l < n_layers; ++l) {
+        RawLayer Ly = lay[l];
+        Ly.tma = 0;
+        Ly.tile_boxes = K1_THREADS * Ly.vec;
+        Ly.tiles = (Ly.F2 / Ly.vec + K1_THREADS - 1) / K1_THREADS;
+        tiles_ldg += Ly.tiles;
+        Pl.layer[Pl.n_layers++] = Ly;
+    }
     for (int l = Pt.n_layers; l < 3; ++l) { Pt.layer[l] = lay[0]; Pt.layer[l].tiles = 0; Pt.layer[l].tma = -1; }
     for (int l = Pl.n_layers; l < 3; ++l) { Pl.layer[l] = lay[0]; Pl.layer[l].tiles = 0; }
 
     // ---- counters (stages bit 2: the caller skipped yl_post_reset) ----
     if (stages & 4) {
-        if (g_split && (stages & 1) && flag_tma && persistent) {
+        if ((stages & 1) && persistent) {
             // the TMA flag kernel zeroes the segment counters itself, but not the two tile counters it draws from
             Pt.reset_words = (int)(L.off_tile_count / sizeof(unsigned));
             YL_CUDA_TRY(cudaMemsetAsync(w + L.off_tile_count, 0, L.counters_bytes - L.off_tile_count, st));
-        } else if (g_split && (stages & 1)) {
+        } else if (stages & 1) {
             Pl.reset_words = (int)(L.counters_bytes / sizeof(unsigned));   // k_flag_raw zeroes the counters (no memset node)
         } else {
             YL_CUDA_TRY(cudaMemsetAsync(ws, 0, L.counters_bytes, st));
         }
     }
 
-    // ---- persistent TMA kernels ----
-    if (persistent && (stages & 1)) {
+    // ---- streaming flag kernel ----
+    const dim3 grid(tiles_ldg, img_count * 3);
+    if ((stages & 1) && persistent) {
         const int nba = img_count * 3;
         unsigned *tile_counter = (unsigned *)(w + L.off_tile_count) + img_first;
         unsigned *scalar_counter = (unsigned *)(w + L.off_tile_count) + B + img_first;
@@ -1462,10 +1153,9 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
             const int rc = encode_plane_map(&maps.m[l], Pt.layer[l].raw, Pt.layer[l].F2, (long)B * 3 * (5 + C));
             if (rc != YL_OK) return rc;
         }
-        if (flag_tma) {
-            const size_t smem = sizeof(FtSmem);
-            const int want = (n_tma_tiles + FT_STREAM - 1) / FT_STREAM;
-            const int grid = want < g_num_sms() ? (want > 0 ? want : 1) : g_num_sms();
+        const size_t smem = sizeof(FtSmem);
+        const int want = (n_tma_tiles + FT_STREAM - 1) / FT_STREAM;
+        const int ft_grid = want < g_num_sms() ? (want > 0 ? want : 1) : g_num_sms();
 #define YL_FT_CASE(NW_)                                                                                              \
     case NW_: {                                                                                                      \
         static bool attr_done = false;                                                                               \
@@ -1473,64 +1163,32 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
             YL_CUDA_TRY(cudaFuncSetAttribute(k_flag_tma<NW_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
             attr_done = true;                                                                                        \
         }                                                                                                            \
-        k_flag_tma<NW_><<<grid, FT_THREADS, smem, st>>>(Pt, maps, nba, tile_counter, scalar_counter);                 \
+        k_flag_tma<NW_><<<ft_grid, FT_THREADS, smem, st>>>(Pt, maps, nba, tile_counter, scalar_counter);              \
     } break;
-            switch (NW) { YL_FT_CASE(1) YL_FT_CASE(2) YL_FT_CASE(3) YL_FT_CASE(4) }
+        switch (NW) { YL_FT_CASE(1) YL_FT_CASE(2) YL_FT_CASE(3) YL_FT_CASE(4) }
 #undef YL_FT_CASE
-        } else {
-            const int n_tiles = nba * tiles_tma;                             // warp tiles, TMA and scalar
-            const size_t smem = sizeof(WtSmem);
-            const int ctas_per_sm = (int)((227 * 1024) / (smem + 1024));
-            const int want = (n_tiles + K1_WARPS - 1) / K1_WARPS;
-            const int grid = want < ctas_per_sm * g_num_sms() ? want : ctas_per_sm * g_num_sms();
-#define YL_TMA_CASE(NW_)                                                                                             \
-    case NW_: {                                                                                                      \
-        static bool attr_done = false;                                                                               \
-        if (!attr_done) {                                                                                            \
-            YL_CUDA_TRY(cudaFuncSetAttribute(k_filter_raw_tma<NW_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-            attr_done = true;                                                                                        \
-        }                                                                                                            \
-        k_filter_raw_tma<NW_><<<grid, K1_THREADS, smem, st>>>(Pt, maps, nba, n_tiles, tile_counter);                  \
-    } break;
-            switch (NW) { YL_TMA_CASE(1) YL_TMA_CASE(2) YL_TMA_CASE(3) YL_TMA_CASE(4) }
-#undef YL_TMA_CASE
+        YL_LAUNCH_CHECK();
+    } else if (stages & 1) {
+        switch (NW) {
+        case 1: k_flag_raw<1><<<grid, K1_THREADS, 0, st>>>(Pl); break;
+        case 2: k_flag_raw<2><<<grid, K1_THREADS, 0, st>>>(Pl); break;
+        case 3: k_flag_raw<3><<<grid, K1_THREADS, 0, st>>>(Pl); break;
+        default: k_flag_raw<4><<<grid, K1_THREADS, 0, st>>>(Pl); break;
         }
         YL_LAUNCH_CHECK();
     }
 
-    // ---- grid kernels ----
-    if (Pl.n_layers > 0) {
-        dim3 grid(tiles_ldg, img_count * 3);
-        if (g_split) {
-            if ((stages & 1) && !(flag_tma && persistent)) {
-                switch (NW) {
-                case 1: k_flag_raw<1><<<grid, K1_THREADS, g_flag_smem, st>>>(Pl); break;
-                case 2: k_flag_raw<2><<<grid, K1_THREADS, g_flag_smem, st>>>(Pl); break;
-                case 3: k_flag_raw<3><<<grid, K1_THREADS, g_flag_smem, st>>>(Pl); break;
-                default: k_flag_raw<4><<<grid, K1_THREADS, g_flag_smem, st>>>(Pl); break;
-                }
-                YL_LAUNCH_CHECK();
-            }
-            if (stages & 2) {
-                const bool pdl = pdl_enabled() && (stages & 1);             // directly behind the flag kernel on the stream
-                cudaError_t le;
-                switch (NW) {
-                case 1: le = launch_after(k_emit_flagged<1>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-                case 2: le = launch_after(k_emit_flagged<2>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-                case 3: le = launch_after(k_emit_flagged<3>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-                default: le = launch_after(k_emit_flagged<4>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-                }
-                if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
-            }
-        } else if (stages & 1) {
-            switch (NW) {
-            case 1: k_filter_raw<1><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-            case 2: k_filter_raw<2><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-            case 3: k_filter_raw<3><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-            default: k_filter_raw<4><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-            }
-            YL_LAUNCH_CHECK();
+    // ---- emit kernel ----
+    if (stages & 2) {
+        const bool pdl = pdl_enabled() && (stages & 1);                     // directly behind the flag kernel on the stream
+        cudaError_t le;
+        switch (NW) {
+        case 1: le = launch_after(k_emit_flagged<1>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
+        case 2: le = launch_after(k_emit_flagged<2>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
+        case 3: le = launch_after(k_emit_flagged<3>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
+        default: le = launch_after(k_emit_flagged<4>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
         }
+        if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
     }
     return YL_OK;
 }
@@ -1568,21 +1226,19 @@ extern "C" int yl_filter_dense(const float *pred, int B, long M, int C, int num_
     const long row_first = (long)img_first * M, row_end = (long)(img_first + img_count) * M, rows_total = (long)B * M;
     uint4 *cand = (uint4 *)(w + L.off_cand);
     unsigned *seg_count = (unsigned *)(w + L.off_seg_count);
-    static const bool dense_groups = getenv("YL_DENSE") && strcmp(getenv("YL_DENSE"), "groups") == 0;   // the round-1 form, for A/B
-    const int nj = (5 + C + 31) / 32;
-    if (((uintptr_t)pred) % 16 == 0 && !dense_groups && nj <= KD_MAXJ) {
-        // row-per-lane form: 2 x 32 rows of shared memory per warp, as many warps per CTA as fit 200 KB, one CTA per SM
+    if (((uintptr_t)pred) % 16 == 0) {
+        // row-per-lane form: 2 x 32 rows of shared memory per warp, as many warps per CTA as fit 226 KB (at most 8), one CTA per SM
+        static_assert(2 * KR_ROWS * (5 + YL_MAX_CLASSES) * sizeof(float) <= 226 * 1024 - 256,
+                      "the two row buffers of one warp must fit the shared-memory budget at YL_MAX_CLASSES");
         const size_t per_warp = (size_t)2 * KR_ROWS * (5 + C) * sizeof(float);
-        static const int max_warps = getenv("YL_KR_WARPS") ? atoi(getenv("YL_KR_WARPS")) : 8;
         int warps = (int)((226 * 1024 - 256) / per_warp);
-        warps = warps > max_warps ? max_warps : warps;
-        if (warps >= 1) {
-            const size_t smem = per_warp * warps + 16 * (size_t)warps;
-            const long batches = (row_end + KR_ROWS - 1) / KR_ROWS - row_first / KR_ROWS;
-            const long ctas = (batches + warps - 1) / warps;
-            const int grid = (int)(ctas < g_num_sms() ? (ctas > 0 ? ctas : 1) : g_num_sms());
-            cudaStream_t st = (cudaStream_t)stream;
-            switch (nj) {
+        warps = warps > 8 ? 8 : warps;
+        const size_t smem = per_warp * warps + 16 * (size_t)warps;
+        const long batches = (row_end + KR_ROWS - 1) / KR_ROWS - row_first / KR_ROWS;
+        const long ctas = (batches + warps - 1) / warps;
+        const int grid = (int)(ctas < g_num_sms() ? (ctas > 0 ? ctas : 1) : g_num_sms());
+        cudaStream_t st = (cudaStream_t)stream;
+        switch ((5 + C + 31) / 32) {
 #define YL_KR_CASE(NJ_)                                                                                               \
     case NJ_: {                                                                                                       \
         static size_t attr_smem = 0;                                                                                  \
@@ -1593,30 +1249,9 @@ extern "C" int yl_filter_dense(const float *pred, int B, long M, int C, int num_
         k_filter_dense_rows<NJ_><<<grid, 32 * warps, smem, st>>>(pred, M, C, num_classes, conf_thre, cap_seg, row_first, row_end, \
                                                                  rows_total, cand, seg_count);                        \
     } break;
-                YL_KR_CASE(1) YL_KR_CASE(2) YL_KR_CASE(3) YL_KR_CASE(4)
-            default: YL_KR_CASE(KD_MAXJ)
+            YL_KR_CASE(1) YL_KR_CASE(2) YL_KR_CASE(3) YL_KR_CASE(4)
+        default: YL_KR_CASE(KD_MAXJ)
 #undef YL_KR_CASE
-            }
-            YL_LAUNCH_CHECK();
-            return YL_OK;
-        }
-    }
-    if (((uintptr_t)pred) % 16 == 0) {
-        const long warps_needed = ((row_end - row_first) / 4 + KD_GROUPS) / KD_GROUPS;
-        const long blocks_needed = (warps_needed + KD_WARPS - 1) / KD_WARPS;
-        const int grid = (int)(blocks_needed < 148L * 8 ? blocks_needed : 148L * 8);
-        switch ((5 + C + 31) / 32) {
-#define YL_KD_CASE(NJ_)                                                                                               \
-    case NJ_:                                                                                                         \
-        k_filter_dense<NJ_><<<grid, KD_THREADS, 0, (cudaStream_t)stream>>>(pred, M, C, num_classes, conf_thre, cap_seg, \
-                                                                          row_first, row_end, rows_total, cand, seg_count); \
-        break;
-            YL_KD_CASE(1) YL_KD_CASE(2) YL_KD_CASE(3) YL_KD_CASE(4)
-        default:
-            k_filter_dense<KD_MAXJ><<<grid, KD_THREADS, 0, (cudaStream_t)stream>>>(pred, M, C, num_classes, conf_thre, cap_seg,
-                                                                                  row_first, row_end, rows_total, cand, seg_count);
-            break;
-#undef YL_KD_CASE
         }
     } else {
         const long blocks_needed = ((row_end - row_first) * 32 + KD_THREADS - 1) / KD_THREADS;
