@@ -10,7 +10,9 @@
  *   - every function returns int: 0 = YL_OK, 1..99 = argument errors, 1000+e = cudaError_t e.  Never throws.
  *   - all device-pointer functions are stream-ordered on `stream` (a cudaStream_t passed as void*), do not
  *     allocate, do not synchronise, and are CUDA-graph capturable.
- *   - fp32 everywhere (the reference trains and evaluates with apex O0, README.md:106,112).
+ *   - fp32 everywhere (the reference trains and evaluates with apex O0, README.md:106,112), except the head tensors of the
+ *     fused detection path (yl_filter_raw_typed, yl_context_create_typed), which may also be fp16 or bf16 as a model run
+ *     with .half() or under autocast produces them: they are widened exactly to fp32 and the fp32 spec applies from there.
  *   - sigmoid / exp / log are the "spec math" of DESIGN.md section 4 (fixed IEEE op sequences), so results are
  *     bit-reproducible and identical to the CPU oracle.
  */
@@ -33,6 +35,11 @@ extern "C" {
 
 #define YL_MAX_CLASSES 128
 #define YL_ABI_VERSION 1
+
+/* element type of the head tensors of the fused detection path */
+#define YL_DTYPE_F32 0
+#define YL_DTYPE_F16 1
+#define YL_DTYPE_BF16 2
 
 typedef void *yl_stream_t; /* cudaStream_t */
 
@@ -115,6 +122,15 @@ int yl_filter_raw_stage(const float *const *raw, const int *F, int n_layers, int
                         const float *anchors_px, const int *anchor_mask, float conf_thre,
                         void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                         int stages, yl_stream_t stream);
+
+/* yl_filter_raw_stage for head tensors of element type `dtype` (YL_DTYPE_*).  A 16-bit value is widened exactly to fp32 (every
+ * fp16 / bf16 value, subnormals, +-0, +-inf and NaN included, has an exact fp32 image), so the candidates are bit for bit those of
+ * yl_filter_raw_stage on the widened tensors; the workspace and everything after this call are unchanged.  16-bit input takes the
+ * register-staged flag kernel (k_flag_raw) on every scale.  yl_filter_raw and yl_filter_raw_stage are this call with
+ * YL_DTYPE_F32.  An unknown dtype returns YL_ERR_ARG before any CUDA call. */
+int yl_filter_raw_typed(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
+                        const float *anchors_px, const int *anchor_mask, float conf_thre, void *ws, size_t ws_bytes,
+                        long M, int cap_seg, int img_first, int img_count, int stages, yl_stream_t stream);
 
 /* pred [B, M, 5+C] decoded (cx,cy,w,h,obj,cls...), not modified (the reference's in-place xyxy overwrite,
  * utils.py:126, is an unobserved side effect).  num_classes <= C limits the row pre-filter (utils.py:139). */
@@ -204,13 +220,19 @@ int yl_loss_backward(const float *gobj, const int *mcell, const float *mgrad, co
  * Host-buffer entry (what a non-Python caller binds; also the bench's end-to-end leg): raw head tensors in
  * HOST memory -> detections in HOST memory.  The context owns device staging buffers, workspace, streams and
  * pinned bounce buffers; H2D copies, kernels and the D2H of rows/counts are all inside the call.
- *   raw_host[l] [B, 3*(5+C), F[l], F[l]] fp32 host (pinned or pageable)
- *   out_rows_host [B, cap_out, 7], counts_host [B]
+ *   raw_host[l] [B, 3*(5+C), F[l], F[l]] host (pinned or pageable), elements of the context's dtype: fp32 for yl_context_create;
+ *               for yl_context_create_typed with YL_DTYPE_F16 / YL_DTYPE_BF16, 16-bit elements (IEEE binary16 / bfloat16 bit
+ *               patterns), which halves the bytes uploaded
+ *   out_rows_host [B, cap_out, 7] fp32, counts_host [B]
  * Returns YL_OK; counts_host[b] > cap_out means image b was truncated.
  * --------------------------------------------------------------------------------------------------------- */
 typedef struct yl_context yl_context;
 int yl_context_create(yl_context **ctx, int device, int B, const int *F, int n_layers, int C,
                       const float *anchors_px, const int *anchor_mask, int cap_seg, long cap_out);
+/* yl_context_create for head tensors of element type `dtype` (YL_DTYPE_*); the device staging buffers hold that type.
+ * An unknown dtype returns YL_ERR_ARG before any CUDA call. */
+int yl_context_create_typed(yl_context **ctx, int device, int B, const int *F, int n_layers, int C, int dtype,
+                            const float *anchors_px, const int *anchor_mask, int cap_seg, long cap_out);
 int yl_context_destroy(yl_context *ctx);
 int yl_detect_host(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre,
                    float *out_rows_host, int *counts_host);

@@ -62,12 +62,13 @@ extern "C" int yl_selftest_rcp(unsigned long long *bad_dev, yl_stream_t stream)
 // group g-2 travel back on a third stream (PCIe is full duplex), so only the last group's results trail the uploads.
 // -------------------------------------------------------------------------------------------------------------
 struct yl_context {
-    int device, B, n_layers, C, cap_seg, n_groups;
+    int device, B, n_layers, C, cap_seg, n_groups, dtype;
+    size_t esize;                  // bytes per head tensor element (dtype)
     long cap_out, M;
     int F[3];
     float anchors[18];
     int mask[9];
-    float *d_raw[3];
+    void *d_raw[3];
     void *ws;
     size_t ws_bytes;
     float *d_rows;
@@ -96,15 +97,17 @@ extern "C" int yl_context_destroy(yl_context *c)
     return YL_OK;
 }
 
-extern "C" int yl_context_create(yl_context **out, int device, int B, const int *F, int n_layers, int C,
-                                 const float *anchors_px, const int *anchor_mask, int cap_seg, long cap_out)
+extern "C" int yl_context_create_typed(yl_context **out, int device, int B, const int *F, int n_layers, int C, int dtype,
+                                       const float *anchors_px, const int *anchor_mask, int cap_seg, long cap_out)
 {
     if (!out || !F || !anchors_px || !anchor_mask || B <= 0 || n_layers < 1 || n_layers > 3 || C <= 0 || cap_seg <= 0 || cap_out <= 0)
         return YL_ERR_ARG;
+    if (dtype != YL_DTYPE_F32 && dtype != YL_DTYPE_F16 && dtype != YL_DTYPE_BF16) return YL_ERR_ARG;
     if (C > YL_MAX_CLASSES) return YL_ERR_CLASSES;
     yl_context *c = (yl_context *)calloc(1, sizeof(yl_context));
     if (!c) return YL_ERR_ARG;
     c->device = device; c->B = B; c->n_layers = n_layers; c->C = C; c->cap_seg = cap_seg; c->cap_out = cap_out;
+    c->dtype = dtype; c->esize = dtype == YL_DTYPE_F32 ? sizeof(float) : 2;
     c->n_groups = B >= 16 ? 8 : (B >= 2 ? 2 : 1);
     memcpy(c->anchors, anchors_px, sizeof(float) * 18);
     memcpy(c->mask, anchor_mask, sizeof(int) * 9);
@@ -114,7 +117,7 @@ extern "C" int yl_context_create(yl_context **out, int device, int B, const int 
 #define CTX_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { rc = YL_ERR_CUDA_BASE + (int)e__; goto fail; } } while (0)
     CTX_TRY(cudaSetDevice(device));
     for (int l = 0; l < n_layers; ++l)
-        CTX_TRY(cudaMalloc(&c->d_raw[l], sizeof(float) * (size_t)B * 3 * (5 + C) * F[l] * F[l]));
+        CTX_TRY(cudaMalloc(&c->d_raw[l], c->esize * (size_t)B * 3 * (5 + C) * F[l] * F[l]));
     c->ws_bytes = yl_post_workspace_bytes(B, c->M, C, cap_seg);
     CTX_TRY(cudaMalloc(&c->ws, c->ws_bytes));
     CTX_TRY(cudaMalloc(&c->d_rows, sizeof(float) * 7 * (size_t)B * cap_out));
@@ -134,6 +137,12 @@ fail:
     return rc;
 }
 
+extern "C" int yl_context_create(yl_context **out, int device, int B, const int *F, int n_layers, int C,
+                                 const float *anchors_px, const int *anchor_mask, int cap_seg, long cap_out)
+{
+    return yl_context_create_typed(out, device, B, F, n_layers, C, YL_DTYPE_F32, anchors_px, anchor_mask, cap_seg, cap_out);
+}
+
 extern "C" int yl_detect_host(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre,
                               float *out_rows_host, int *counts_host)
 {
@@ -147,13 +156,15 @@ extern "C" int yl_detect_host(yl_context *c, const float *const *raw_host, float
         if (i1 == i0) continue;
         for (int l = 0; l < c->n_layers; ++l) {
             const size_t per_img = (size_t)3 * (5 + C) * c->F[l] * c->F[l];
-            YL_CUDA_TRY(cudaMemcpyAsync(c->d_raw[l] + per_img * i0, raw_host[l] + per_img * i0, sizeof(float) * per_img * (i1 - i0),
+            // raw_host[l] holds elements of the context's dtype, whatever the declared pointer type
+            const size_t off = c->esize * per_img * i0;
+            YL_CUDA_TRY(cudaMemcpyAsync((char *)c->d_raw[l] + off, (const char *)raw_host[l] + off, c->esize * per_img * (i1 - i0),
                                         cudaMemcpyHostToDevice, c->s_copy));
         }
         YL_CUDA_TRY(cudaEventRecord(c->ev_copied[g], c->s_copy));
         YL_CUDA_TRY(cudaStreamWaitEvent(c->s_comp, c->ev_copied[g], 0));
-        rc = yl_filter_raw((const float *const *)c->d_raw, c->F, c->n_layers, B, C, c->anchors, c->mask, conf_thre, c->ws,
-                           c->ws_bytes, c->M, c->cap_seg, i0, i1 - i0, c->s_comp);
+        rc = yl_filter_raw_typed((const void *const *)c->d_raw, c->dtype, c->F, c->n_layers, B, C, c->anchors, c->mask, conf_thre,
+                                 c->ws, c->ws_bytes, c->M, c->cap_seg, i0, i1 - i0, 3, c->s_comp);
         if (rc != YL_OK) return rc;
         rc = yl_nms(c->ws, c->ws_bytes, B, c->M, C, c->cap_seg, nms_thre, c->d_rows, c->cap_out, c->d_meta, i0, i1 - i0, c->s_comp);
         if (rc != YL_OK) return rc;

@@ -41,13 +41,44 @@ __device__ __forceinline__ void flag_or(unsigned &bits, float t, float lth, unsi
     asm("{\n\t.reg .pred p;\n\tsetp.lt.f32 p, %1, %2;\n\t@!p or.b32 %0, %0, %3;\n\t}" : "+r"(bits) : "f"(t), "f"(lth), "r"(bit));
 }
 
+// The same test for a packed pair of 16-bit logits (boxes 2j, 2j+1 of one class plane) against the pair's bounds rounded down to
+// the element type once per box: one HSETP2 for two logits.  Still conservative (t >= lth implies t >= rd(lth)); a NaN half sets
+// its bit, as in flag_or.
+__device__ __forceinline__ void flag_or2(unsigned &b0, unsigned &b1, unsigned t2, unsigned l2, unsigned bit, __half)
+{
+    asm("{\n\t.reg .pred p, q;\n\tsetp.lt.f16x2 p|q, %2, %3;\n\t@!p or.b32 %0, %0, %4;\n\t@!q or.b32 %1, %1, %4;\n\t}"
+        : "+r"(b0), "+r"(b1) : "r"(t2), "r"(l2), "r"(bit));
+}
+__device__ __forceinline__ void flag_or2(unsigned &b0, unsigned &b1, unsigned t2, unsigned l2, unsigned bit, __nv_bfloat16)
+{
+    asm("{\n\t.reg .pred p, q;\n\tsetp.lt.bf16x2 p|q, %2, %3;\n\t@!p or.b32 %0, %0, %4;\n\t@!q or.b32 %1, %1, %4;\n\t}"
+        : "+r"(b0), "+r"(b1) : "r"(t2), "r"(l2), "r"(bit));
+}
+__device__ __forceinline__ unsigned short round_down_bits(float x, __half) { return __half_as_ushort(__float2half_rd(x)); }
+__device__ __forceinline__ unsigned short round_down_bits(float x, __nv_bfloat16) { return __bfloat16_as_ushort(__float2bfloat16_rd(x)); }
+
+// Flags one class plane's VEC logits of a lane into word w of bits.  fp32 and scalar 16-bit elements: flag_or on the (widened)
+// value; 16-bit pairs: flag_or2 against the packed rounded-down bounds lpk.
+template <typename T, int VEC, int NW>
+__device__ __forceinline__ void flag_plane(unsigned (&bits)[VEC][NW], int w, const PlaneVec<T, VEC> &t, const float (&lth)[VEC],
+                                           const unsigned (&lpk)[(VEC + 1) / 2], unsigned bit)
+{
+    if constexpr (sizeof(T) == 4 || VEC == 1) {
+#pragma unroll
+        for (int v = 0; v < VEC; ++v) flag_or(bits[v][w], t.at(v), lth[v], bit);
+    } else {
+#pragma unroll
+        for (int j = 0; j < VEC / 2; ++j) flag_or2(bits[2 * j][w], bits[2 * j + 1][w], t.w[j], lpk[j], bit, T());
+    }
+}
+
 // One scale of the head as the kernel sees it.
 struct RawLayer {
-    const float *raw;      // [B, 3, 5+C, F, F]
+    const void *raw;       // [B, 3, 5+C, F, F] of the element type the kernel is instantiated for
     int Fw, F2;
     int row_off;           // rows of the lower scales in the concatenated [M] axis (yolov4.py:324)
     int tiles;             // CTAs along x for this scale
-    int vec;               // 4 = 128-bit loads, 1 = scalar loads (planes not 16-byte aligned, e.g. 19x19)
+    int vec;               // 4 = 128-bit loads (64-bit for 16-bit elements), 1 = scalar loads (planes not aligned, e.g. 19x19)
     int tma;               // streamed with TMA by k_flag_tma (else register-staged loads)
     int tile_boxes;        // boxes per tile (k_flag_tma: 128 TMA, 32 scalar; grid kernels: K1_THREADS * vec)
     float stride;
@@ -93,9 +124,10 @@ __device__ __forceinline__ float4 decode_box_v(float tx, float ty, float tw, flo
 }
 
 // Decode one box (yololayer.py:150-162) and convert to corners (utils.py:117-126).
-__device__ __forceinline__ float4 decode_box(const float *bp, int F2, int Fw, int p, float aw, float ah, float stride)
+template <typename T>
+__device__ __forceinline__ float4 decode_box(const T *bp, int F2, int Fw, int p, float aw, float ah, float stride)
 {
-    const float tx = bp[0], ty = bp[(size_t)F2], tw = bp[2 * (size_t)F2], th = bp[3 * (size_t)F2];
+    const float tx = widen(bp[0]), ty = widen(bp[(size_t)F2]), tw = widen(bp[2 * (size_t)F2]), th = widen(bp[3 * (size_t)F2]);
     return decode_box_v(tx, ty, tw, th, Fw, p, aw, ah, stride);
 }
 
@@ -118,14 +150,14 @@ __device__ __forceinline__ int nth_slot(const unsigned (&w)[4], const int (&c)[4
     return 32 * j + (int)__fns(wsel, 0, i - cs + 1);
 }
 
-template <int VEC>
+template <typename T, int VEC>
 __device__ __forceinline__ void emit_batch(const RawParams &P, const RawLayer &Ly, EmitWarp &E, const float *sobj,
-                                           const float *wbase, int b, int a, int wp0, int total)
+                                           const T *wbase, int b, int a, int wp0, int total)
 {
     const int lane = threadIdx.x & 31;
     const int C = P.C, F2 = Ly.F2;
     const float thr = P.thr;
-    const float *wcp = wbase + 5 * (size_t)F2;
+    const T *wcp = wbase + 5 * (size_t)F2;
     const int row_base = Ly.row_off + a * F2;                        // + p = row inside the image
     __syncwarp();                                                    // queue entries and flg/any/nan masks are visible
     unsigned fw[4];
@@ -140,8 +172,8 @@ __device__ __forceinline__ void emit_batch(const RawParams &P, const RawLayer &L
     float tx = 0.f, ty = 0.f, tw = 0.f, th = 0.f;
     if (lane < nflag) {
         sbs = nth_slot(fw, fc, lane);
-        const float *bp = wbase + sbs;
-        tx = bp[0]; ty = bp[(size_t)F2]; tw = bp[2 * (size_t)F2]; th = bp[3 * (size_t)F2];
+        const T *bp = wbase + sbs;
+        tx = widen(bp[0]); ty = widen(bp[(size_t)F2]); tw = widen(bp[2 * (size_t)F2]); th = widen(bp[3 * (size_t)F2]);
     }
     for (int e0 = 0; e0 < total; e0 += 128) {
         float t[4];
@@ -150,7 +182,7 @@ __device__ __forceinline__ void emit_batch(const RawParams &P, const RawLayer &L
         for (int u = 0; u < 4; ++u) {
             const int q = e0 + 32 * u + lane;
             en[u] = (q < total) ? E.ent[q] : 0u;
-            t[u] = (q < total) ? wcp[(size_t)(en[u] & 0x7F) * F2 + (en[u] >> 8)] : 0.0f;
+            t[u] = (q < total) ? widen(wcp[(size_t)(en[u] & 0x7F) * F2 + (en[u] >> 8)]) : 0.0f;
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -268,7 +300,7 @@ __device__ __forceinline__ void queue_pairs(const unsigned (&bits)[VEC][NW], con
 // position a warp prefix sum gives it, and the queue is resolved as one batch.  Dense tiles fall back to expanding the
 // flag words box by box and resolving the queue in batches of whole boxes.  sobj must already hold
 // sigmoid(objectness) per box slot.
-template <int VEC, int NW>
+template <typename T, int VEC, int NW>
 __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &Ly, int ba, int wp0,
                                            const float (&lth)[VEC], unsigned (&bits)[VEC][NW], EmitWarp &E, const float *sobj)
 {
@@ -279,12 +311,12 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
     int first;
     const int total = pair_prefix<VEC, NW>(lth, bits, anyv, first);
     if (total == 0) return;                                          // warp-uniform
-    const float *wbase = Ly.raw + ((size_t)ba * (5 + P.C)) * Ly.F2 + wp0;
+    const T *wbase = (const T *)Ly.raw + ((size_t)ba * (5 + P.C)) * Ly.F2 + wp0;
     if (lane < 4) { E.any[lane] = 0u; E.nan[lane] = 0u; E.flg[lane] = 0u; }
     __syncwarp();
     if (total <= K1_QCAP) {
         queue_pairs<VEC, NW>(bits, anyv, first, E.ent, E.flg);
-        emit_batch<VEC>(P, Ly, E, sobj, wbase, b, a, wp0, total);
+        emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, total);
         return;
     }
     unsigned flagged[VEC];
@@ -301,7 +333,7 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
             int n = 0;
 #pragma unroll
             for (int w = 0; w < NW; ++w) { m[w] = __shfl_sync(FULL, bits[v][w], L); n += __popc(m[w]); }
-            if (qb + n > K1_QCAP) { emit_batch<VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb); qb = 0; __syncwarp(); }
+            if (qb + n > K1_QCAP) { emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb); qb = 0; __syncwarp(); }
             const int bs = L * VEC + v;
             if (lane == 0) E.flg[bs >> 5] |= 1u << (bs & 31);
             const unsigned hdr = (unsigned)bs << 8;
@@ -312,7 +344,7 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
             }
         }
     }
-    if (qb) emit_batch<VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb);
+    if (qb) emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb);
 }
 
 // One tile = K1_THREADS*VEC consecutive boxes of one (image, anchor).  Phase 1 (the flag kernels) streams the class
@@ -323,49 +355,61 @@ struct LdgSmem {
     float sobj[K1_WARPS][128];
 };
 
-// Register-staged phase 1 for one lane: VEC consecutive boxes starting at p0 of (image, anchor) ba.
-template <int VEC, int NW>
+// Register-staged phase 1 for one lane: VEC consecutive boxes starting at p0 of (image, anchor) ba.  KB class planes are
+// requested per batch: eight for fp32, sixteen for 16-bit elements, so a lane keeps as many bytes in flight as the fp32 form of
+// its vector shape (16-bit vectors are 64-bit loads: a 128-bit form with 8 boxes per lane would need twice the flag-word
+// registers and spills at 80 classes).
+template <typename T, int VEC, int NW>
 __device__ __forceinline__ void ldg_stream(const RawParams &P, const RawLayer &Ly, int ba, int p0, bool inb,
                                            float (&obj)[VEC], float (&lth)[VEC], unsigned (&bits)[VEC][NW])
 {
+    constexpr int KB = sizeof(T) == 4 ? 8 : 16;
     const int C = P.C, F2 = Ly.F2;
     const float thr = P.thr;
     const int nch = 5 + C;
-    const float *base = Ly.raw + ((size_t)ba * nch) * F2 + (inb ? p0 : 0);
-    const float *cp = base + 5 * (size_t)F2;
-    // The objectness plane and the first eight class planes are requested together: the bound needs sigmoid(obj),
+    const T *base = (const T *)Ly.raw + ((size_t)ba * nch) * F2 + (inb ? p0 : 0);
+    const T *cp = base + 5 * (size_t)F2;
+    // The objectness plane and the first KB class planes are requested together: the bound needs sigmoid(obj),
     // but the class loads do not, so no load latency is spent with nothing else in flight.
     // (With a high threshold -- detect setting, conf 0.2 -- almost every box is dead on objectness alone; then the
     // objectness plane is read first and the class planes of dead vectors are never requested.)
-    Vec<VEC> tob, t0[8];
-    const int kn0 = min(8, C);
+    PlaneVec<T, VEC> tob, t0[KB];
+    const int kn0 = min(KB, C);
     bool any_alive = false;
     if (P.sparse) {
         if (inb) tob.load(base + 4 * (size_t)F2);
 #pragma unroll
         for (int v = 0; v < VEC; ++v) {
-            obj[v] = inb ? spec_sigmoidf(tob.v[v]) : 0.0f;
+            obj[v] = inb ? spec_sigmoidf(tob.at(v)) : 0.0f;
             lth[v] = inb ? class_logit_bound(obj[v], thr) : kInf;
             any_alive |= (lth[v] != kInf);
         }
         if (any_alive) {
 #pragma unroll
-            for (int u = 0; u < 8; ++u)
+            for (int u = 0; u < KB; ++u)
                 if (u < kn0) t0[u].load(cp + (size_t)u * F2);
         }
     } else {
         if (inb) {
             tob.load(base + 4 * (size_t)F2);
 #pragma unroll
-            for (int u = 0; u < 8; ++u)
+            for (int u = 0; u < KB; ++u)
                 if (u < kn0) t0[u].load(cp + (size_t)u * F2);
         }
 #pragma unroll
         for (int v = 0; v < VEC; ++v) {
-            obj[v] = inb ? spec_sigmoidf(tob.v[v]) : 0.0f;
+            obj[v] = inb ? spec_sigmoidf(tob.at(v)) : 0.0f;
             lth[v] = inb ? class_logit_bound(obj[v], thr) : kInf;
             any_alive |= (lth[v] != kInf);
         }
+    }
+    unsigned lpk[(VEC + 1) / 2];                                     // 16-bit pairs: the bounds rounded down, packed
+#pragma unroll
+    for (int j = 0; j < (VEC + 1) / 2; ++j) {
+        if constexpr (sizeof(T) == 2 && VEC > 1)
+            lpk[j] = (unsigned)round_down_bits(lth[2 * j], T()) | ((unsigned)round_down_bits(lth[2 * j + 1], T()) << 16);
+        else
+            lpk[j] = 0u;
     }
 #pragma unroll
     for (int v = 0; v < VEC; ++v)
@@ -373,27 +417,21 @@ __device__ __forceinline__ void ldg_stream(const RawParams &P, const RawLayer &L
         for (int w = 0; w < NW; ++w) bits[v][w] = 0u;
     if (any_alive) {
 #pragma unroll
-        for (int u = 0; u < 8; ++u)
-            if (u < kn0) {
-#pragma unroll
-                for (int v = 0; v < VEC; ++v) flag_or(bits[v][0], t0[u].v[v], lth[v], 1u << u);
-            }
+        for (int u = 0; u < KB; ++u)
+            if (u < kn0) flag_plane<T, VEC, NW>(bits, 0, t0[u], lth, lpk, 1u << u);
 #pragma unroll
         for (int w = 0; w < NW; ++w) {
             const int kn = min(32, C - 32 * w);
 #pragma unroll
-            for (int kk = (w == 0 ? 8 : 0); kk < 32; kk += 8) {      // fully unrolled: every bit mask is an immediate
+            for (int kk = (w == 0 ? KB : 0); kk < 32; kk += KB) {    // fully unrolled: every bit mask is an immediate
                 if (kk < kn) {
-                    Vec<VEC> t[8];
+                    PlaneVec<T, VEC> t[KB];
 #pragma unroll
-                    for (int u = 0; u < 8; ++u)
+                    for (int u = 0; u < KB; ++u)
                         if (kk + u < kn) t[u].load(cp + (size_t)(32 * w + kk + u) * F2);
 #pragma unroll
-                    for (int u = 0; u < 8; ++u)
-                        if (kk + u < kn) {
-#pragma unroll
-                            for (int v = 0; v < VEC; ++v) flag_or(bits[v][w], t[u].v[v], lth[v], 1u << (kk + u));
-                        }
+                    for (int u = 0; u < KB; ++u)
+                        if (kk + u < kn) flag_plane<T, VEC, NW>(bits, w, t[u], lth, lpk, 1u << (kk + u));
                 }
             }
         }
@@ -410,14 +448,14 @@ __device__ __forceinline__ void ldg_stream(const RawParams &P, const RawLayer &L
 // The streaming kernel does nothing but load, compare and store 16 bytes per box (flag words + sigmoid(objectness)),
 // so it runs at the memory system's pace; k_emit_flagged then resolves the flagged pairs.
 // ---------------------------------------------------------------------------------------------------------------
-template <int VEC, int NW>
+template <typename T, int VEC, int NW>
 __device__ __forceinline__ void flag_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba)
 {
     const int p0 = (tile * K1_THREADS + threadIdx.x) * VEC;
     if (p0 >= Ly.F2) return;                                         // F2 % VEC == 0: a vector is all in or all out
     float obj[VEC], lth[VEC];
     unsigned bits[VEC][NW];
-    ldg_stream<VEC, NW>(P, Ly, ba, p0, true, obj, lth, bits);
+    ldg_stream<T, VEC, NW>(P, Ly, ba, p0, true, obj, lth, bits);
     const int b = ba / 3, a = ba - 3 * b;
     const size_t r = (size_t)b * P.M4 + (Ly.row_off + a * Ly.F2 + p0);
     // the emit kernel reads these 16 B per box right after this kernel: keep them in L2 while the raw stream passes through
@@ -437,7 +475,7 @@ __device__ __forceinline__ void flag_tile(const RawParams &P, const RawLayer &Ly
 #ifndef YL_FLAG_MINB
 #define YL_FLAG_MINB 8
 #endif
-template <int NW>
+template <typename T, int NW>
 __global__ void __launch_bounds__(K1_THREADS, YL_FLAG_MINB)
 k_flag_raw(const __grid_constant__ RawParams P)
 {
@@ -451,11 +489,11 @@ k_flag_raw(const __grid_constant__ RawParams P)
     int tile = blockIdx.x;
     int l = 0;
     while (l < P.n_layers - 1 && tile >= P.layer[l].tiles) { tile -= P.layer[l].tiles; ++l; }
-    if (P.layer[l].vec == 4) flag_tile<4, NW>(P, P.layer[l], tile, ba);
-    else flag_tile<1, NW>(P, P.layer[l], tile, ba);
+    if (P.layer[l].vec == 4) flag_tile<T, 4, NW>(P, P.layer[l], tile, ba);
+    else flag_tile<T, 1, NW>(P, P.layer[l], tile, ba);
 }
 
-template <int VEC, int NW>
+template <typename T, int VEC, int NW>
 __device__ __forceinline__ void emit_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba, LdgSmem &sm)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -491,13 +529,13 @@ __device__ __forceinline__ void emit_tile(const RawParams &P, const RawLayer &Ly
     if (!__any_sync(0xFFFFFFFFu, any != 0u)) return;                 // warp-uniform: nothing flagged in these 32*VEC boxes
     if (VEC == 4) *reinterpret_cast<float4 *>(&sm.sobj[warp][lane * 4]) = o;
     else sm.sobj[warp][lane] = o.x;
-    emit_pairs<VEC, NW>(P, Ly, ba, (tile * K1_THREADS + warp * 32) * VEC, lth, bits, sm.e[warp], sm.sobj[warp]);
+    emit_pairs<T, VEC, NW>(P, Ly, ba, (tile * K1_THREADS + warp * 32) * VEC, lth, bits, sm.e[warp], sm.sobj[warp]);
 }
 
 #ifndef YL_EMIT_MINB
 #define YL_EMIT_MINB 8
 #endif
-template <int NW>
+template <typename T, int NW>
 __global__ void __launch_bounds__(K1_THREADS, YL_EMIT_MINB)
 k_emit_flagged(const __grid_constant__ RawParams P)
 {
@@ -510,8 +548,8 @@ k_emit_flagged(const __grid_constant__ RawParams P)
     int tile = (int)gridDim.x - 1 - (int)blockIdx.x;
     int l = 0;
     while (l < P.n_layers - 1 && tile >= P.layer[l].tiles) { tile -= P.layer[l].tiles; ++l; }
-    if (P.layer[l].vec == 4) emit_tile<4, NW>(P, P.layer[l], tile, ba, sm);
-    else emit_tile<1, NW>(P, P.layer[l], tile, ba, sm);
+    if (P.layer[l].vec == 4) emit_tile<T, 4, NW>(P, P.layer[l], tile, ba, sm);
+    else emit_tile<T, 1, NW>(P, P.layer[l], tile, ba, sm);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -617,7 +655,7 @@ __device__ __forceinline__ WtTile ft_tile(const RawParams &P, int t, int nba, in
             T.ba = P.img_first * 3 + bal;
             T.p0 = tx * P.layer[l].tile_boxes;
             T.np = min(P.layer[l].tile_boxes, P.layer[l].F2 - T.p0);
-            T.src = P.layer[l].raw + ((size_t)T.ba * (5 + P.C)) * P.layer[l].F2 + T.p0;
+            T.src = (const float *)P.layer[l].raw + ((size_t)T.ba * (5 + P.C)) * P.layer[l].F2 + T.p0;
             T.row0 = T.ba * (5 + P.C) + 5;
             return T;
         }
@@ -764,7 +802,7 @@ k_flag_tma(const __grid_constant__ RawParams P, const __grid_constant__ TmaMaps 
             float obj1[1], lth1[1];
             unsigned bits1[1][NW];
             const bool inb = lane < T.np;
-            ldg_stream<1, NW>(P, Ly, T.ba, T.p0 + lane, inb, obj1, lth1, bits1);
+            ldg_stream<float, 1, NW>(P, Ly, T.ba, T.p0 + lane, inb, obj1, lth1, bits1);
             if (inb) {
                 const int b = T.ba / 3, a = T.ba - 3 * b;
                 const size_t r = (size_t)b * P.M4 + (Ly.row_off + a * Ly.F2 + T.p0 + lane);
@@ -1049,11 +1087,39 @@ extern "C" int yl_post_reset(void *ws, size_t ws_bytes, int B, long M, int C, in
     return YL_OK;
 }
 
-static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, int B, int C,
+// The register-staged flag kernel (unless the caller has already streamed the scales with k_flag_tma) and the emit kernel for
+// element type T.
+template <typename T>
+static int launch_flag_emit(const RawParams &P, dim3 grid, bool flag, bool emit, bool pdl, int NW, cudaStream_t st)
+{
+    if (flag) {
+        switch (NW) {
+        case 1: k_flag_raw<T, 1><<<grid, K1_THREADS, 0, st>>>(P); break;
+        case 2: k_flag_raw<T, 2><<<grid, K1_THREADS, 0, st>>>(P); break;
+        case 3: k_flag_raw<T, 3><<<grid, K1_THREADS, 0, st>>>(P); break;
+        default: k_flag_raw<T, 4><<<grid, K1_THREADS, 0, st>>>(P); break;
+        }
+        YL_LAUNCH_CHECK();
+    }
+    if (emit) {
+        cudaError_t le;
+        switch (NW) {
+        case 1: le = launch_after(k_emit_flagged<T, 1>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
+        case 2: le = launch_after(k_emit_flagged<T, 2>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
+        case 3: le = launch_after(k_emit_flagged<T, 3>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
+        default: le = launch_after(k_emit_flagged<T, 4>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
+        }
+        if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
+    }
+    return YL_OK;
+}
+
+static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
                            const float *anchors_px, const int *anchor_mask, float conf_thre,
                            void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                            yl_stream_t stream, int stages)
 {
+    if (dtype != YL_DTYPE_F32 && dtype != YL_DTYPE_F16 && dtype != YL_DTYPE_BF16) return YL_ERR_ARG;
     if (!raw || !F || !anchors_px || !anchor_mask || !ws) return YL_ERR_ARG;
     if (n_layers < 1 || n_layers > 3 || B <= 0 || C <= 0 || cap_seg <= 0) return YL_ERR_ARG;
     if (img_first < 0 || img_count < 0 || img_first + img_count > B) return YL_ERR_ARG;
@@ -1081,8 +1147,9 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
     int row_off = 0, n_tma = 0;
     const int n_cc = (C + WT_KC - 1) / WT_KC;
     // the TMA flag kernel streams every plane of every box; with a high threshold the register-staged kernel's objectness-first
-    // mode skips most class planes instead
-    const bool flag_tma = g_flag_tma && !base.sparse;
+    // mode skips most class planes instead.  It has an fp32 form only.
+    const bool f32 = dtype == YL_DTYPE_F32;
+    const bool flag_tma = g_flag_tma && !base.sparse && f32;
     for (int l = 0; l < n_layers; ++l) {
         RawLayer &Ly = lay[l];
         Ly.raw = raw[l]; Ly.Fw = F[l]; Ly.F2 = F[l] * F[l]; Ly.row_off = row_off;
@@ -1093,8 +1160,11 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
             Ly.aw[a] = (float)((double)anchors_px[2 * q] / (double)Ly.stride);
             Ly.ah[a] = (float)((double)anchors_px[2 * q + 1] / (double)Ly.stride);
         }
-        // 128-bit loads / bulk copies need 16-byte aligned planes: F^2 % 4 == 0 and an aligned base (19x19, 13x13 fall back)
-        Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 16 == 0)) ? 4 : 1;
+        // 128-bit loads / bulk copies need 16-byte aligned planes: F^2 % 4 == 0 and an aligned base (19x19, 13x13 fall back).
+        // 16-bit planes are read with 64-bit loads where F^2 % 4 == 0 and the base is 8-byte aligned; their tables are then
+        // stored as uint4, so the scale's rows of them must start 16-byte aligned as well.
+        if (f32) Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 16 == 0)) ? 4 : 1;
+        else Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 8 == 0) && row_off % 4 == 0) ? 4 : 1;
         Ly.tma = (Ly.vec == 4 && n_cc >= FT_STAGES) ? 1 : 0;              // k_flag_tma's ring needs FT_STAGES class chunks
         Ly.tile_boxes = 0; Ly.tiles = 0;
         n_tma += Ly.tma;
@@ -1150,7 +1220,7 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
         for (int l = 0; l < Pt.n_layers; ++l) {
             if (Pt.layer[l].tma != 1) continue;
             n_tma_tiles += Pt.layer[l].tiles * nba;
-            const int rc = encode_plane_map(&maps.m[l], Pt.layer[l].raw, Pt.layer[l].F2, (long)B * 3 * (5 + C));
+            const int rc = encode_plane_map(&maps.m[l], (const float *)Pt.layer[l].raw, Pt.layer[l].F2, (long)B * 3 * (5 + C));
             if (rc != YL_OK) return rc;
         }
         const size_t smem = sizeof(FtSmem);
@@ -1168,29 +1238,26 @@ static int filter_raw_impl(const float *const *raw, const int *F, int n_layers, 
         switch (NW) { YL_FT_CASE(1) YL_FT_CASE(2) YL_FT_CASE(3) YL_FT_CASE(4) }
 #undef YL_FT_CASE
         YL_LAUNCH_CHECK();
-    } else if (stages & 1) {
-        switch (NW) {
-        case 1: k_flag_raw<1><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-        case 2: k_flag_raw<2><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-        case 3: k_flag_raw<3><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-        default: k_flag_raw<4><<<grid, K1_THREADS, 0, st>>>(Pl); break;
-        }
-        YL_LAUNCH_CHECK();
     }
 
-    // ---- emit kernel ----
-    if (stages & 2) {
-        const bool pdl = pdl_enabled() && (stages & 1);                     // directly behind the flag kernel on the stream
-        cudaError_t le;
-        switch (NW) {
-        case 1: le = launch_after(k_emit_flagged<1>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-        case 2: le = launch_after(k_emit_flagged<2>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-        case 3: le = launch_after(k_emit_flagged<3>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-        default: le = launch_after(k_emit_flagged<4>, grid, dim3(K1_THREADS), 0, st, pdl, Pl); break;
-        }
-        if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
+    // ---- register-staged flag kernel and emit kernel ----
+    const bool flag_ldg = (stages & 1) && !persistent;
+    const bool pdl = pdl_enabled() && (stages & 1);                         // the emit kernel directly follows the flag kernel
+    switch (dtype) {
+    case YL_DTYPE_F16: return launch_flag_emit<__half>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
+    case YL_DTYPE_BF16: return launch_flag_emit<__nv_bfloat16>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
+    default: return launch_flag_emit<float>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
     }
-    return YL_OK;
+}
+
+extern "C" int yl_filter_raw_typed(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
+                                   const float *anchors_px, const int *anchor_mask, float conf_thre,
+                                   void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
+                                   int stages, yl_stream_t stream)
+{
+    if (stages < 1 || stages > 7 || (stages & 3) == 0) return YL_ERR_ARG;
+    return filter_raw_impl(raw, dtype, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws, ws_bytes, M, cap_seg, img_first,
+                           img_count, stream, stages);
 }
 
 extern "C" int yl_filter_raw(const float *const *raw, const int *F, int n_layers, int B, int C,
@@ -1198,8 +1265,8 @@ extern "C" int yl_filter_raw(const float *const *raw, const int *F, int n_layers
                              void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                              yl_stream_t stream)
 {
-    return filter_raw_impl(raw, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws, ws_bytes, M, cap_seg, img_first,
-                           img_count, stream, 3);
+    return yl_filter_raw_typed((const void *const *)raw, YL_DTYPE_F32, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws,
+                               ws_bytes, M, cap_seg, img_first, img_count, 3, stream);
 }
 
 extern "C" int yl_filter_raw_stage(const float *const *raw, const int *F, int n_layers, int B, int C,
@@ -1207,9 +1274,8 @@ extern "C" int yl_filter_raw_stage(const float *const *raw, const int *F, int n_
                                    void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                                    int stages, yl_stream_t stream)
 {
-    if (stages < 1 || stages > 7 || (stages & 3) == 0) return YL_ERR_ARG;
-    return filter_raw_impl(raw, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws, ws_bytes, M, cap_seg, img_first,
-                           img_count, stream, stages);
+    return yl_filter_raw_typed((const void *const *)raw, YL_DTYPE_F32, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws,
+                               ws_bytes, M, cap_seg, img_first, img_count, stages, stream);
 }
 
 extern "C" int yl_filter_dense(const float *pred, int B, long M, int C, int num_classes, float conf_thre,

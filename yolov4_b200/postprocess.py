@@ -20,6 +20,9 @@ ANCHOR_MASK = [[0, 1, 2], [3, 4, 5], [6, 7, 8]]
 _DEFAULT_CAP_SEG = 1024
 _DEFAULT_CAP_OUT = 16384
 
+# head tensor dtypes of the fused path -> YL_DTYPE_* (include/yolo_head.h)
+_DTYPE_CODES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
 
 def _f32(x):
     """Python-float thresholds are compared in fp32 by torch / NumPy (SURVEY.md 7-4)."""
@@ -153,11 +156,13 @@ def _check_raws(head_outputs, num_classes):
     for r in head_outputs:
         if r.dim() != 4 or r.shape[0] != B or r.shape[1] != 3 * (5 + num_classes) or r.shape[2] != r.shape[3]:
             raise ValueError("head tensor must be [B, 3*(5+C), F, F], got %s" % (tuple(r.shape),))
-        if r.dtype != torch.float32 or not r.is_cuda:
-            raise TypeError("head tensors must be float32 CUDA tensors")
+        if r.dtype not in _DTYPE_CODES or not r.is_cuda:
+            raise TypeError("head tensors must be float32, float16 or bfloat16 CUDA tensors")
+        if r.dtype != head_outputs[0].dtype:
+            raise TypeError("head tensors must share one dtype, got %s and %s" % (head_outputs[0].dtype, r.dtype))
         raws.append(r.contiguous())
         Fs.append(int(r.shape[2]))
-    return raws, B, Fs
+    return raws, B, Fs, _DTYPE_CODES[raws[0].dtype]
 
 
 def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK):
@@ -166,8 +171,14 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     head_outputs: the three raw head conv outputs [B, 3*(5+C), F_l, F_l] (stride 8, 16, 32; yolov4.py:235-251).
     Equivalent to postprocess(torch.cat([YOLOLayer_l(x_l)], 1), num_classes, conf_thre, nms_thre) but reads the
     raw tensors once and never writes the dense decoded tensor.
+
+    The heads may be float32, float16 or bfloat16 (all of one dtype), as a model run with .half() or under
+    torch.autocast produces them.  A 16-bit head is widened exactly to float32 and the float32 computation follows, so
+    the result is bit for bit detect_raw([h.float() for h in head_outputs], ...).  This is not the reference's own
+    half-precision arithmetic, which rounds every sigmoid, exp and product to fp16.  Rows are float32 for every input
+    dtype: this entry is not a reference call surface, and float32 rows are what the exact widening produces.
     """
-    raws, B, Fs = _check_raws(head_outputs, num_classes)
+    raws, B, Fs, dt = _check_raws(head_outputs, num_classes)
     C = int(num_classes)
     M = sum(3 * f * f for f in Fs)
     L = _cabi.lib()
@@ -178,8 +189,8 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     fs = _cabi.ints(Fs)
     with torch.cuda.device(dev):
         def front(ws, cap_seg):
-            _cabi.check(L.yl_filter_raw(rp, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes, M,
-                                        cap_seg, 0, B, _stream()))
+            _cabi.check(L.yl_filter_raw_typed(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes,
+                                              M, cap_seg, 0, B, 3, _stream()))
         rows, mh = _run(front, dev, B, M, C, nms_thre)
     return _split(rows, mh, B, dev, torch.float32)
 
@@ -191,7 +202,8 @@ class HeadPostprocessor:
     device tensors owned by this object (overwritten by the next run).  With n_groups > 1 image groups are pipelined
     over two streams (NMS of group g next to the streaming filter of group g+1); on B200 one group is fastest because
     every kernel already fills the machine.  capture() records the chain into a CUDA graph bound to the given input
-    tensors; replay() launches it.
+    tensors; replay() launches it.  The head tensors may be float32, float16 or bfloat16 (see detect_raw); each run takes
+    the dtype from the tensors it is given.
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
@@ -220,7 +232,7 @@ class HeadPostprocessor:
 
     def run(self, head_outputs):
         L, B, C, M = self.L, self.B, self.C, self.M
-        raws, Bc, Fs = _check_raws(head_outputs, C)      # shape / dtype / device checked, non-contiguous inputs copied
+        raws, Bc, Fs, dt = _check_raws(head_outputs, C)  # shape / dtype / device checked, non-contiguous inputs copied
         if Bc != B or Fs != self.Fs:
             raise ValueError("shape mismatch with the configured postprocessor")
         self._live_inputs = raws                         # a contiguous copy must outlive the enqueued kernels
@@ -233,19 +245,19 @@ class HeadPostprocessor:
         for g in range(G):
             i0, i1 = B * g // G, B * (g + 1) // G
             if fold_reset:
-                _cabi.check(L.yl_filter_raw_stage(rp, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf, self.ws.ptr(),
-                                                  self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7, main.cuda_stream))
+                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
+                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7, main.cuda_stream))
                 self.side.wait_stream(main)
             elif self.mode in ("emit_side", "pipe3"):
                 # streaming flag kernels back to back on the main stream; everything else follows on the side stream
-                _cabi.check(L.yl_filter_raw_stage(rp, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf, self.ws.ptr(),
-                                                  self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 1, main.cuda_stream))
+                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
+                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 1, main.cuda_stream))
                 self.side.wait_stream(main)
-                _cabi.check(L.yl_filter_raw_stage(rp, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf, self.ws.ptr(),
-                                                  self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 2, self.side.cuda_stream))
+                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
+                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 2, self.side.cuda_stream))
             else:
-                _cabi.check(L.yl_filter_raw(rp, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf, self.ws.ptr(),
-                                            self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, main.cuda_stream))
+                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
+                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 3, main.cuda_stream))
                 self.side.wait_stream(main)
             nms_stream = self.side
             if self.mode == "pipe3":
@@ -260,7 +272,7 @@ class HeadPostprocessor:
         return self.rows, self.meta
 
     def capture(self, head_outputs):
-        raws, B, Fs = _check_raws(head_outputs, self.C)
+        raws, B, Fs, _ = _check_raws(head_outputs, self.C)
         if B != self.B or Fs != self.Fs:
             raise ValueError("shape mismatch with the configured postprocessor")
         self._captured_inputs = raws
