@@ -140,6 +140,21 @@ int yl_filter_dense(const float *pred, int B, long M, int C, int num_classes, fl
 int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre,
            float *out_rows, long cap_out, int *meta, int img_first, int img_count, yl_stream_t stream);
 
+/* yl_nms with a per-image detection cap (max_det; the max_det / detections_per_img option of other detectors).  Let K_b be
+ * image b's uncapped row count and s = fl32(obj_conf * cls_conf) (rows' columns 4 x 5, -0 counted as +0).  When K_b > max_det,
+ * the kept rows are the first max_det of a STABLE descending sort of the uncapped rows by s (equal scores keep the uncapped
+ * order: lower class first, then the order inside the class), emitted in the uncapped order (class ascending, score
+ * descending), so every consumer of yl_nms output takes them unchanged.  Within a class the uncapped rows are already in
+ * score order, so the cap keeps a prefix of every (image, class) segment: one extra kernel (k_select_topk, one CTA per
+ * image, radix select of the max_det-th largest score) lowers the per-class counts before the concatenation.
+ *   max_det   0 = no cap (exactly yl_nms: same launches, no extra kernel); 1 <= max_det <= cap_out caps every image;
+ *             anything else returns YL_ERR_ARG before any CUDA call
+ *   meta[b]   = rows written = min(K_b, max_det); meta[B+b], meta[2B+b] as for yl_nms
+ *   uncapped  device int32 [B] receiving K_b for the images of this call, or NULL
+ * The workspace is that of yl_post_workspace_bytes(); yl_nms is this call with max_det = 0 and uncapped = NULL. */
+int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,
+                float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * A6+A7  YOLOLoss.build_target(output, pred, layer_no, labels)      replaces yolo/model/yololoss.py:118-371
  *        (and bboxes_iou, yololoss.py:16-91, which it calls twice per image)
@@ -236,6 +251,11 @@ int yl_context_create_typed(yl_context **ctx, int device, int B, const int *F, i
 int yl_context_destroy(yl_context *ctx);
 int yl_detect_host(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre,
                    float *out_rows_host, int *counts_host);
+/* yl_detect_host with a per-image detection cap (yl_nms_topk): counts_host[b] = min(K_b, max_det) and only those rows are
+ * copied back.  max_det = 0 is no cap (yl_detect_host is this call with 0); 1 <= max_det <= the context's cap_out, anything
+ * else returns YL_ERR_ARG before any CUDA call. */
+int yl_detect_host_topk(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
+                        float *out_rows_host, int *counts_host);
 
 /* ---------------------------------------------------------------------------------------------------------
  * (e) Multi-GPU: the final exchange of the image-sharded path            (SURVEY.md 8(e); no reference counterpart: the

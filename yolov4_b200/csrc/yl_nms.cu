@@ -771,6 +771,150 @@ k_gather_rows(const uint4 *__restrict__ cand, const unsigned *__restrict__ seg_c
     if (tid < (nf & 3u)) dst[4 * nf4 + tid] = src[4 * nf4 + tid];
 }
 
+// ---- per-image detection cap (max_det) -----------------------------------------------------------------------
+// The kept rows of an image are the first max_det of a stable descending sort of its class-ordered rows by
+// s = fl(obj * cls_conf).  Inside a segment the rows are already in that order (score desc, ties by row desc), so the
+// kept set is a prefix of every segment: k_select_topk only lowers kept_count and k_gather_rows copies the prefixes.
+//   1. T = the max_det-th largest score key of the image: MSB-first radix select, SEL_PASSES histogram passes over the
+//      keys (staged in shared memory when the image has at most SEL_SMEM_KEYS rows, otherwise re-read from the rows in
+//      global memory on every pass: the degenerate all-ties images, correctness only);
+//   2. per class, binary searches on the sorted segment give gt_c (keys > T) and eq_c (keys == T); the ties are admitted
+//      in class order: take_c = gt_c + min(eq_c, max(0, need - sum_{c' < c} eq_c')).
+constexpr int SEL_THREADS = 512;
+constexpr int SEL_SMEM_KEYS = 16384;                         // 64 KB of keys: an image at 608 / conf 1e-4 keeps ~11.5k rows
+constexpr int SEL_PASSES = 3;                                // digits of 11, 11 and 10 bits
+constexpr int SEL_BINS = 1 << 11;
+constexpr size_t SEL_SMEM_BYTES = sizeof(unsigned) * SEL_SMEM_KEYS;
+
+// Order-preserving key of the nms score of a finished row; -0 and +0 get the same key.
+__device__ __forceinline__ unsigned row_score_key(const float *row)
+{
+    const float s = __fadd_rn(__fmul_rn(row[4], row[5]), 0.0f);  // the filter kernels' score expression
+    const unsigned u = __float_as_uint(s) == 0x80000000u ? 0u : __float_as_uint(s);
+    return u ^ ((u >> 31) ? 0xFFFFFFFFu : 0x80000000u);
+}
+
+__global__ void __launch_bounds__(SEL_THREADS)
+k_select_topk(const uint4 *__restrict__ cand, unsigned *__restrict__ kept_count, int C, int cap_seg, int max_det,
+              int *__restrict__ uncapped, int img_first)
+{
+    extern __shared__ unsigned sh_keys[];                     // [SEL_SMEM_KEYS], used when the image's rows fit
+    __shared__ unsigned sh_hist[SEL_BINS];
+    __shared__ unsigned sh_pre[YL_MAX_CLASSES + 1];           // exclusive prefix of kept_count over the classes
+    __shared__ unsigned sh_eq[YL_MAX_CLASSES];
+    __shared__ unsigned sh_warp[SEL_THREADS / 32];
+    __shared__ unsigned sh_digit, sh_above;
+    pdl_trigger();
+    pdl_wait();                                                 // kept counts and finished rows of both NMS tiers
+    const int b = img_first + blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float *seg_rows0 = reinterpret_cast<const float *>(cand + (size_t)b * C * cap_seg * 2);
+    const size_t seg_stride = (size_t)cap_seg * 8;             // floats per segment (two uint4 per record)
+    {
+        // exclusive prefix over the classes (C <= 128: the first four warps, one class per lane)
+        const unsigned v = tid < C ? kept_count[b * C + tid] : 0u;
+        unsigned incl = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned u = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+            if (lane >= o) incl += u;
+        }
+        if (lane == 31) sh_warp[warp] = incl;
+        __syncthreads();
+        unsigned off = 0u;
+        for (int w = 0; w < warp && w < YL_MAX_CLASSES / 32; ++w) off += sh_warp[w];
+        if (tid < C) sh_pre[tid] = off + incl - v;
+        if (tid == C - 1) sh_pre[C] = off + incl;
+        __syncthreads();
+    }
+    const unsigned n = sh_pre[C];
+    if (tid == 0 && uncapped) uncapped[b] = (int)n;
+    if (n <= (unsigned)max_det) return;                         // CTA-uniform
+
+    // key of the image's i-th row in class order
+    auto global_key = [&](unsigned i) -> unsigned {
+        int lo = 0, hi = C;                                     // largest c with sh_pre[c] <= i
+        while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sh_pre[mid] <= i) lo = mid; else hi = mid; }
+        return row_score_key(seg_rows0 + (size_t)lo * seg_stride + (size_t)(i - sh_pre[lo]) * 7);
+    };
+    const bool staged = n <= (unsigned)SEL_SMEM_KEYS;
+    if (staged) {
+        for (unsigned i = tid; i < n; i += SEL_THREADS) sh_keys[i] = global_key(i);
+    }
+
+    // ---- 1. radix select: prefix / mask describe the digits of T fixed so far, need = rows still to take at >= prefix ----
+    unsigned prefix = 0u, mask = 0u, need = (unsigned)max_det;
+    int shift = 32;
+#pragma unroll 1
+    for (int p = 0; p < SEL_PASSES; ++p) {
+        const int bits = p < 2 ? 11 : 10;
+        shift -= bits;
+        const unsigned dmask = (1u << bits) - 1u;
+        for (int i = tid; i < SEL_BINS; i += SEL_THREADS) sh_hist[i] = 0u;
+        __syncthreads();
+        for (unsigned i = tid; i < n; i += SEL_THREADS) {
+            const unsigned k = staged ? sh_keys[i] : global_key(i);
+            if ((k & mask) == prefix) atomicAdd(&sh_hist[(k >> shift) & dmask], 1u);
+        }
+        __syncthreads();
+        // the digit d where the count of keys with a larger digit is < need <= the count at >= d: a suffix sum over the bins,
+        // each thread owning a run of SEL_BINS / SEL_THREADS bins from the top
+        constexpr int RUN = SEL_BINS / SEL_THREADS;
+        const int top = (int)dmask - RUN * tid;                 // this thread's bins: top, top-1, .., top-RUN+1
+        unsigned run = 0u;
+#pragma unroll
+        for (int k = 0; k < RUN; ++k) if (top - k >= 0) run += sh_hist[top - k];
+        unsigned incl = run;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+            if (lane >= o) incl += v;
+        }
+        if (lane == 31) sh_warp[warp] = incl;
+        __syncthreads();
+        unsigned above = 0u;                                    // keys in the bins above this thread's run
+        for (int w = 0; w < warp; ++w) above += sh_warp[w];
+        above += incl - run;
+        if (above < need && above + run >= need) {              // exactly one thread
+            unsigned a = above;
+            for (int k = 0; k < RUN; ++k) {
+                const unsigned h = sh_hist[top - k];
+                if (a + h >= need) { sh_digit = (unsigned)(top - k); sh_above = a; break; }
+                a += h;
+            }
+        }
+        __syncthreads();
+        prefix |= sh_digit << shift;
+        mask |= dmask << shift;
+        need -= sh_above;
+        __syncthreads();                                        // sh_digit / sh_above / sh_hist are rewritten next pass
+    }
+    const unsigned T = prefix;                                  // need (>= 1) of the keys equal to T are taken
+
+    // ---- 2. per class: gt_c, eq_c by binary search on the descending keys of the segment's kept rows ----
+    unsigned gt = 0u, eq = 0u;
+    const int c = tid;
+    if (c < C) {
+        const unsigned base = sh_pre[c], cnt = sh_pre[c + 1] - base;
+        auto key_at = [&](unsigned j) -> unsigned {
+            return staged ? sh_keys[base + j] : row_score_key(seg_rows0 + (size_t)c * seg_stride + (size_t)j * 7);
+        };
+        unsigned lo = 0u, hi = cnt;                             // first j with key <= T
+        while (lo < hi) { const unsigned mid = (lo + hi) >> 1; if (key_at(mid) > T) lo = mid + 1u; else hi = mid; }
+        gt = lo;
+        hi = cnt;                                               // first j with key < T
+        while (lo < hi) { const unsigned mid = (lo + hi) >> 1; if (key_at(mid) >= T) lo = mid + 1u; else hi = mid; }
+        eq = lo - gt;
+        sh_eq[c] = eq;
+    }
+    __syncthreads();
+    if (c < C) {
+        unsigned before = 0u;
+        for (int k = 0; k < c; ++k) before += sh_eq[k];
+        const unsigned ties = need > before ? min(eq, need - before) : 0u;
+        kept_count[b * C + c] = gt + ties;
+    }
+}
+
 // Smallest K such that two positive areas whose bins (float bits >> 21: four per octave) differ by at least K have a
 // ratio above 1/(0.999 thr) * (1 + 1e-3): then IoU <= amin/amax < thr with a margin far above fp32 rounding, which is
 // the condition under which suppresses_pos returns false on the area test alone.
@@ -795,11 +939,12 @@ static int area_bin_gap(float thr)
 
 using namespace yl;
 
-extern "C" int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre,
-                      float *out_rows, long cap_out, int *meta, int img_first, int img_count, yl_stream_t stream)
+extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,
+                           float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
 {
     if (!ws || !out_rows || !meta || B <= 0 || M <= 0 || C <= 0 || cap_seg <= 0 || cap_out <= 0) return YL_ERR_ARG;
     if (img_first < 0 || img_count < 0 || img_first + img_count > B) return YL_ERR_ARG;
+    if (max_det < 0 || max_det > cap_out) return YL_ERR_ARG;
     if (C > YL_MAX_CLASSES) return YL_ERR_CLASSES;
     const PostLayout L = post_layout(B, M, C, cap_seg);
     if (ws_bytes < L.total) return YL_ERR_WORKSPACE;
@@ -821,7 +966,19 @@ extern "C" int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_s
     const int grid_big = nseg < 148 * 2 ? nseg : 148 * 2;
     YL_CUDA_TRY(launch_after(k_segment_nms_big, dim3(grid_big), dim3(NMS_THREADS), 0, st, pdl, cand, (const unsigned *)seg_count, kept_count,
                              C, cap_seg, nms_thre, (const unsigned *)big_count, (const unsigned *)big_list, kept_scratch));
+    if (max_det > 0) {
+        // per device, so set on every call (a host-side attribute: allowed during stream capture)
+        YL_CUDA_TRY(cudaFuncSetAttribute(k_select_topk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SEL_SMEM_BYTES));
+        YL_CUDA_TRY(launch_after(k_select_topk, dim3(img_count), dim3(SEL_THREADS), SEL_SMEM_BYTES, st, pdl, (const uint4 *)cand,
+                                 kept_count, C, cap_seg, max_det, uncapped, img_first));
+    }
     YL_CUDA_TRY(launch_after(k_gather_rows, dim3(nseg), dim3(GATHER_THREADS), 0, st, pdl, (const uint4 *)cand, (const unsigned *)seg_count,
                              (const unsigned *)kept_count, C, cap_seg, B, out_rows, cap_out, meta, seg_first));
     return YL_OK;
+}
+
+extern "C" int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre,
+                      float *out_rows, long cap_out, int *meta, int img_first, int img_count, yl_stream_t stream)
+{
+    return yl_nms_topk(ws, ws_bytes, B, M, C, cap_seg, nms_thre, 0, out_rows, cap_out, meta, nullptr, img_first, img_count, stream);
 }

@@ -71,6 +71,19 @@ class _Workspace:
 _cap_hint = {}    # (B, M, C) -> (cap_seg, cap_out) that were last sufficient
 
 
+def _check_max_det(max_det):
+    """None (no cap) or an int >= 1; checked before any CUDA work."""
+    if max_det is None:
+        return None
+    if isinstance(max_det, bool) or not isinstance(max_det, (int, np.integer)) or int(max_det) < 1:
+        raise ValueError("max_det must be None or an int >= 1, got %r" % (max_det,))
+    return int(max_det)
+
+
+def _round4(n):
+    return (n + 3) // 4 * 4
+
+
 def _split(rows, meta_host, B, out_device, out_dtype):
     out = []
     for b in range(B):
@@ -85,10 +98,15 @@ def _split(rows, meta_host, B, out_device, out_dtype):
     return out
 
 
-def _run(front_end, device, B, M, C, nms_thre):
-    """Runs front end + NMS, growing cap_seg / cap_out and re-running when the device reports an overflow."""
+def _run(front_end, device, B, M, C, nms_thre, max_det=None):
+    """Runs front end + NMS, growing cap_seg / cap_out and re-running when the device reports an overflow.  With a cap the
+    output holds max_det rows per image (rounded up to a multiple of 4), which no image can exceed; the capacities a capped
+    call settles on are kept apart from those of uncapped calls."""
     L = _cabi.lib()
-    cap_seg, cap_out = _cap_hint.get((B, M, C), (_DEFAULT_CAP_SEG, _DEFAULT_CAP_OUT))
+    hint_key = (B, M, C) if max_det is None else (B, M, C, max_det)
+    cap_seg, cap_out = _cap_hint.get(hint_key, (_DEFAULT_CAP_SEG, _DEFAULT_CAP_OUT))
+    if max_det is not None:
+        cap_out = _round4(max_det)
     cap_seg = min(cap_seg, _next_pow2(M))
     while True:
         ws = _Workspace.get(device, B, M, C, cap_seg)
@@ -96,22 +114,23 @@ def _run(front_end, device, B, M, C, nms_thre):
         meta = torch.empty((3 * B,), dtype=torch.int32, device=device)
         _cabi.check(L.yl_post_reset(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _stream()))
         front_end(ws, cap_seg)
-        _cabi.check(L.yl_nms(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), rows.data_ptr(), cap_out,
-                             meta.data_ptr(), 0, B, _stream()))
+        _cabi.check(L.yl_nms_topk(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), max_det or 0, rows.data_ptr(), cap_out,
+                                  meta.data_ptr(), None, 0, B, _stream()))
         mh = meta.cpu().numpy()                      # the one D2H sync the list-of-tensors contract requires
         max_seg, max_rows = int(mh[B:2 * B].max()), int(mh[:B].max())
         if max_seg > cap_seg:
             cap_seg = _next_pow2(max_seg)
-            cap_out = max(cap_out, _next_pow2(int(mh[2 * B:].max())))
+            if max_det is None:
+                cap_out = max(cap_out, _next_pow2(int(mh[2 * B:].max())))
             continue
         if max_rows > cap_out:
             cap_out = _next_pow2(max_rows)
             continue
-        _cap_hint[(B, M, C)] = (cap_seg, cap_out)
+        _cap_hint[hint_key] = (cap_seg, cap_out)
         return rows, mh
 
 
-def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45):
+def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_det=None):
     """Same contract as the reference's postprocess (yolo/util/utils.py:92).
 
     prediction: [B, M, 5+C] decoded (cx, cy, w, h, obj, cls...), fp32, on a CUDA device (a CPU tensor, as
@@ -121,7 +140,10 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45):
     Differences from the reference, none observable by its callers: `prediction[:, :, :4]` is not overwritten
     in place with the corner form (utils.py:126), and score ties are ordered (score desc, box index desc),
     the order of a stable argsort, where NumPy's default sort leaves them unspecified (utils.py:58).
+    max_det (keyword only, not part of the reference signature): keep at most this many detections per image, those with the
+    highest obj_conf * cls_conf (equal scores keep the order above), still listed classes ascending then score descending.
     """
+    max_det = _check_max_det(max_det)
     if prediction.dim() != 3 or prediction.shape[2] < 6:
         raise ValueError("prediction must be [B, M, 5+C]")
     if prediction.dtype != torch.float32:
@@ -139,7 +161,7 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45):
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_dense(pred.data_ptr(), B, M, C, num_classes, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                           cap_seg, 0, B, _stream()))
-        rows, mh = _run(front, pred.device, B, M, C, nms_thre)
+        rows, mh = _run(front, pred.device, B, M, C, nms_thre, max_det)
     return _split(rows, mh, B, in_device, prediction.dtype)
 
 
@@ -165,7 +187,7 @@ def _check_raws(head_outputs, num_classes):
     return raws, B, Fs, _DTYPE_CODES[raws[0].dtype]
 
 
-def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK):
+def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None):
     """Fused YOLOLayer eval decode (yololayer.py:88-166) + postprocess (utils.py:92-223).
 
     head_outputs: the three raw head conv outputs [B, 3*(5+C), F_l, F_l] (stride 8, 16, 32; yolov4.py:235-251).
@@ -177,7 +199,12 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     the result is bit for bit detect_raw([h.float() for h in head_outputs], ...).  This is not the reference's own
     half-precision arithmetic, which rounds every sigmoid, exp and product to fp16.  Rows are float32 for every input
     dtype: this entry is not a reference call surface, and float32 rows are what the exact widening produces.
+
+    max_det: keep at most this many detections per image, those with the highest obj_conf * cls_conf; ties keep the
+    uncapped order (lower class first, then the order inside the class).  The kept rows stay in the uncapped order, classes
+    ascending then score descending.  None (the default) keeps every detection.
     """
+    max_det = _check_max_det(max_det)
     raws, B, Fs, dt = _check_raws(head_outputs, num_classes)
     C = int(num_classes)
     M = sum(3 * f * f for f in Fs)
@@ -191,7 +218,7 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_raw_typed(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                               M, cap_seg, 0, B, 3, _stream()))
-        rows, mh = _run(front, dev, B, M, C, nms_thre)
+        rows, mh = _run(front, dev, B, M, C, nms_thre, max_det)
     return _split(rows, mh, B, dev, torch.float32)
 
 
@@ -204,11 +231,21 @@ class HeadPostprocessor:
     every kernel already fills the machine.  capture() records the chain into a CUDA graph bound to the given input
     tensors; replay() launches it.  The head tensors may be float32, float16 or bfloat16 (see detect_raw); each run takes
     the dtype from the tensors it is given.
+
+    max_det caps the detections of every image as in detect_raw; cap_out then defaults to max_det rounded up to a multiple
+    of 4, so the output (and a DetectionExchange built with hp.cap_out) is sized by the cap.  uncapped is a device int32 [B]
+    with every image's uncapped count, refreshed by every run and replay: meta[b] < uncapped[b] means image b was capped.
+    Without a cap uncapped is the view meta[:B].
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
-                 cap_out=_DEFAULT_CAP_OUT, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, side_priority=0,
-                 mode="nms_side"):
+                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, side_priority=0,
+                 mode="nms_side", max_det=None):
+        self.max_det = _check_max_det(max_det)
+        if cap_out is None:
+            cap_out = _DEFAULT_CAP_OUT if self.max_det is None else _round4(self.max_det)
+        if self.max_det is not None and self.max_det > int(cap_out):
+            raise ValueError("max_det %d exceeds cap_out %d" % (self.max_det, int(cap_out)))
         self.L = _cabi.lib()
         self.device = torch.device(device if device is not None else "cuda")
         self.B, self.Fs, self.C = int(batch), [int(f) for f in grid_sizes], int(num_classes)
@@ -223,6 +260,7 @@ class HeadPostprocessor:
             self.ws = _Workspace(self.device, self.B, self.M, self.C, self.cap_seg)
             self.rows = torch.empty((self.B, self.cap_out, 7), dtype=torch.float32, device=self.device)
             self.meta = torch.zeros((3 * self.B,), dtype=torch.int32, device=self.device)
+            self.uncapped = self.meta[:self.B] if self.max_det is None else torch.zeros((self.B,), dtype=torch.int32, device=self.device)
             self.side = torch.cuda.Stream(device=self.device, priority=side_priority)
             self.side2 = torch.cuda.Stream(device=self.device, priority=side_priority)
         self.mode = mode
@@ -264,8 +302,9 @@ class HeadPostprocessor:
                 # three-deep: flag(g+1) on the main stream, emit(g) on the first side stream, NMS + gather(g-1) on the second
                 self.side2.wait_stream(self.side)
                 nms_stream = self.side2
-            _cabi.check(L.yl_nms(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.rows.data_ptr(),
-                                 self.cap_out, self.meta.data_ptr(), i0, i1 - i0, nms_stream.cuda_stream))
+            _cabi.check(L.yl_nms_topk(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
+                                      self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
+                                      None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, nms_stream.cuda_stream))
         main.wait_stream(self.side)
         if self.mode == "pipe3":
             main.wait_stream(self.side2)
