@@ -155,6 +155,27 @@ int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float n
 int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,
                 float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream);
 
+/* yl_nms_topk with class-agnostic NMS (the agnostic / --agnostic-nms option of other YOLO code bases).  The candidates of an
+ * image are the (box, class) pairs of the filter, unchanged; s = fl32(obj_conf * cls_conf), -0 counted as +0.
+ *   order        s descending, then class ascending, then box row descending (the stable descending sort by s of the
+ *                class-ascending concatenation of the per-class orders: the tie rule of max_det)
+ *   suppression  walking that order, a candidate is dropped when IoU >= nms_thre (the literal NaN-propagating formula of
+ *                utils.py:71-77) with any earlier kept candidate, whatever either class is
+ *   output       the kept candidates as ordinary rows, classes ascending, then s descending, then row descending; max_det then
+ *                caps the agnostic rows as stated for yl_nms_topk
+ * So a box keeps at most one label, its best-scoring passing class -- except a degenerate box (NaN, zero or negative extent,
+ * overflowing area), whose self-IoU is below nms_thre: it keeps every copy, as the literal algorithm does.
+ *   agnostic   0 = yl_nms_topk (same launches, same bytes); 1 = class-agnostic; anything else returns YL_ERR_ARG before any
+ *              CUDA call.  With 1, ws must hold yl_post_workspace_bytes_ex(B, M, C, cap_seg, 1) bytes, M < 2^25 and
+ *              C * cap_seg < 2^32 (else YL_ERR_ARG).  meta[b] is the agnostic row count (capped by max_det), meta[B+b] and
+ *              meta[2B+b] are as for yl_nms; uncapped receives the agnostic count before the cap.
+ * Image groups (img_first / img_count) use only their own images' slices of the workspace. */
+int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
+              float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream);
+/* Workspace bytes for yl_nms_ex: agnostic = 0 is yl_post_workspace_bytes(); 1 adds 8 bytes per candidate slot
+ * (B * C * cap_seg) of scratch for images whose survivors exceed shared memory; anything else returns 0. */
+size_t yl_post_workspace_bytes_ex(int B, long M, int C, int cap_seg, int agnostic);
+
 /* ---------------------------------------------------------------------------------------------------------
  * A6+A7  YOLOLoss.build_target(output, pred, layer_no, labels)      replaces yolo/model/yololoss.py:118-371
  *        (and bboxes_iou, yololoss.py:16-91, which it calls twice per image)
@@ -256,6 +277,11 @@ int yl_detect_host(yl_context *ctx, const float *const *raw_host, float conf_thr
  * else returns YL_ERR_ARG before any CUDA call. */
 int yl_detect_host_topk(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
                         float *out_rows_host, int *counts_host);
+/* yl_detect_host_topk with class-agnostic NMS (yl_nms_ex): agnostic = 0 is yl_detect_host_topk, 1 is class-agnostic, anything
+ * else returns YL_ERR_ARG before any CUDA call.  The first agnostic call enlarges the context's workspace to
+ * yl_post_workspace_bytes_ex(..., 1). */
+int yl_detect_host_ex(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det, int agnostic,
+                      float *out_rows_host, int *counts_host);
 
 /* ---------------------------------------------------------------------------------------------------------
  * (e) Multi-GPU: the final exchange of the image-sharded path            (SURVEY.md 8(e); no reference counterpart: the

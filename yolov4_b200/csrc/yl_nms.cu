@@ -9,6 +9,8 @@
 //                       shared memory (<= SMEM_R) or in place in global memory (degenerate all-ties inputs, SURVEY 7-2).
 //   k_gather_rows       class-ascending concatenation of the kept rows of an image [utils.py:191-220] into
 //                       out_rows[b] = (x1,y1,x2,y2,obj,cls_conf,cls) and the per-image counts.
+//   k_select_topk       per-image detection cap (max_det), between the NMS tiers and the gather.
+//   k_segment_nms_agnostic  class-agnostic NMS, one CTA per image, in place of the two NMS tiers (yl_nms_ex).
 //
 // Candidate record (written by the filter kernels, yl_filter.cu): two uint4,
 //   A = {score bits, box row, cls_conf bits, obj_conf bits}    B = {x1, y1, x2, y2}
@@ -553,19 +555,19 @@ struct GlobalStore {
 
 // Bitonic network in the "flip" formulation: every compare-exchange orders ascending, so virtual +inf padding
 // beyond n never moves and non-power-of-two n works by skipping out-of-range partners.
-template <class Store>
+template <class Store, int NT = NMS_THREADS>
 __device__ void bitonic_sort(Store &s, int n)
 {
     int P = 1;
     while (P < n) P <<= 1;
     for (int k = 2; k <= P; k <<= 1) {
-        for (int i = threadIdx.x; i < n; i += NMS_THREADS) {
+        for (int i = threadIdx.x; i < n; i += NT) {
             const int l = i ^ (k - 1);
             if (l > i && l < n) s.cswap(i, l);
         }
         __syncthreads();
         for (int j = k >> 2; j > 0; j >>= 1) {
-            for (int i = threadIdx.x; i < n; i += NMS_THREADS) {
+            for (int i = threadIdx.x; i < n; i += NT) {
                 const int l = i ^ j;
                 if (l > i && l < n) s.cswap(i, l);
             }
@@ -580,7 +582,7 @@ __device__ void bitonic_sort(Store &s, int n)
 //   (3) warp 0 resolves the chunk serially with the rows in registers
 //   (4) survivors are appended to the kept list (compacted in place: a kept box never moves to a higher index)
 // kept_of[q] = sorted position of the q-th kept box.  Returns the number kept.
-template <bool POS, class Store>
+template <bool POS, class Store, int NT = NMS_THREADS>
 __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, unsigned *kept_g,
                           unsigned *sh_supp /*[2]*/, unsigned long long *sh_rows /*[64]*/, int *sh_nk)
 {
@@ -600,7 +602,7 @@ __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, un
                 const float4 bi = s.get_box(c0 + i);
                 const float ai = s.get_area(c0 + i);
                 bool dead = false;
-                for (int q = tid / CHUNK; q < nk && !dead; q += NMS_THREADS / CHUNK) {
+                for (int q = tid / CHUNK; q < nk && !dead; q += NT / CHUNK) {
                     const int kq = kept_s ? (int)kept_s[q] : (int)kept_g[q];
                     const float4 bk = s.get_box(kq);
                     const float ak = s.get_area(kq);
@@ -610,7 +612,7 @@ __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, un
             }
         }
         // (2) intra-chunk rows: row i has bit j set (j > i) when i suppresses j
-        for (int pr = tid; pr < CHUNK * CHUNK; pr += NMS_THREADS) {
+        for (int pr = tid; pr < CHUNK * CHUNK; pr += NT) {
             const int i = pr / CHUNK, j = pr - i * CHUNK;
             if (j > i && j < cn) {
                 const float4 bi = s.get_box(c0 + i), bj = s.get_box(c0 + j);
@@ -915,6 +917,280 @@ k_select_topk(const uint4 *__restrict__ cand, unsigned *__restrict__ kept_count,
     }
 }
 
+// ---- class-agnostic NMS ----------------------------------------------------------------------------------------------
+// One greedy NMS per image over all its (box, class) candidates, in the image-wide order s desc, class asc, box row desc
+// (the stable descending sort by s of the class-ascending concatenation of the per-class orders); a candidate is dropped when
+// IoU >= thr with any earlier kept candidate, whatever either class is.  Only the FIRST copy of a box (its earliest candidate
+// in that order) can matter when the literal self-IoU of the box is >= thr: a kept first copy suppresses the later copies,
+// and a kept box that suppresses the first copy suppresses every later copy with the same bits.  So the image is reduced to
+// first copies, plus every copy of a box whose self-IoU is below thr (NaN, empty or overflowing boxes, thr > 1), before the
+// greedy pass.  k_segment_nms_agnostic (one CTA per image) replaces k_segment_nms_bins + k_segment_nms_big and leaves the
+// workspace as they do: each class's kept rows at the front of its segment, kept_count written for every class.
+//   1. first copies: a per-box table indexed by box row, in the image's slices of the obj / flag tables (dead once the emit or
+//      dense filter kernel has run): tab_key[row] = min score key (atomicMin), then tab_cls[row] = lowest class at that key;
+//   2. survivors are staged in shared memory (<= AGN_CAP) as (64-bit image-wide key, box, cls_conf / obj_conf), bitonic
+//      sorted and suppressed with the chunked greedy_nms; each kept survivor's row goes to its rank within its class;
+//   3. more survivors than AGN_CAP (conf <= 0, very large inputs): the same algorithm in global memory.  Every segment is
+//      sorted in place, a survivor's image-wide rank is found by binary searches in the other segments, greedy_nms runs
+//      over that order (order / kept lists in the agnostic scratch of yl_post_workspace_bytes_ex), and each segment's kept
+//      records are compacted in place into rows (a row is shorter than a record and lands at or before its record).
+constexpr int AGN_THREADS = 512;
+constexpr int AGN_CAP = 4096;                                 // survivors staged in shared memory
+constexpr int AGN_ROW_BITS = 25;                              // box rows < 2^25; the class takes the 7 bits above them
+constexpr size_t AGN_SMEM_BYTES = (size_t)AGN_CAP * (sizeof(unsigned long long) + sizeof(float4) + sizeof(uint2) + 2 * sizeof(unsigned short));
+static_assert(YL_MAX_CLASSES <= (1 << (32 - AGN_ROW_BITS)), "the class must fit above the row in the low key word");
+
+// Image-wide ascending key: (score desc, class asc, row desc).
+__device__ __forceinline__ unsigned long long agn_key(unsigned score_bits, int c, unsigned row)
+{
+    return ((unsigned long long)score_desc_bits(score_bits) << 32) | ((unsigned)c << AGN_ROW_BITS) |
+           (~row & ((1u << AGN_ROW_BITS) - 1u));
+}
+
+// Survivors in global memory, in image-wide order: order[i] = c * cap_seg + e, the record's offset in the image's segments.
+struct MergedStore {
+    const uint4 *img;          // the image's first segment
+    const unsigned *order;
+    bool pos;
+    __device__ __forceinline__ float4 get_box(int i) const
+    {
+        const float4 b = as_float4(img[2 * (size_t)order[i] + 1]);
+        return pos ? sanitise(b) : b;
+    }
+    __device__ __forceinline__ float get_area(int i) const { return box_area(as_float4(img[2 * (size_t)order[i] + 1])); }
+};
+
+// Exclusive prefix of one flag per thread over the CTA; *total receives the sum.  Ends with a barrier.
+__device__ __forceinline__ unsigned agn_block_scan(bool f, unsigned *sh_w /*[AGN_THREADS / 32]*/, unsigned &total)
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned m = __ballot_sync(0xFFFFFFFFu, f);
+    if (lane == 0) sh_w[warp] = __popc(m);
+    __syncthreads();
+    unsigned before = 0u;
+    total = 0u;
+#pragma unroll
+    for (int w = 0; w < AGN_THREADS / 32; ++w) { const unsigned v = sh_w[w]; before += w < warp ? v : 0u; total += v; }
+    __syncthreads();
+    return before + __popc(m & ((1u << lane) - 1u));
+}
+
+__global__ void __launch_bounds__(AGN_THREADS, 1)
+k_segment_nms_agnostic(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_count, unsigned *__restrict__ kept_count,
+                       int C, int cap_seg, float thr, unsigned *__restrict__ tab_key_all, unsigned *__restrict__ tab_cls_all,
+                       long M4, unsigned *__restrict__ scratch, int img_first)
+{
+    extern __shared__ __align__(16) unsigned char agn_smem[];
+    unsigned long long *sh_key = reinterpret_cast<unsigned long long *>(agn_smem);       // [AGN_CAP] staging order
+    float4 *sh_box = reinterpret_cast<float4 *>(sh_key + AGN_CAP);                       // [AGN_CAP] staging order
+    uint2 *sh_co = reinterpret_cast<uint2 *>(sh_box + AGN_CAP);                           // [AGN_CAP] {cls_conf, obj_conf} bits
+    unsigned short *sh_idx = reinterpret_cast<unsigned short *>(sh_co + AGN_CAP);         // sorted position -> staging index
+    unsigned short *sh_kept = sh_idx + AGN_CAP;                                           // kept survivors, sorted positions
+    __shared__ unsigned sh_pre[YL_MAX_CLASSES + 1];           // exclusive prefix of seg_count over the classes
+    __shared__ unsigned sh_cnt[AGN_THREADS / 32][YL_MAX_CLASSES];
+    __shared__ unsigned sh_w[AGN_THREADS / 32];
+    __shared__ unsigned long long sh_rows[CHUNK];
+    __shared__ unsigned sh_supp[2];
+    __shared__ int sh_nk;
+    __shared__ unsigned sh_ns;
+
+    pdl_trigger();
+    pdl_wait();                                                 // segment counts and records of the filter kernel
+    const int b = img_first + blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned FULL = 0xFFFFFFFFu;
+    uint4 *img = cand + (size_t)b * C * cap_seg * 2;
+    unsigned *tab_key = tab_key_all + (size_t)b * M4, *tab_cls = tab_cls_all + (size_t)b * M4;
+    bool over = false;
+    {
+        // exclusive prefix over the classes (C <= 128: the first four warps, one class per lane)
+        const unsigned v = tid < C ? seg_count[b * C + tid] : 0u;
+        over = v > (unsigned)cap_seg;
+        unsigned incl = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned u = __shfl_up_sync(FULL, incl, o);
+            if (lane >= o) incl += u;
+        }
+        if (lane == 31) sh_w[warp] = incl;
+        if (tid == 0) sh_ns = 0u;
+        __syncthreads();
+        unsigned off = 0u;
+        for (int w = 0; w < warp && w < YL_MAX_CLASSES / 32; ++w) off += sh_w[w];
+        if (tid < C) sh_pre[tid] = off + incl - v;
+        if (tid == C - 1) sh_pre[C] = off + incl;
+    }
+    if (__syncthreads_or(over)) {                                // overflow: reported through meta[], caller re-runs
+        for (int c = tid; c < C; c += AGN_THREADS) kept_count[b * C + c] = 0u;
+        return;
+    }
+    const unsigned n = sh_pre[C];
+    auto locate = [&](unsigned i, int &c) -> uint4 * {         // i-th record of the image in class order
+        int lo = 0, hi = C;                                     // largest c with sh_pre[c] <= i
+        while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sh_pre[mid] <= i) lo = mid; else hi = mid; }
+        c = lo;
+        return img + ((size_t)lo * cap_seg + (i - sh_pre[lo])) * 2;
+    };
+    // ---- 1. first copies: the dense filter never writes the tables, so the entries in use are set here ----
+    for (unsigned i = tid; i < n; i += AGN_THREADS) {
+        int c;
+        const unsigned row = locate(i, c)[0].y;
+        tab_key[row] = FULL;
+        tab_cls[row] = FULL;
+    }
+    __syncthreads();
+    for (unsigned i = tid; i < n; i += AGN_THREADS) {
+        int c;
+        const uint4 a = locate(i, c)[0];
+        atomicMin(&tab_key[a.y], score_desc_bits(a.x));
+    }
+    __syncthreads();
+    for (unsigned i = tid; i < n; i += AGN_THREADS) {
+        int c;
+        const uint4 a = locate(i, c)[0];
+        if (score_desc_bits(a.x) == __ldcg(&tab_key[a.y])) atomicMin(&tab_cls[a.y], (unsigned)c);
+    }
+    __syncthreads();
+    // a copy survives when it is the box's first copy or when the literal self-IoU of its box is below thr
+    auto survives = [&](const uint4 &a, const float4 &bx, int c) -> bool {
+        if (score_desc_bits(a.x) == __ldcg(&tab_key[a.y]) && (unsigned)c == __ldcg(&tab_cls[a.y])) return true;
+        const float ar = box_area(bx);
+        return !suppresses_any(bx, ar, bx, ar, thr);
+    };
+    for (unsigned i = tid; i < n; i += AGN_THREADS) {
+        int c;
+        const uint4 *r = locate(i, c);
+        const uint4 a = r[0];
+        const float4 bx = as_float4(r[1]);
+        if (survives(a, bx, c)) {
+            const unsigned slot = atomicAdd(&sh_ns, 1u);
+            if (slot < (unsigned)AGN_CAP) {
+                sh_key[slot] = agn_key(a.x, c, a.y);
+                sh_box[slot] = bx;
+                sh_co[slot] = make_uint2(a.z, a.w);
+                sh_idx[slot] = (unsigned short)slot;
+            }
+        }
+    }
+    __syncthreads();
+    const unsigned ns = sh_ns;
+    const bool pos = thr > 0.0f;
+
+    if (ns <= (unsigned)AGN_CAP) {
+        // ---- 2. shared-memory path.  Every read of the image's records is done: rows may overwrite them from here ----
+        SmemStore s{sh_key, sh_idx, sh_box, pos};
+        bitonic_sort<SmemStore, AGN_THREADS>(s, (int)ns);
+        const int nk = pos ? greedy_nms<true, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk)
+                           : greedy_nms<false, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk);
+        // rank within the class: each warp takes a contiguous slice of the kept list; per-class counts per warp, a prefix over
+        // the warps, then ranks inside the slice from peer masks
+        const int q0 = (int)(((long)nk * warp) / (AGN_THREADS / 32)), q1 = (int)(((long)nk * (warp + 1)) / (AGN_THREADS / 32));
+        for (int c = lane; c < C; c += 32) sh_cnt[warp][c] = 0u;
+        __syncwarp();
+        for (int q = q0 + lane; q < q1; q += 32)
+            atomicAdd(&sh_cnt[warp][(int)(sh_key[sh_kept[q]] >> AGN_ROW_BITS) & (YL_MAX_CLASSES - 1)], 1u);
+        __syncthreads();
+        if (tid < C) {
+            unsigned run = 0u;
+            for (int w = 0; w < AGN_THREADS / 32; ++w) { const unsigned t = sh_cnt[w][tid]; sh_cnt[w][tid] = run; run += t; }
+            kept_count[b * C + tid] = run;
+        }
+        __syncthreads();
+        for (int qb = q0; qb < q1; qb += 32) {                  // warp-uniform trip count
+            const int q = qb + lane;
+            const bool act = q < q1;
+            const unsigned am = __ballot_sync(FULL, act);
+            if (act) {
+                const int p = sh_kept[q];
+                const int c = (int)(sh_key[p] >> AGN_ROW_BITS) & (YL_MAX_CLASSES - 1);
+                const unsigned peers = __match_any_sync(am, c);
+                const unsigned rank = sh_cnt[warp][c] + __popc(peers & ((1u << lane) - 1u));
+                const int e = sh_idx[p];
+                const uint2 co = sh_co[e];
+                store_row(reinterpret_cast<float *>(img + (size_t)c * cap_seg * 2) + (size_t)rank * 7, sh_box[e], co.x, co.y, (float)c);
+                __syncwarp(am);
+                if (lane == __ffs(peers) - 1) sh_cnt[warp][c] += __popc(peers);
+            }
+            __syncwarp();
+        }
+        return;
+    }
+
+    // ---- 3. global-memory path (correctness only) ----
+    unsigned *order = scratch + (size_t)b * C * cap_seg * 2, *kept_g = order + (size_t)C * cap_seg;
+    unsigned *sh_spre = sh_cnt[1];                              // exclusive prefix of the survivors per class
+    for (int c = tid; c < C; c += AGN_THREADS) sh_cnt[0][c] = 0u;
+    __syncthreads();
+    // records -> sort keys in place: survivors {score desc, ~row}, the others {~0, ~0} (sorted behind every survivor)
+    for (unsigned i = tid; i < n; i += AGN_THREADS) {
+        int c;
+        uint4 *r = locate(i, c);
+        const uint4 a = r[0];
+        const bool sv = survives(a, as_float4(r[1]), c);
+        r[0] = sv ? make_uint4(score_desc_bits(a.x), ~a.y, a.z, a.w) : make_uint4(FULL, FULL, a.z, a.w);
+        if (sv) atomicAdd(&sh_cnt[0][c], 1u);
+    }
+    __syncthreads();
+    for (int c = 0; c < C; ++c) {
+        GlobalStore g{img + (size_t)c * cap_seg * 2, false};
+        bitonic_sort<GlobalStore, AGN_THREADS>(g, (int)(sh_pre[c + 1] - sh_pre[c]));
+    }
+    if (tid == 0) {
+        unsigned run = 0u;
+        for (int c = 0; c < C; ++c) { sh_spre[c] = run; run += sh_cnt[0][c]; }
+        sh_spre[C] = run;
+    }
+    __syncthreads();
+    // image-wide rank of survivor (c, e): e, plus the survivors of lower classes with a score key <= its own, plus those of
+    // higher classes with a key < its own (binary searches on the sorted segments)
+    for (unsigned i = tid; i < ns; i += AGN_THREADS) {
+        int lo = 0, hi = C;
+        while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (sh_spre[mid] <= i) lo = mid; else hi = mid; }
+        const int c = lo;
+        const unsigned e = i - sh_spre[c];
+        const unsigned k = img[((size_t)c * cap_seg + e) * 2].x;
+        unsigned rank = e;
+        for (int c2 = 0; c2 < C; ++c2) {
+            if (c2 == c) continue;
+            const uint4 *seg = img + (size_t)c2 * cap_seg * 2;
+            unsigned l = 0u, h = sh_cnt[0][c2];                // first position whose key is > k (c2 < c) or >= k (c2 > c)
+            while (l < h) {
+                const unsigned mid = (l + h) >> 1;
+                const unsigned km = seg[2 * (size_t)mid].x;
+                if (c2 < c ? km <= k : km < k) l = mid + 1u; else h = mid;
+            }
+            rank += l;
+        }
+        order[rank] = (unsigned)c * (unsigned)cap_seg + e;
+    }
+    __syncthreads();
+    MergedStore ms{img, order, pos};
+    const int nk = pos ? greedy_nms<true, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk)
+                       : greedy_nms<false, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk);
+    // mark the kept records (the key word is free now), then compact every segment in place
+    for (unsigned i = tid; i < ns; i += AGN_THREADS) img[2 * (size_t)order[i]].x = 0u;
+    __syncthreads();
+    for (int q = tid; q < nk; q += AGN_THREADS) img[2 * (size_t)order[kept_g[q]]].x = 1u;
+    __syncthreads();
+    for (int c = 0; c < C; ++c) {
+        uint4 *seg = img + (size_t)c * cap_seg * 2;
+        float *rows = reinterpret_cast<float *>(seg);
+        const unsigned nsc = sh_cnt[0][c];
+        unsigned done = 0u;
+        for (unsigned e0 = 0; e0 < nsc; e0 += AGN_THREADS) {
+            const unsigned e = e0 + tid;
+            uint4 a = make_uint4(0u, 0u, 0u, 0u), bb = a;
+            if (e < nsc) { a = seg[2 * (size_t)e]; bb = seg[2 * (size_t)e + 1]; }
+            const bool kf = e < nsc && a.x == 1u;
+            unsigned tot;
+            const unsigned q = done + agn_block_scan(kf, sh_w, tot);     // barrier inside: every read of the chunk is done
+            if (kf) store_row(rows + (size_t)q * 7, as_float4(bb), a.z, a.w, (float)c);
+            __syncthreads();
+            done += tot;
+        }
+        if (tid == 0) kept_count[b * C + c] = done;
+    }
+}
+
 // Smallest K such that two positive areas whose bins (float bits >> 21: four per octave) differ by at least K have a
 // ratio above 1/(0.999 thr) * (1 + 1e-3): then IoU <= amin/amax < thr with a margin far above fp32 rounding, which is
 // the condition under which suppresses_pos returns false on the area test alone.
@@ -939,15 +1215,31 @@ static int area_bin_gap(float thr)
 
 using namespace yl;
 
-extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,
-                           float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
+// Scratch of the agnostic global-memory path, behind the standard workspace: u32 [B][2][C*cap_seg] (order, kept list).
+static size_t agn_scratch_bytes(int B, int C, int cap_seg)
 {
+    return align_up(sizeof(unsigned) * 2 * (size_t)B * C * cap_seg, 256);
+}
+
+extern "C" size_t yl_post_workspace_bytes_ex(int B, long M, int C, int cap_seg, int agnostic)
+{
+    if (agnostic != 0 && agnostic != 1) return 0;
+    const size_t base = yl_post_workspace_bytes(B, M, C, cap_seg);
+    return (base == 0 || !agnostic) ? base : base + agn_scratch_bytes(B, C, cap_seg);
+}
+
+extern "C" int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
+                         float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
+{
+    if (agnostic != 0 && agnostic != 1) return YL_ERR_ARG;
     if (!ws || !out_rows || !meta || B <= 0 || M <= 0 || C <= 0 || cap_seg <= 0 || cap_out <= 0) return YL_ERR_ARG;
     if (img_first < 0 || img_count < 0 || img_first + img_count > B) return YL_ERR_ARG;
     if (max_det < 0 || max_det > cap_out) return YL_ERR_ARG;
     if (C > YL_MAX_CLASSES) return YL_ERR_CLASSES;
+    // agnostic keys hold the box row in AGN_ROW_BITS bits; the global path addresses an image's records with 32 bits
+    if (agnostic && (M >= (1L << AGN_ROW_BITS) || (unsigned long long)C * (unsigned long long)cap_seg > 0xFFFFFFFFull)) return YL_ERR_ARG;
     const PostLayout L = post_layout(B, M, C, cap_seg);
-    if (ws_bytes < L.total) return YL_ERR_WORKSPACE;
+    if (ws_bytes < L.total + (agnostic ? agn_scratch_bytes(B, C, cap_seg) : 0)) return YL_ERR_WORKSPACE;
     if (img_count == 0) return YL_OK;
     char *w = (char *)ws;
     uint4 *cand = (uint4 *)(w + L.off_cand);
@@ -961,13 +1253,20 @@ extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int 
     // each kernel may become resident while its predecessor drains (PDL); it waits before reading the predecessor's output.
     // The first one follows the emit / dense filter kernel of yl_filter_* on the same stream.
     const bool pdl = pdl_enabled();
-    YL_CUDA_TRY(launch_after(k_segment_nms_bins, dim3(nseg), dim3(SMALL_THREADS), 0, st, pdl, cand, seg_count, kept_count, C, cap_seg,
-                             nms_thre, area_bin_gap(nms_thre), seg_first, big_count, big_list));
-    const int grid_big = nseg < 148 * 2 ? nseg : 148 * 2;
-    YL_CUDA_TRY(launch_after(k_segment_nms_big, dim3(grid_big), dim3(NMS_THREADS), 0, st, pdl, cand, (const unsigned *)seg_count, kept_count,
-                             C, cap_seg, nms_thre, (const unsigned *)big_count, (const unsigned *)big_list, kept_scratch));
-    if (max_det > 0) {
+    if (agnostic) {
         // per device, so set on every call (a host-side attribute: allowed during stream capture)
+        YL_CUDA_TRY(cudaFuncSetAttribute(k_segment_nms_agnostic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AGN_SMEM_BYTES));
+        YL_CUDA_TRY(launch_after(k_segment_nms_agnostic, dim3(img_count), dim3(AGN_THREADS), AGN_SMEM_BYTES, st, pdl, cand,
+                                 (const unsigned *)seg_count, kept_count, C, cap_seg, nms_thre, (unsigned *)(w + L.off_obj),
+                                 (unsigned *)(w + L.off_flags), L.M4, (unsigned *)(w + L.total), img_first));
+    } else {
+        YL_CUDA_TRY(launch_after(k_segment_nms_bins, dim3(nseg), dim3(SMALL_THREADS), 0, st, pdl, cand, seg_count, kept_count, C, cap_seg,
+                                 nms_thre, area_bin_gap(nms_thre), seg_first, big_count, big_list));
+        const int grid_big = nseg < 148 * 2 ? nseg : 148 * 2;
+        YL_CUDA_TRY(launch_after(k_segment_nms_big, dim3(grid_big), dim3(NMS_THREADS), 0, st, pdl, cand, (const unsigned *)seg_count, kept_count,
+                                 C, cap_seg, nms_thre, (const unsigned *)big_count, (const unsigned *)big_list, kept_scratch));
+    }
+    if (max_det > 0) {
         YL_CUDA_TRY(cudaFuncSetAttribute(k_select_topk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SEL_SMEM_BYTES));
         YL_CUDA_TRY(launch_after(k_select_topk, dim3(img_count), dim3(SEL_THREADS), SEL_SMEM_BYTES, st, pdl, (const uint4 *)cand,
                                  kept_count, C, cap_seg, max_det, uncapped, img_first));
@@ -975,6 +1274,13 @@ extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int 
     YL_CUDA_TRY(launch_after(k_gather_rows, dim3(nseg), dim3(GATHER_THREADS), 0, st, pdl, (const uint4 *)cand, (const unsigned *)seg_count,
                              (const unsigned *)kept_count, C, cap_seg, B, out_rows, cap_out, meta, seg_first));
     return YL_OK;
+}
+
+extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,
+                           float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
+{
+    return yl_nms_ex(ws, ws_bytes, B, M, C, cap_seg, nms_thre, max_det, 0, out_rows, cap_out, meta, uncapped, img_first, img_count,
+                     stream);
 }
 
 extern "C" int yl_nms(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre,

@@ -46,22 +46,23 @@ class _Workspace:
 
     _cache = {}
 
-    def __init__(self, device, B, M, C, cap_seg):
+    def __init__(self, device, B, M, C, cap_seg, agnostic=False):
         self.B, self.M, self.C, self.cap_seg = B, M, C, cap_seg
-        self.nbytes = _cabi.lib().yl_post_workspace_bytes(B, M, C, cap_seg)
+        self.nbytes = _cabi.lib().yl_post_workspace_bytes_ex(B, M, C, cap_seg, int(agnostic))
         if self.nbytes == 0:
             raise _cabi.YoloHeadError("invalid postprocess shape B=%d M=%d C=%d" % (B, M, C))
         self.buf = torch.empty(self.nbytes, dtype=torch.uint8, device=device)
 
     @classmethod
-    def get(cls, device, B, M, C, cap_seg):
-        key = (str(device), int(torch.cuda.current_stream(device).cuda_stream), threading.get_ident(), B, M, C, cap_seg)
+    def get(cls, device, B, M, C, cap_seg, agnostic=False):
+        # agnostic workspaces carry extra scratch (yl_post_workspace_bytes_ex) and are kept apart from the others
+        key = (str(device), int(torch.cuda.current_stream(device).cuda_stream), threading.get_ident(), B, M, C, agnostic, cap_seg)
         ws = cls._cache.get(key)
         if ws is None:
-            # keep one workspace per (device, stream, thread, B, M, C): drop smaller-capacity predecessors
-            for k in [k for k in cls._cache if k[:6] == key[:6]]:
+            # keep one workspace per (device, stream, thread, B, M, C, agnostic): drop smaller-capacity predecessors
+            for k in [k for k in cls._cache if k[:7] == key[:7]]:
                 del cls._cache[k]
-            ws = cls._cache[key] = cls(device, B, M, C, cap_seg)
+            ws = cls._cache[key] = cls(device, B, M, C, cap_seg, agnostic)
         return ws
 
     def ptr(self):
@@ -78,6 +79,13 @@ def _check_max_det(max_det):
     if isinstance(max_det, bool) or not isinstance(max_det, (int, np.integer)) or int(max_det) < 1:
         raise ValueError("max_det must be None or an int >= 1, got %r" % (max_det,))
     return int(max_det)
+
+
+def _check_agnostic(agnostic):
+    """A bool; checked before any CUDA work."""
+    if not isinstance(agnostic, bool):
+        raise TypeError("agnostic must be a bool, got %r" % (agnostic,))
+    return agnostic
 
 
 def _round4(n):
@@ -98,24 +106,24 @@ def _split(rows, meta_host, B, out_device, out_dtype):
     return out
 
 
-def _run(front_end, device, B, M, C, nms_thre, max_det=None):
+def _run(front_end, device, B, M, C, nms_thre, max_det=None, agnostic=False):
     """Runs front end + NMS, growing cap_seg / cap_out and re-running when the device reports an overflow.  With a cap the
     output holds max_det rows per image (rounded up to a multiple of 4), which no image can exceed; the capacities a capped
-    call settles on are kept apart from those of uncapped calls."""
+    or agnostic call settles on are kept apart from those of plain calls."""
     L = _cabi.lib()
-    hint_key = (B, M, C) if max_det is None else (B, M, C, max_det)
+    hint_key = (B, M, C) if max_det is None and not agnostic else (B, M, C, max_det, agnostic)
     cap_seg, cap_out = _cap_hint.get(hint_key, (_DEFAULT_CAP_SEG, _DEFAULT_CAP_OUT))
     if max_det is not None:
         cap_out = _round4(max_det)
     cap_seg = min(cap_seg, _next_pow2(M))
     while True:
-        ws = _Workspace.get(device, B, M, C, cap_seg)
+        ws = _Workspace.get(device, B, M, C, cap_seg, agnostic)
         rows = torch.empty((B, cap_out, 7), dtype=torch.float32, device=device)
         meta = torch.empty((3 * B,), dtype=torch.int32, device=device)
         _cabi.check(L.yl_post_reset(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _stream()))
         front_end(ws, cap_seg)
-        _cabi.check(L.yl_nms_topk(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), max_det or 0, rows.data_ptr(), cap_out,
-                                  meta.data_ptr(), None, 0, B, _stream()))
+        _cabi.check(L.yl_nms_ex(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), max_det or 0, int(agnostic), rows.data_ptr(),
+                                cap_out, meta.data_ptr(), None, 0, B, _stream()))
         mh = meta.cpu().numpy()                      # the one D2H sync the list-of-tensors contract requires
         max_seg, max_rows = int(mh[B:2 * B].max()), int(mh[:B].max())
         if max_seg > cap_seg:
@@ -130,7 +138,7 @@ def _run(front_end, device, B, M, C, nms_thre, max_det=None):
         return rows, mh
 
 
-def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_det=None):
+def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_det=None, agnostic=False):
     """Same contract as the reference's postprocess (yolo/util/utils.py:92).
 
     prediction: [B, M, 5+C] decoded (cx, cy, w, h, obj, cls...), fp32, on a CUDA device (a CPU tensor, as
@@ -142,8 +150,10 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
     the order of a stable argsort, where NumPy's default sort leaves them unspecified (utils.py:58).
     max_det (keyword only, not part of the reference signature): keep at most this many detections per image, those with the
     highest obj_conf * cls_conf (equal scores keep the order above), still listed classes ascending then score descending.
+    agnostic (keyword only, not part of the reference signature): class-agnostic NMS, see detect_raw.
     """
     max_det = _check_max_det(max_det)
+    agnostic = _check_agnostic(agnostic)
     if prediction.dim() != 3 or prediction.shape[2] < 6:
         raise ValueError("prediction must be [B, M, 5+C]")
     if prediction.dtype != torch.float32:
@@ -161,7 +171,7 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_dense(pred.data_ptr(), B, M, C, num_classes, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                           cap_seg, 0, B, _stream()))
-        rows, mh = _run(front, pred.device, B, M, C, nms_thre, max_det)
+        rows, mh = _run(front, pred.device, B, M, C, nms_thre, max_det, agnostic)
     return _split(rows, mh, B, in_device, prediction.dtype)
 
 
@@ -187,7 +197,8 @@ def _check_raws(head_outputs, num_classes):
     return raws, B, Fs, _DTYPE_CODES[raws[0].dtype]
 
 
-def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None):
+def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None,
+               agnostic=False):
     """Fused YOLOLayer eval decode (yololayer.py:88-166) + postprocess (utils.py:92-223).
 
     head_outputs: the three raw head conv outputs [B, 3*(5+C), F_l, F_l] (stride 8, 16, 32; yolov4.py:235-251).
@@ -203,8 +214,15 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     max_det: keep at most this many detections per image, those with the highest obj_conf * cls_conf; ties keep the
     uncapped order (lower class first, then the order inside the class).  The kept rows stay in the uncapped order, classes
     ascending then score descending.  None (the default) keeps every detection.
+
+    agnostic: class-agnostic NMS.  One greedy NMS per image over all its (box, class) candidates, in the order score
+    descending, class ascending, box index descending; a candidate is dropped at IoU >= nms_thre with any earlier kept
+    candidate, whatever the classes.  A box then keeps at most one label, its best-scoring passing class (a degenerate box --
+    NaN, zero or negative extent, overflowing area -- never suppresses itself and keeps all its labels).  The kept rows are
+    listed as usual, classes ascending then score descending; max_det applies to them.  Default False: per-class NMS.
     """
     max_det = _check_max_det(max_det)
+    agnostic = _check_agnostic(agnostic)
     raws, B, Fs, dt = _check_raws(head_outputs, num_classes)
     C = int(num_classes)
     M = sum(3 * f * f for f in Fs)
@@ -218,7 +236,7 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_raw_typed(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                               M, cap_seg, 0, B, 3, _stream()))
-        rows, mh = _run(front, dev, B, M, C, nms_thre, max_det)
+        rows, mh = _run(front, dev, B, M, C, nms_thre, max_det, agnostic)
     return _split(rows, mh, B, dev, torch.float32)
 
 
@@ -235,13 +253,15 @@ class HeadPostprocessor:
     max_det caps the detections of every image as in detect_raw; cap_out then defaults to max_det rounded up to a multiple
     of 4, so the output (and a DetectionExchange built with hp.cap_out) is sized by the cap.  uncapped is a device int32 [B]
     with every image's uncapped count, refreshed by every run and replay: meta[b] < uncapped[b] means image b was capped.
-    Without a cap uncapped is the view meta[:B].
+    Without a cap uncapped is the view meta[:B].  agnostic selects class-agnostic NMS as in detect_raw (uncapped then counts
+    the agnostic rows).
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
                  cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, side_priority=0,
-                 mode="nms_side", max_det=None):
+                 mode="nms_side", max_det=None, agnostic=False):
         self.max_det = _check_max_det(max_det)
+        self.agnostic = _check_agnostic(agnostic)
         if cap_out is None:
             cap_out = _DEFAULT_CAP_OUT if self.max_det is None else _round4(self.max_det)
         if self.max_det is not None and self.max_det > int(cap_out):
@@ -257,7 +277,7 @@ class HeadPostprocessor:
         self.mask = _cabi.ints([v for m in anchor_mask for v in m])
         self.fs = _cabi.ints(self.Fs)
         with torch.cuda.device(self.device):
-            self.ws = _Workspace(self.device, self.B, self.M, self.C, self.cap_seg)
+            self.ws = _Workspace(self.device, self.B, self.M, self.C, self.cap_seg, self.agnostic)
             self.rows = torch.empty((self.B, self.cap_out, 7), dtype=torch.float32, device=self.device)
             self.meta = torch.zeros((3 * self.B,), dtype=torch.int32, device=self.device)
             self.uncapped = self.meta[:self.B] if self.max_det is None else torch.zeros((self.B,), dtype=torch.int32, device=self.device)
@@ -302,9 +322,9 @@ class HeadPostprocessor:
                 # three-deep: flag(g+1) on the main stream, emit(g) on the first side stream, NMS + gather(g-1) on the second
                 self.side2.wait_stream(self.side)
                 nms_stream = self.side2
-            _cabi.check(L.yl_nms_topk(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
-                                      self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
-                                      None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, nms_stream.cuda_stream))
+            _cabi.check(L.yl_nms_ex(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
+                                    int(self.agnostic), self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
+                                    None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, nms_stream.cuda_stream))
         main.wait_stream(self.side)
         if self.mode == "pipe3":
             main.wait_stream(self.side2)
