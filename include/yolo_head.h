@@ -288,7 +288,7 @@ int yl_detect_host_ex(yl_context *ctx, const float *const *raw_host, float conf_
  *     reference validates on rank 0 only, yolo/engine/build.py:110-190, main_amp.py:175,207)
  * One process per GPU; rank r owns B images and ends up with the detections of all world*B images (rank-major).  Each rank
  * owns one device window (rows / counts / flags) that the peers map through CUDA IPC over NVLink; yl_xchg_push copies
- * exactly counts[b] rows per image into every rank's window with plain peer stores (no collective, no staging, no host
+ * exactly counts[b] rows per image into every rank's window with one bulk store per peer (no collective, no host
  * synchronisation), yl_xchg_wait blocks the stream until every rank's rows of that slot have landed, yl_xchg_release
  * hands the slot back (a peer's next push into it waits for that).  All three are graph-capturable, so the exchange of
  * step i runs under the kernels of step i+1 (double-buffered `slots`).
@@ -304,9 +304,9 @@ int yl_xchg_create(yl_xchg **out, int device, int rank, int world, int B, long c
 int yl_xchg_destroy(yl_xchg *x);
 /* The same object over windows the CALLER owns: `windows[p]` = rank p's window as mapped into this process (all of
  * yl_xchg_window_bytes() bytes, 256-byte aligned; e.g. torch symmetric memory), `multicast` = an NVSwitch multicast mapping of the
- * same windows or NULL.  With a multicast mapping yl_xchg_push issues ONE multimem.st per 16 bytes and the switch replicates it into
- * every window (a rank sends 1/world of the peer-store forms' bytes).  No CUDA IPC; yl_xchg_destroy leaves the windows alone.
- * The caller synchronises the ranks between creation and the first push. */
+ * same windows or NULL.  With a multicast mapping yl_xchg_push issues one bulk store to the multicast mapping and the switch
+ * replicates it into every window (a rank sends 1/world of the bytes of the per-peer stores).  No CUDA IPC; yl_xchg_destroy
+ * leaves the windows alone.  The caller synchronises the ranks between creation and the first push. */
 size_t yl_xchg_window_bytes(int world, int B, long cap_out, int slots);
 int yl_xchg_create_external(yl_xchg **out, int device, int rank, int world, int B, long cap_out, int slots,
                             void *const *windows, void *multicast);

@@ -106,11 +106,6 @@ def test_exchange_single_rank_self_window():
     _run(1)
 
 
-def test_exchange_single_rank_register_staged_push(monkeypatch):
-    monkeypatch.setenv("YL_XCHG_BULK", "0")          # read by yl_xchg_create in the spawned worker
-    _run(1)
-
-
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_exchange_two_ranks_bit_exact_over_reused_slots():
     _run(2)

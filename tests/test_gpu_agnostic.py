@@ -162,14 +162,13 @@ def test_with_max_det():
         assert_lists_bit_equal(_fused(raws, 80, 1e-4, 0.4, max_det=k), cap_detections(unc, k), what=f"max_det {k}")
 
 
-@pytest.mark.parametrize("n_groups,mode,dt", [(1, "nms_side", torch.float32), (2, "nms_side", torch.float32),
-                                              (2, "pipe3", torch.float32), (1, "nms_side", torch.float16)])
-def test_head_postprocessor_run_and_replay(n_groups, mode, dt):
+@pytest.mark.parametrize("n_groups,dt", [(1, torch.float32), (2, torch.float32), (1, torch.float16), (3, torch.bfloat16)])
+def test_head_postprocessor_run_and_replay(n_groups, dt):
     B = 6
     raws = [r.to(dt) for r in synth_head_outputs(B, 608, 80, seed=11, device="cuda")]
     want = _fused(raws, 80, 1e-4, 0.4)
     assert_lists_bit_equal(want, spec.detect([r.float() for r in raws], 80, 1e-4, 0.4), what="detect_raw")
-    hp = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=n_groups, mode=mode, agnostic=True)
+    hp = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=n_groups, agnostic=True)
     hp.run(raws)
     torch.cuda.synchronize()
     assert_lists_bit_equal(hp.results(), want, what="run")
@@ -185,7 +184,7 @@ def test_head_postprocessor_run_and_replay(n_groups, mode, dt):
     torch.cuda.synchronize()
     assert_lists_bit_equal(hp.results(), _fused(fresh, 80, 1e-4, 0.4), what="replay, new inputs")
     # with a cap, uncapped counts the agnostic rows
-    hk = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=n_groups, mode=mode, agnostic=True, max_det=300)
+    hk = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=n_groups, agnostic=True, max_det=300)
     hk.run(fresh)
     torch.cuda.synchronize()
     assert_lists_bit_equal(hk.results(), _fused(fresh, 80, 1e-4, 0.4, max_det=300), what="capped run")

@@ -1,5 +1,5 @@
 """Image-group pipelining probe: flag/emit of group g+1 on the main stream next to NMS/gather of group g on a side
-stream, with and without a high-priority side stream, as a CUDA graph."""
+stream, as a CUDA graph, for each group count."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import yolov4_b200 as yb
@@ -13,11 +13,8 @@ def timeit(hp, n=100):
     for _ in range(n): hp.replay()
     ev1.record(); torch.cuda.synchronize()
     return ev0.elapsed_time(ev1) * 1e3 / n
-MODES = os.environ.get("MODES", "nms_side,emit_side,pipe3").split(",")
 GROUPS = [int(g) for g in os.environ.get("GROUPS", "1,2,4,8").split(",")]
-for mode in MODES:
-    for prio in (0, -1):
-        for G in GROUPS:
-            hp = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=G, side_priority=prio, mode=mode).capture(raws)
-            t = timeit(hp)
-            print("mode %-9s prio %2d groups %2d: %.1f us/step %.0f img/s" % (mode, prio, G, t, B / t * 1e6), flush=True)
+for G in GROUPS:
+    hp = yb.HeadPostprocessor(B, [76, 38, 19], 80, 1e-4, 0.4, n_groups=G).capture(raws)
+    t = timeit(hp)
+    print("groups %2d: %.1f us/step %.0f img/s" % (G, t, B / t * 1e6), flush=True)

@@ -34,7 +34,7 @@ loss = yb.fused_yolo_loss(raws_g, labels, CFG, 0.7)
 loss.backward()
 ok &= bool(torch.isfinite(raws_g[0].grad).any().item())
 # round 2: the three scales of build_target in one launch pair, the train decode's backward from the raw tensor, the padded epilogue,
-# the single-rank exchange (both push forms), and (YL_FLAG=tma in the environment) the TMA flag kernel through detect_raw above
+# the single-rank exchange, and (YL_FLAG=tma in the environment) the TMA flag kernel through detect_raw above
 ds = [yb.YOLOLayer(CFG, l, device="cuda").train()(raws[l].clone().requires_grad_(True)) for l in range(3)]
 one = yb.build_targets3([x["output"] for x in ds], [x["pred"] for x in ds], [0, 1, 2], labels, yb.ANCHORS_PX, yb.ANCHOR_MASK, 0.7, 80)
 for a, b in zip(one[1], yb.YOLOLoss(CFG, 0.7, device="cuda").build_target(ds[1]["output"], ds[1]["pred"], 1, labels)):
@@ -45,16 +45,14 @@ rows, meta = hp.run(raws)
 out = yb.coco_rows_padded(rows, meta[:2], [[480, 640, 312, 416]] * 2, [7, 9], list(range(1, 81)))
 ok &= out.shape[0] == int(meta[:2].sum())
 from yolov4_b200.sharded import DetectionExchange
-for bulk in ("1", "0"):
-    os.environ["YL_XCHG_BULK"] = bulk
-    ex = DetectionExchange(2, 8192, torch.device("cuda", 0), slots=2)
-    for slot in (0, 1, 0):
-        ex.push(rows, meta[:2], slot); ex.wait(slot)
-        got = ex.results(slot)
-        ok &= all(torch.equal(g, rows[b, :g.shape[0]]) for b, g in enumerate(got) if g is not None)
-        ex.release(slot)
-    ok &= ex.status() == 0
-    ex.close()
+ex = DetectionExchange(2, 8192, torch.device("cuda", 0), slots=2)
+for slot in (0, 1, 0):
+    ex.push(rows, meta[:2], slot); ex.wait(slot)
+    got = ex.results(slot)
+    ok &= all(torch.equal(g, rows[b, :g.shape[0]]) for b, g in enumerate(got) if g is not None)
+    ex.release(slot)
+ok &= ex.status() == 0
+ex.close()
 torch.cuda.synchronize()
 print("sanitize_small:", "ok" if ok else "MISMATCH")
 sys.exit(0 if ok else 1)

@@ -6,13 +6,14 @@
 //     flag   [slots][world] u32   "source s has delivered epoch e of this slot"      (written by the peers)
 //     ack    [slots][world] u32   "reader s has released epoch e of this slot"       (written by the peers)
 //     epoch  [slots] u32          completed exchanges of the slot                      (local)
-// k_xchg_push copies the kept rows of the local images (exactly counts[b] rows each, 128-bit loads, one store per peer over
-// NVLink: fire-and-forget writes, no collective, no staging) into every window, then publishes flag = epoch + 1 behind a
-// system-scope fence.  k_xchg_wait spins (bounded) until every source's flag reached epoch + 1; k_xchg_release bumps the
-// epoch and tells every peer that this rank is done reading the slot, which is what a peer's next push into that slot
-// waits for (credit: a slot is never overwritten while somebody still reads it).  Nothing here needs a host
-// synchronisation or a changing kernel argument, so push / wait / release are captured into the step's CUDA graph on a
-// side branch and the exchange of step i runs under the kernels of step i+1.
+// k_xchg_push_bulk copies the kept rows of the local images (exactly counts[b] rows each) into every window: bulk copies
+// through shared memory, then one bulk store per peer over NVLink, or one bulk store to the windows' multicast mapping that
+// the switch replicates (fire-and-forget writes, no collective); it then publishes flag = epoch + 1 behind a system-scope
+// fence.  k_xchg_wait spins (bounded) until every source's flag reached epoch + 1; k_xchg_release bumps the epoch and tells
+// every peer that this rank is done reading the slot, which is what a peer's next push into that slot waits for (credit: a
+// slot is never overwritten while somebody still reads it).  Nothing here needs a host synchronisation or a changing kernel
+// argument, so push / wait / release are captured into the step's CUDA graph on a side branch and the exchange of step i
+// runs under the kernels of step i+1.
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
@@ -23,9 +24,6 @@
 namespace yl {
 
 constexpr int XCHG_MAX_WORLD = 16;
-constexpr int XCHG_THREADS = 256;
-constexpr int XCHG_UNROLL = 8;                   // independent 128-bit loads in flight per thread
-constexpr unsigned XCHG_CHUNK = XCHG_THREADS * XCHG_UNROLL;   // float4s per work unit (32 KB)
 
 struct XchgWindow {                  // device pointers into ONE rank's window
     float *rows;
@@ -82,79 +80,12 @@ __device__ __forceinline__ bool spin_ge(const unsigned *p, unsigned want, unsign
     return true;
 }
 
-__global__ void __launch_bounds__(XCHG_THREADS)
-k_xchg_push(const __grid_constant__ XchgPeers P, int rank, int world, int B, long cap_out, int slots, int slot,
-            const float *__restrict__ rows, const int *__restrict__ counts, unsigned *__restrict__ done,
-            int *__restrict__ status, unsigned long long limit_ns)
-{
-    __shared__ unsigned sh_epoch;
-    __shared__ int sh_ok;
-    const XchgWindow &me = P.w[rank];
-    if (threadIdx.x == 0) { sh_epoch = me.epoch[slot]; sh_ok = 1; }
-    __syncthreads();
-    const unsigned epoch = sh_epoch;
-    // credit: every reader has released the previous use of this slot (ack >= epoch; epoch counts completed exchanges)
-    if (threadIdx.x < world && !spin_ge(me.ack + slot * XCHG_MAX_WORLD + threadIdx.x, epoch, limit_ns)) sh_ok = 0;
-    __syncthreads();
-    if (!sh_ok) {
-        if (threadIdx.x == 0) atomicExch(status, 1);
-        return;
-    }
-    const size_t img_f4 = (size_t)cap_out * 7 / 4;                   // float4s per image slot (cap_out % 4 == 0)
-    // Work unit = (image, chunk of XCHG_CHUNK float4s); a thread keeps XCHG_UNROLL independent 128-bit loads in flight and then
-    // issues their world stores (fire-and-forget over NVLink): with one load in flight per thread the kernel ran at the pace
-    // of one L2 / DRAM round trip per 16 bytes and thread (8 CTAs: 415 us per 20 MB; 32 CTAs: 208 us).
-    const int n_chunks = (int)((img_f4 + XCHG_CHUNK - 1) / XCHG_CHUNK);
-    for (int u = blockIdx.x; u < B * n_chunks; u += gridDim.x) {
-        const int b = u / n_chunks, c = u - b * n_chunks;
-        const int n = min(max(counts[b], 0), (int)cap_out);
-        const unsigned nf4 = ((unsigned)n * 7u + 3u) >> 2;           // whole float4s: the padding lies inside the image's own capacity
-        const unsigned lo = (unsigned)c * XCHG_CHUNK;
-        if (lo >= nf4) {
-            if (c == 0 && threadIdx.x < world) P.w[threadIdx.x].counts[(size_t)slot * world * B + (size_t)rank * B + b] = n;
-            continue;
-        }
-        const unsigned hi = min(nf4, lo + XCHG_CHUNK);
-        const float4 *src = reinterpret_cast<const float4 *>(rows) + (size_t)b * img_f4;
-        const size_t dst_img = ((size_t)slot * world * B + (size_t)rank * B + b);
-        for (unsigned i0 = lo + threadIdx.x; i0 < hi; i0 += XCHG_THREADS * XCHG_UNROLL) {
-            float4 v[XCHG_UNROLL];
-#pragma unroll
-            for (int k = 0; k < XCHG_UNROLL; ++k) {
-                const unsigned i = i0 + k * XCHG_THREADS;
-                if (i < hi) v[k] = src[i];
-            }
-#pragma unroll
-            for (int k = 0; k < XCHG_UNROLL; ++k) {
-                const unsigned i = i0 + k * XCHG_THREADS;
-                if (i < hi)
-                    for (int p = 0; p < world; ++p) reinterpret_cast<float4 *>(P.w[p].rows)[dst_img * img_f4 + i] = v[k];
-            }
-        }
-        if (c == 0 && threadIdx.x < world) P.w[threadIdx.x].counts[dst_img] = n;
-    }
-    // publish: all CTAs' stores are fenced at system scope before the last CTA raises the flags
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        sh_ok = (atomicAdd(done + slot, 1u) == gridDim.x - 1) ? 2 : 1;
-    }
-    __syncthreads();
-    if (sh_ok == 2) {
-        if (threadIdx.x == 0) done[slot] = 0u;
-        __threadfence_system();
-        if (threadIdx.x < world) st_sys(P.w[threadIdx.x].flag + slot * XCHG_MAX_WORLD + rank, epoch + 1u);
-    }
-}
-
-// ---- bulk-copy form of the push (default): the rows go global -> shared memory -> every window as cp.async.bulk transfers of
-// XB_BYTES (SASS UBLKCP), issued by ONE thread per CTA over a ring of XB_STAGES shared-memory stages.  No register staging, no
-// per-thread 16-byte stores: the copy engines of the SM (TMA) produce large NVLink write bursts while the CTA's other warps do not
-// exist at all (32 threads per CTA), so the push takes almost nothing from the step's kernels it runs next to.
-__device__ __forceinline__ void mc_st4(float *mc, const float4 &v)
-{
-    asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(mc), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
+// ---- the push: the rows go global -> shared memory -> every window as cp.async.bulk transfers of XB_BYTES (SASS UBLKCP),
+// issued by ONE thread per CTA over a ring of XB_STAGES shared-memory stages.  No register staging, no per-thread 16-byte
+// stores: the copy engines of the SM (TMA) produce large NVLink write bursts while the CTA's other warps do not exist at all
+// (32 threads per CTA), so the push takes almost nothing from the step's kernels it runs next to.  With a multicast mapping
+// (windows in symmetric memory; torch does the CUDA VMM / fabric plumbing) one bulk store reaches every rank's window and the
+// switch replicates it: a rank sends 1/world of the bytes of the per-peer stores, and what arrives is unchanged.
 __device__ __forceinline__ void mc_st1(unsigned *mc, unsigned v)
 {
     asm volatile("multimem.st.relaxed.sys.global.u32 [%0], %1;" ::"l"(mc), "r"(v) : "memory");
@@ -164,6 +95,7 @@ constexpr unsigned XB_BYTES = 16384;
 constexpr int XB_STAGES = 4;
 constexpr int XB_DEPTH = 1;                    // bulk loads in flight ahead of the stores (XB_DEPTH < XB_STAGES); deeper look-ahead with
                                                // 4 KB units measured no better (the push is not what bounds the exchange)
+constexpr int XB_SMEM = XB_STAGES * (int)XB_BYTES;     // dynamic shared memory of k_xchg_push_bulk
 
 __device__ __forceinline__ unsigned xb_smem(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 
@@ -272,67 +204,6 @@ k_xchg_push_bulk(const __grid_constant__ XchgPeers P, XchgWindow mc, int rank, i
     }
 }
 
-// ---- NVSwitch multicast form of the push: the window lives in symmetric memory with a multicast mapping (torch's symmetric
-// memory does the CUDA VMM / fabric plumbing); ONE multimem.st per 16 bytes reaches every rank's window, the switch replicates.
-// A rank then sends 1/world of what the peer-store forms send; what arrives is unchanged.
-__global__ void __launch_bounds__(XCHG_THREADS)
-k_xchg_push_mc(const __grid_constant__ XchgPeers P, XchgWindow mc, int rank, int world, int B, long cap_out, int slots, int slot,
-               const float *__restrict__ rows, const int *__restrict__ counts, unsigned *__restrict__ done,
-               int *__restrict__ status, unsigned long long limit_ns)
-{
-    __shared__ unsigned sh_epoch;
-    __shared__ int sh_ok;
-    const XchgWindow &me = P.w[rank];
-    if (threadIdx.x == 0) { sh_epoch = me.epoch[slot]; sh_ok = 1; }
-    __syncthreads();
-    const unsigned epoch = sh_epoch;
-    if (threadIdx.x < world && !spin_ge(me.ack + slot * XCHG_MAX_WORLD + threadIdx.x, epoch, limit_ns)) sh_ok = 0;
-    __syncthreads();
-    if (!sh_ok) {
-        if (threadIdx.x == 0) atomicExch(status, 1);
-        return;
-    }
-    const size_t img_f4 = (size_t)cap_out * 7 / 4;
-    const int n_chunks = (int)((img_f4 + XCHG_CHUNK - 1) / XCHG_CHUNK);
-    for (int u = blockIdx.x; u < B * n_chunks; u += gridDim.x) {
-        const int b = u / n_chunks, c = u - b * n_chunks;
-        const int n = min(max(counts[b], 0), (int)cap_out);
-        const unsigned nf4 = ((unsigned)n * 7u + 3u) >> 2;
-        const unsigned lo = (unsigned)c * XCHG_CHUNK;
-        const size_t dst_img = ((size_t)slot * world * B + (size_t)rank * B + b);
-        if (c == 0 && threadIdx.x == 0) mc_st1(reinterpret_cast<unsigned *>(mc.counts) + dst_img, (unsigned)n);
-        if (lo >= nf4) continue;
-        const unsigned hi = min(nf4, lo + XCHG_CHUNK);
-        const float4 *src = reinterpret_cast<const float4 *>(rows) + (size_t)b * img_f4;
-        for (unsigned i0 = lo + threadIdx.x; i0 < hi; i0 += XCHG_THREADS * XCHG_UNROLL) {
-            float4 v[XCHG_UNROLL];
-#pragma unroll
-            for (int k = 0; k < XCHG_UNROLL; ++k) {
-                const unsigned i = i0 + k * XCHG_THREADS;
-                if (i < hi) v[k] = src[i];
-            }
-#pragma unroll
-            for (int k = 0; k < XCHG_UNROLL; ++k) {
-                const unsigned i = i0 + k * XCHG_THREADS;
-                if (i < hi) mc_st4(mc.rows + (dst_img * img_f4 + i) * 4, v[k]);
-            }
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence_system();
-        sh_ok = (atomicAdd(done + slot, 1u) == gridDim.x - 1) ? 2 : 1;
-    }
-    __syncthreads();
-    if (sh_ok == 2) {
-        if (threadIdx.x == 0) {
-            done[slot] = 0u;
-            __threadfence_system();
-            mc_st1(mc.flag + slot * XCHG_MAX_WORLD + rank, epoch + 1u);      // one store raises this source's flag everywhere
-        }
-    }
-}
-
 __global__ void k_xchg_wait(const __grid_constant__ XchgPeers P, int rank, int world, int slot, int *__restrict__ status,
                             unsigned long long limit_ns)
 {
@@ -365,7 +236,7 @@ struct yl_xchg {
     char *peer[XCHG_MAX_WORLD];        // mapped windows (peer[rank] == window)
     XchgPeers P;
     unsigned long long limit_ns;
-    bool connected, bulk, external;    // external: the windows belong to the caller (symmetric memory), not to this object
+    bool connected, external;          // external: the windows belong to the caller (symmetric memory), not to this object
     char *mc;                          // multicast mapping of the windows, or null
     XchgWindow MC;
 };
@@ -394,24 +265,42 @@ extern "C" int yl_xchg_destroy(yl_xchg *x)
     return YL_OK;
 }
 
-extern "C" int yl_xchg_create(yl_xchg **out, int device, int rank, int world, int B, long cap_out, int slots)
+// What both creation paths share on the host: the argument checks, the window layout, the time limit and the push grid.  Returns
+// null for arguments they reject and when the allocation fails (both YL_ERR_ARG).  Through the multicast mapping a rank sends
+// 1/world of the bytes: 16 single-warp CTAs keep the switch busy (8 GPUs: 267 us per step with 16, 273 us with 64); the stores
+// to every peer want 64.
+static yl_xchg *xchg_new(int device, int rank, int world, int B, long cap_out, int slots, bool multicast)
 {
-    if (!out || rank < 0 || world < 1 || world > XCHG_MAX_WORLD || rank >= world || B <= 0 || cap_out <= 0 || cap_out % 4 != 0 ||
-        slots < 1 || slots > 8)
-        return YL_ERR_ARG;
+    if (rank < 0 || world < 1 || world > XCHG_MAX_WORLD || rank >= world || B <= 0 || cap_out <= 0 || cap_out % 4 != 0 || slots < 1 ||
+        slots > 8)
+        return nullptr;
     yl_xchg *x = (yl_xchg *)calloc(1, sizeof(yl_xchg));
-    if (!x) return YL_ERR_ARG;
+    if (!x) return nullptr;
     x->device = device; x->rank = rank; x->world = world; x->B = B; x->cap_out = cap_out; x->slots = slots;
     x->L = xchg_layout(world, B, cap_out, slots);
     x->limit_ns = 5000000000ull;                                     // 5 s: a missing peer is reported, not waited for forever
-    x->push_ctas = getenv("YL_XCHG_CTAS") ? atoi(getenv("YL_XCHG_CTAS")) : 64;
-    if (x->push_ctas < 1) x->push_ctas = 1;
-    x->bulk = !(getenv("YL_XCHG_BULK") && getenv("YL_XCHG_BULK")[0] == '0');     // YL_XCHG_BULK=0: the register-staged push
-    cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaMalloc(&x->window, x->L.total);
-    // flags, acks, epochs, counters start at zero; the row area needs no initialisation
+    x->push_ctas = multicast ? 16 : 64;
+    return x;
+}
+
+// What both share on the object's device, once it is current and x->window is set: the push kernel may use XB_SMEM bytes of
+// dynamic shared memory (an attribute of each device, so every object sets it on its own device and the push sets nothing),
+// and this rank's flags, acks, epochs and counters start at zero (the row area needs no initialisation).
+static cudaError_t xchg_init_window(yl_xchg *x)
+{
+    cudaError_t e = cudaFuncSetAttribute(k_xchg_push_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, XB_SMEM);
     if (e == cudaSuccess) e = cudaMemset(x->window + x->L.off_counts, 0, x->L.total - x->L.off_counts);
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    return e;
+}
+
+extern "C" int yl_xchg_create(yl_xchg **out, int device, int rank, int world, int B, long cap_out, int slots)
+{
+    yl_xchg *x = out ? xchg_new(device, rank, world, B, cap_out, slots, false) : nullptr;
+    if (!x) return YL_ERR_ARG;
+    cudaError_t e = cudaSetDevice(device);
+    if (e == cudaSuccess) e = cudaMalloc(&x->window, x->L.total);
+    if (e == cudaSuccess) e = xchg_init_window(x);
     if (e != cudaSuccess) { yl_xchg_destroy(x); return YL_ERR_CUDA_BASE + (int)e; }
     x->peer[rank] = x->window;
     *out = x;
@@ -427,30 +316,18 @@ extern "C" size_t yl_xchg_window_bytes(int world, int B, long cap_out, int slots
 extern "C" int yl_xchg_create_external(yl_xchg **out, int device, int rank, int world, int B, long cap_out, int slots,
                                        void *const *windows, void *multicast)
 {
-    if (!out || !windows || rank < 0 || world < 1 || world > XCHG_MAX_WORLD || rank >= world || B <= 0 || cap_out <= 0 ||
-        cap_out % 4 != 0 || slots < 1 || slots > 8)
-        return YL_ERR_ARG;
-    for (int p = 0; p < world; ++p)
-        if (!windows[p] || ((uintptr_t)windows[p]) % 256 != 0) return YL_ERR_ARG;
-    yl_xchg *x = (yl_xchg *)calloc(1, sizeof(yl_xchg));
+    yl_xchg *x = (out && windows) ? xchg_new(device, rank, world, B, cap_out, slots, multicast != nullptr) : nullptr;
     if (!x) return YL_ERR_ARG;
-    x->device = device; x->rank = rank; x->world = world; x->B = B; x->cap_out = cap_out; x->slots = slots;
-    x->L = xchg_layout(world, B, cap_out, slots);
-    x->limit_ns = 5000000000ull;
-    // through the multicast mapping a rank sends 1/world of the bytes: 16 single-warp CTAs keep the switch busy (8 GPUs: 267 us per
-    // step with 16, 273 us with 64), the peer-store forms want 64
-    x->push_ctas = getenv("YL_XCHG_CTAS") ? atoi(getenv("YL_XCHG_CTAS")) : (multicast ? 16 : 64);
-    if (x->push_ctas < 1) x->push_ctas = 1;
-    x->bulk = !(getenv("YL_XCHG_BULK") && getenv("YL_XCHG_BULK")[0] == '0');
+    for (int p = 0; p < world; ++p)
+        if (!windows[p] || ((uintptr_t)windows[p]) % 256 != 0) { free(x); return YL_ERR_ARG; }
     x->external = true;
     for (int p = 0; p < world; ++p) { x->peer[p] = (char *)windows[p]; x->P.w[p] = window_of(x->peer[p], x->L); }
     x->window = x->peer[rank];
     x->mc = (char *)multicast;
     if (x->mc) x->MC = window_of(x->mc, x->L);
+    // only THIS rank's window is zeroed: the caller synchronises the ranks before the first push
     cudaError_t e = cudaSetDevice(device);
-    // flags, acks, epochs, counters of THIS rank's window start at zero (the caller synchronises the ranks before the first push)
-    if (e == cudaSuccess) e = cudaMemset(x->window + x->L.off_counts, 0, x->L.total - x->L.off_counts);
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e == cudaSuccess) e = xchg_init_window(x);
     if (e != cudaSuccess) { free(x); return YL_ERR_CUDA_BASE + (int)e; }
     x->connected = true;
     *out = x;
@@ -490,32 +367,10 @@ extern "C" int yl_xchg_push(yl_xchg *x, const float *rows, const int *counts, in
 {
     if (!x || !rows || !counts || slot < 0 || slot >= x->slots || !x->connected) return YL_ERR_ARG;
     if (((uintptr_t)rows) % 16 != 0) return YL_ERR_ARG;
-    const int grid = x->push_ctas;
-    if (x->mc && !x->bulk) {
-        k_xchg_push_mc<<<grid, XCHG_THREADS, 0, (cudaStream_t)stream>>>(x->P, x->MC, x->rank, x->world, x->B, x->cap_out, x->slots, slot, rows,
-                                                                        counts, (unsigned *)(x->window + x->L.off_done),
-                                                                        (int *)(x->window + x->L.off_status), x->limit_ns);
-        YL_LAUNCH_CHECK();
-        return YL_OK;
-    }
-    if (x->bulk) {
-        static bool attr_done = false;
-        const int smem = XB_STAGES * (int)XB_BYTES;
-        if (!attr_done) {
-            YL_CUDA_TRY(cudaFuncSetAttribute(k_xchg_push_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            attr_done = true;
-        }
-        XchgWindow mcw = x->MC;
-        if (!x->mc) mcw.rows = nullptr;
-        k_xchg_push_bulk<<<grid, 32, smem, (cudaStream_t)stream>>>(x->P, mcw, x->rank, x->world, x->B, x->cap_out, x->slots, slot, rows, counts,
-                                                                   (unsigned *)(x->window + x->L.off_done),
-                                                                   (int *)(x->window + x->L.off_status), x->limit_ns);
-        YL_LAUNCH_CHECK();
-        return YL_OK;
-    }
-    k_xchg_push<<<grid, XCHG_THREADS, 0, (cudaStream_t)stream>>>(x->P, x->rank, x->world, x->B, x->cap_out, x->slots, slot, rows, counts,
-                                                                 (unsigned *)(x->window + x->L.off_done),
-                                                                 (int *)(x->window + x->L.off_status), x->limit_ns);
+    // without a multicast mapping x->MC is all null and the kernel stores to every peer's window
+    k_xchg_push_bulk<<<x->push_ctas, 32, XB_SMEM, (cudaStream_t)stream>>>(x->P, x->MC, x->rank, x->world, x->B, x->cap_out, x->slots, slot,
+                                                                          rows, counts, (unsigned *)(x->window + x->L.off_done),
+                                                                          (int *)(x->window + x->L.off_status), x->limit_ns);
     YL_LAUNCH_CHECK();
     return YL_OK;
 }

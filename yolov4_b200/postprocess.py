@@ -244,11 +244,11 @@ class HeadPostprocessor:
     """Fixed-shape fused decode + filter + NMS with no host synchronisation: the serving / benchmark form.
 
     run(head_outputs) enqueues the whole chain on the current stream and returns (rows [B,cap_out,7], meta [3B])
-    device tensors owned by this object (overwritten by the next run).  With n_groups > 1 image groups are pipelined
-    over two streams (NMS of group g next to the streaming filter of group g+1); on B200 one group is fastest because
-    every kernel already fills the machine.  capture() records the chain into a CUDA graph bound to the given input
-    tensors; replay() launches it.  The head tensors may be float32, float16 or bfloat16 (see detect_raw); each run takes
-    the dtype from the tensors it is given.
+    device tensors owned by this object (overwritten by the next run).  The filter (flag + emit) of every image group runs
+    on the current stream and its NMS on a side stream, so with n_groups > 1 the NMS of group g runs next to the filter of
+    group g+1; on B200 one group is fastest because every kernel already fills the machine.  capture() records the chain into
+    a CUDA graph bound to the given input tensors; replay() launches it.  The head tensors may be float32, float16 or
+    bfloat16 (see detect_raw); each run takes the dtype from the tensors it is given.
 
     max_det caps the detections of every image as in detect_raw; cap_out then defaults to max_det rounded up to a multiple
     of 4, so the output (and a DetectionExchange built with hp.cap_out) is sized by the cap.  uncapped is a device int32 [B]
@@ -258,8 +258,7 @@ class HeadPostprocessor:
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
-                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, side_priority=0,
-                 mode="nms_side", max_det=None, agnostic=False):
+                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None, agnostic=False):
         self.max_det = _check_max_det(max_det)
         self.agnostic = _check_agnostic(agnostic)
         if cap_out is None:
@@ -281,9 +280,7 @@ class HeadPostprocessor:
             self.rows = torch.empty((self.B, self.cap_out, 7), dtype=torch.float32, device=self.device)
             self.meta = torch.zeros((3 * self.B,), dtype=torch.int32, device=self.device)
             self.uncapped = self.meta[:self.B] if self.max_det is None else torch.zeros((self.B,), dtype=torch.int32, device=self.device)
-            self.side = torch.cuda.Stream(device=self.device, priority=side_priority)
-            self.side2 = torch.cuda.Stream(device=self.device, priority=side_priority)
-        self.mode = mode
+            self.side = torch.cuda.Stream(device=self.device)
         self.graph = None
         # kernels launched per run(): per group flag + emit + segment NMS + fix-up (+ 1 memset node)
         self.launches_per_run = self.n_groups * 5
@@ -297,37 +294,19 @@ class HeadPostprocessor:
         rp = _cabi.ptrs([r.data_ptr() for r in raws])
         main = torch.cuda.current_stream(self.device)
         G = self.n_groups
-        fold_reset = (G == 1 and self.mode not in ("emit_side", "pipe3"))    # one group: the flag kernel zeroes the counters itself
+        fold_reset = G == 1                              # one group: the flag kernel zeroes the counters itself
         if not fold_reset:
             _cabi.check(L.yl_post_reset(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, main.cuda_stream))
         for g in range(G):
             i0, i1 = B * g // G, B * (g + 1) // G
-            if fold_reset:
-                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
-                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7, main.cuda_stream))
-                self.side.wait_stream(main)
-            elif self.mode in ("emit_side", "pipe3"):
-                # streaming flag kernels back to back on the main stream; everything else follows on the side stream
-                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
-                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 1, main.cuda_stream))
-                self.side.wait_stream(main)
-                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
-                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 2, self.side.cuda_stream))
-            else:
-                _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
-                                                  self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 3, main.cuda_stream))
-                self.side.wait_stream(main)
-            nms_stream = self.side
-            if self.mode == "pipe3":
-                # three-deep: flag(g+1) on the main stream, emit(g) on the first side stream, NMS + gather(g-1) on the second
-                self.side2.wait_stream(self.side)
-                nms_stream = self.side2
+            _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
+                                              self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7 if fold_reset else 3,
+                                              main.cuda_stream))
+            self.side.wait_stream(main)
             _cabi.check(L.yl_nms_ex(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
                                     int(self.agnostic), self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
-                                    None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, nms_stream.cuda_stream))
+                                    None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, self.side.cuda_stream))
         main.wait_stream(self.side)
-        if self.mode == "pipe3":
-            main.wait_stream(self.side2)
         return self.rows, self.meta
 
     def capture(self, head_outputs):

@@ -87,9 +87,9 @@ class DetectionExchange:
             dist.barrier(group=group)                      # every window is mapped before anybody pushes
 
     def _try_multicast(self, dev_index, group):
-        """Windows in torch symmetric memory with an NVSwitch multicast mapping: yl_xchg_push then issues one multimem.st per 16
-        bytes and the switch replicates it (a rank sends 1/world of the bytes).  torch only allocates and maps the memory; the
-        kernels are the library's.  All ranks agree on the outcome; any failure falls back to the CUDA IPC windows."""
+        """Windows in torch symmetric memory with an NVSwitch multicast mapping: yl_xchg_push then issues one bulk store to the
+        multicast mapping and the switch replicates it (a rank sends 1/world of the bytes).  torch only allocates and maps the
+        memory; the kernels are the library's.  All ranks agree on the outcome; any failure falls back to the CUDA IPC windows."""
         import ctypes
         ok, ptrs, mc = 1, None, 0
         try:
