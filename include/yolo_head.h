@@ -11,8 +11,10 @@
  *   - all device-pointer functions are stream-ordered on `stream` (a cudaStream_t passed as void*), do not
  *     allocate, do not synchronise, and are CUDA-graph capturable.
  *   - fp32 everywhere (the reference trains and evaluates with apex O0, README.md:106,112), except the head tensors of the
- *     fused detection path (yl_filter_raw_typed, yl_context_create_typed), which may also be fp16 or bf16 as a model run
- *     with .half() or under autocast produces them: they are widened exactly to fp32 and the fp32 spec applies from there.
+ *     fused detection path (yl_filter_raw_typed, yl_context_create_typed) and of the fused loss (yl_loss_forward_typed,
+ *     yl_loss_forward_chained_typed, yl_loss_backward_typed), which may also be fp16 or bf16 as a model run with .half(), under
+ *     autocast or apex O1/O2 produces them: they are widened exactly to fp32 and the fp32 spec applies from there; the loss
+ *     gradient is then written in the head's element type.
  *   - sigmoid / exp / log are the "spec math" of DESIGN.md section 4 (fixed IEEE op sequences), so results are
  *     bit-reproducible and identical to the CPU oracle.
  */
@@ -36,7 +38,7 @@ extern "C" {
 #define YL_MAX_CLASSES 128
 #define YL_ABI_VERSION 1
 
-/* element type of the head tensors of the fused detection path */
+/* element type of the head tensors of the fused detection path and of the fused loss */
 #define YL_DTYPE_F32 0
 #define YL_DTYPE_F16 1
 #define YL_DTYPE_BF16 2
@@ -251,6 +253,25 @@ int yl_loss_forward_chained(const float *raw, const float *labels, int B, int F,
                     yl_stream_t stream);
 int yl_loss_backward(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
                      int B, int F, int K, int C, float *grad_raw, yl_stream_t stream);
+/* The three loss calls for head tensors of element type `dtype` (YL_DTYPE_*); yl_loss_forward, yl_loss_forward_chained and
+ * yl_loss_backward are these calls with YL_DTYPE_F32.  An unknown dtype returns YL_ERR_ARG before any CUDA call.
+ *   forward    raw [B, 3*(5+C), F, F] of that type.  Every fp16 / bf16 value (subnormals, +-0, +-inf and NaN included) has an
+ *              exact fp32 image: each element is widened on load and the fp32 loss of the fp32 call applies unchanged, so loss4
+ *              equals that of the fp32 call on the widened tensor up to the order of the fp64 sums.  The saved tables (gobj,
+ *              tcell_all, mcell, mgrad) stay fp32 with the same shapes, and the aliasing rule above is unchanged.
+ *   backward   grad_raw [B, 3*(5+C), F, F] of that type: every element is the fp32 call's value fl32(d * upstream[0]), rounded
+ *              once to nearest-even into the type (so a large loss scale overflows to +-inf where the rounded value does).
+ * This is not the reference's own half-precision arithmetic; it is the fp32 loss of the widened heads. */
+int yl_loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                          const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                          double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                          yl_stream_t stream);
+int yl_loss_forward_chained_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                                  const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                                  double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                                  yl_stream_t stream);
+int yl_loss_backward_typed(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
+                           int B, int F, int K, int C, void *grad_raw, int dtype, yl_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Host-buffer entry (what a non-Python caller binds; also the bench's end-to-end leg): raw head tensors in

@@ -14,6 +14,10 @@
 //   k_loss_bwd_*   grad_raw = upstream * (objectness plane from k_loss_obj, matched cells from the table); the rest of
 //                  grad_raw is the zero background (cudaMemsetAsync).
 //
+// 16-bit heads (fp16 / bf16): the forward kernels widen every element on load (yl_common.cuh: every 16-bit value has an exact
+// fp32 image) and the fp32 arithmetic below applies unchanged; the backward kernels form the same fp32 product and round it once
+// into the head's element type, so a 16-bit gradient is the fp32 path's gradient on the widened head, rounded to nearest-even.
+//
 // Per-term arithmetic is fp32 like the reference's (ATen binary_cross_entropy: (t-1) max(log(1-x), -100) - t max(log x, -100),
 // backward (x-t)/max((1-x) x, 1e-12); mse_loss); sums are accumulated in fp64.  Parity: loss and gradient within 1e-5 /
 // 2e-5 relative of the reference (tests/golden/loss.npz), not bit-exact (the reference's reduction order is unspecified).
@@ -50,8 +54,14 @@ __device__ __forceinline__ double warp_sum(double v)
 
 struct LossAnchors { AnchorSet an; float maw[3], mah[3]; };          // all nine / the layer's three anchors, grid units
 
+// fp32 -> element type of the gradient, round to nearest-even (overflow to +-inf)
+__device__ __forceinline__ float narrow(float x, float *) { return x; }
+__device__ __forceinline__ __half narrow(float x, __half *) { return __float2half_rn(x); }
+__device__ __forceinline__ __nv_bfloat16 narrow(float x, __nv_bfloat16 *) { return __float2bfloat16_rn(x); }
+
+template <typename T>
 __global__ void __launch_bounds__(LS_THREADS)
-k_loss_match(const float *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
+k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
              double *__restrict__ loss4, int *__restrict__ tcell_all, int *__restrict__ mcell, float *__restrict__ mgrad,
              int *__restrict__ status)
 {
@@ -84,7 +94,7 @@ k_loss_match(const float *__restrict__ raw, const float *__restrict__ labels, in
         for (int u = t + 1 + lane; u < n; u += 32) overridden |= (tcell[u] == cell);
         if (__any_sync(0xFFFFFFFFu, overridden)) continue;
         const int a = cell / F2, r = cell - a * F2;
-        const float *cp = raw + ((size_t)(b * 3 + a) * nch) * F2 + r;   // channel k of this cell at cp[k * F2]
+        const T *cp = raw + ((size_t)(b * 3 + a) * nch) * F2 + r;       // channel k of this cell at cp[k * F2]
         const float tw = tb[t][2], th = tb[t][3];
         const float sc = __fsqrt_rn(__fsub_rn(2.0f, __fdiv_rn(__fdiv_rn(__fmul_rn(tw, th), (float)F), (float)F)));   // :337
         const float w2 = __fmul_rn(sc, sc);                                                                          // :417
@@ -99,7 +109,7 @@ k_loss_match(const float *__restrict__ raw, const float *__restrict__ labels, in
         }
         for (int kk = lane; kk < nk; kk += 32) {
             const int k = kk < 4 ? kk : kk + 1;
-            const float v = cp[(size_t)k * F2];
+            const float v = widen(cp[(size_t)k * F2]);
             float g;
             if (kk < 2) {                                              // xy: weighted BCE (:421)
                 const float x = spec_sigmoidf(v);
@@ -144,8 +154,9 @@ k_loss_match(const float *__restrict__ raw, const float *__restrict__ labels, in
     pdl_wait();
 }
 
+template <typename T>
 __global__ void __launch_bounds__(LS_THREADS)
-k_loss_obj(const float *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
+k_loss_obj(const T *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
            float ignore_thre, const int *__restrict__ tcell_all, double *__restrict__ loss4, float *__restrict__ gobj)
 {
     __shared__ __align__(16) float tb[TG_MAXK][4];
@@ -170,9 +181,9 @@ k_loss_obj(const float *__restrict__ raw, const float *__restrict__ labels, int 
     if (cell < cells) {
         const int a = cell / F2, r = cell - a * F2;
         const int j = r / F, i = r - j * F;
-        const float *cp = raw + ((size_t)(b * 3 + a) * nch) * F2 + r;
-        const float t0 = cp[0], t1 = cp[(size_t)F2], t2 = cp[2 * (size_t)F2], t3 = cp[3 * (size_t)F2];
-        t4 = cp[4 * (size_t)F2];
+        const T *cp = raw + ((size_t)(b * 3 + a) * nch) * F2 + r;
+        const float t0 = widen(cp[0]), t1 = widen(cp[(size_t)F2]), t2 = widen(cp[2 * (size_t)F2]), t3 = widen(cp[3 * (size_t)F2]);
+        t4 = widen(cp[4 * (size_t)F2]);
         if (n > 0) {                                                   // :225-227: no labels => obj_mask stays 1
             // pred exactly as the train-mode YOLOLayer forms it (yololayer.py:126-134): grid units, no stride
             float sx, sy, ew, eh;
@@ -215,20 +226,22 @@ k_loss_obj(const float *__restrict__ raw, const float *__restrict__ labels, int 
     }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(LS_THREADS)
 k_loss_bwd_obj(const float *__restrict__ gobj, const float *__restrict__ upstream, int F2, int C, long n_cells,
-               float *__restrict__ grad_raw)
+               T *__restrict__ grad_raw)
 {
     const long c = (long)blockIdx.x * LS_THREADS + threadIdx.x;       // cell index over [B*3, F2]
     if (c >= n_cells) return;
     const long ba = c / F2;
     const int r = (int)(c - ba * F2);
-    grad_raw[((size_t)ba * (5 + C) + 4) * F2 + r] = __fmul_rn(gobj[c], upstream[0]);
+    grad_raw[((size_t)ba * (5 + C) + 4) * F2 + r] = narrow(__fmul_rn(gobj[c], upstream[0]), grad_raw);
 }
 
+template <typename T>
 __global__ void __launch_bounds__(LS_THREADS)
 k_loss_bwd_sparse(const int *__restrict__ mcell, const float *__restrict__ mgrad, const float *__restrict__ upstream,
-                  int F2, int K, int C, int n_gt, float *__restrict__ grad_raw)
+                  int F2, int K, int C, int n_gt, T *__restrict__ grad_raw)
 {
     const int gt = blockIdx.x * (LS_THREADS / 32) + (threadIdx.x >> 5);   // one warp per (image, GT slot)
     if (gt >= n_gt) return;
@@ -236,9 +249,9 @@ k_loss_bwd_sparse(const int *__restrict__ mcell, const float *__restrict__ mgrad
     if (cell < 0) return;
     const int lane = threadIdx.x & 31, b = gt / K, nch = 5 + C, nk = 4 + C;
     const int a = cell / F2, r = cell - a * F2;
-    float *gp = grad_raw + ((size_t)(b * 3 + a) * nch) * F2 + r;
+    T *gp = grad_raw + ((size_t)(b * 3 + a) * nch) * F2 + r;
     const float up = upstream[0];
-    for (int kk = lane; kk < nk; kk += 32) gp[(size_t)(kk < 4 ? kk : kk + 1) * F2] = __fmul_rn(mgrad[(size_t)gt * nk + kk], up);
+    for (int kk = lane; kk < nk; kk += 32) gp[(size_t)(kk < 4 ? kk : kk + 1) * F2] = narrow(__fmul_rn(mgrad[(size_t)gt * nk + kk], up), gp);
 }
 
 static int fill_anchors(LossAnchors &A, const float *anchors_px, const int *anchor_mask3, float stride)
@@ -260,7 +273,8 @@ static int fill_anchors(LossAnchors &A, const float *anchors_px, const int *anch
 
 using namespace yl;
 
-static int loss_forward_impl(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,
+template <typename T>
+static int loss_forward_impl(const T *raw, const float *labels, int B, int F, int K, int C, int layer_no,
                              const float *anchors_px, const int *anchor_mask3, float ignore_thre,
                              double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                              int chained, yl_stream_t stream)
@@ -278,12 +292,32 @@ static int loss_forward_impl(const float *raw, const float *labels, int B, int F
     // own k_loss_obj (chained != 0): behind a foreign kernel (the producer of raw or labels, the fill of loss4) it is a
     // normal launch, fully ordered after everything earlier on the stream.
     const bool pdl = pdl_enabled();
-    YL_CUDA_TRY(launch_after(k_loss_match, dim3(B, 8), dim3(LS_THREADS), 0, st, pdl && chained != 0, raw, labels, F, K, C, stride, A,
+    YL_CUDA_TRY(launch_after(k_loss_match<T>, dim3(B, 8), dim3(LS_THREADS), 0, st, pdl && chained != 0, raw, labels, F, K, C, stride, A,
                              loss4, tcell_all, mcell, mgrad, status));
     dim3 grid((3 * F * F + LS_THREADS - 1) / LS_THREADS, B);
-    YL_CUDA_TRY(launch_after(k_loss_obj, grid, dim3(LS_THREADS), 0, st, pdl, raw, labels, F, K, C, stride, A, ignore_thre,
+    YL_CUDA_TRY(launch_after(k_loss_obj<T>, grid, dim3(LS_THREADS), 0, st, pdl, raw, labels, F, K, C, stride, A, ignore_thre,
                              (const int *)tcell_all, loss4, gobj));
     return YL_OK;
+}
+
+static int loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                              const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                              double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                              int chained, yl_stream_t stream)
+{
+    switch (dtype) {
+    case YL_DTYPE_F32:
+        return loss_forward_impl((const float *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4,
+                                 gobj, tcell_all, mcell, mgrad, status, chained, stream);
+    case YL_DTYPE_F16:
+        return loss_forward_impl((const __half *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4,
+                                 gobj, tcell_all, mcell, mgrad, status, chained, stream);
+    case YL_DTYPE_BF16:
+        return loss_forward_impl((const __nv_bfloat16 *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
+                                 loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+    default:
+        return YL_ERR_ARG;
+    }
 }
 
 extern "C" int yl_loss_forward(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -291,8 +325,8 @@ extern "C" int yl_loss_forward(const float *raw, const float *labels, int B, int
                                double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                yl_stream_t stream)
 {
-    return loss_forward_impl(raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj, tcell_all,
-                             mcell, mgrad, status, 0, stream);
+    return loss_forward_typed(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
+                              tcell_all, mcell, mgrad, status, 0, stream);
 }
 
 extern "C" int yl_loss_forward_chained(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -300,23 +334,57 @@ extern "C" int yl_loss_forward_chained(const float *raw, const float *labels, in
                                        double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                        yl_stream_t stream)
 {
-    return loss_forward_impl(raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj, tcell_all,
-                             mcell, mgrad, status, 1, stream);
+    return loss_forward_typed(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
+                              tcell_all, mcell, mgrad, status, 1, stream);
+}
+
+extern "C" int yl_loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                                     const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                                     double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                                     yl_stream_t stream)
+{
+    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
+                              tcell_all, mcell, mgrad, status, 0, stream);
+}
+
+extern "C" int yl_loss_forward_chained_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C,
+                                             int layer_no, const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                                             double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                                             yl_stream_t stream)
+{
+    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
+                              tcell_all, mcell, mgrad, status, 1, stream);
+}
+
+template <typename T>
+static int loss_backward_impl(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
+                              int B, int F, int K, int C, T *grad_raw, cudaStream_t st)
+{
+    const int F2 = F * F;
+    const long n_cells = (long)B * 3 * F2;
+    YL_CUDA_TRY(cudaMemsetAsync(grad_raw, 0, sizeof(T) * (size_t)n_cells * (5 + C), st));
+    k_loss_bwd_obj<T><<<(unsigned)((n_cells + LS_THREADS - 1) / LS_THREADS), LS_THREADS, 0, st>>>(gobj, upstream, F2, C, n_cells, grad_raw);
+    YL_LAUNCH_CHECK();
+    const int n_gt = B * K;
+    k_loss_bwd_sparse<T><<<(n_gt + LS_THREADS / 32 - 1) / (LS_THREADS / 32), LS_THREADS, 0, st>>>(mcell, mgrad, upstream, F2, K, C, n_gt,
+                                                                                                grad_raw);
+    YL_LAUNCH_CHECK();
+    return YL_OK;
+}
+
+extern "C" int yl_loss_backward_typed(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
+                                      int B, int F, int K, int C, void *grad_raw, int dtype, yl_stream_t stream)
+{
+    if (dtype != YL_DTYPE_F32 && dtype != YL_DTYPE_F16 && dtype != YL_DTYPE_BF16) return YL_ERR_ARG;
+    if (!gobj || !mcell || !mgrad || !upstream || !grad_raw || B <= 0 || F <= 0 || K <= 0 || C <= 0) return YL_ERR_ARG;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == YL_DTYPE_F16) return loss_backward_impl(gobj, mcell, mgrad, upstream, B, F, K, C, (__half *)grad_raw, st);
+    if (dtype == YL_DTYPE_BF16) return loss_backward_impl(gobj, mcell, mgrad, upstream, B, F, K, C, (__nv_bfloat16 *)grad_raw, st);
+    return loss_backward_impl(gobj, mcell, mgrad, upstream, B, F, K, C, (float *)grad_raw, st);
 }
 
 extern "C" int yl_loss_backward(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
                                 int B, int F, int K, int C, float *grad_raw, yl_stream_t stream)
 {
-    if (!gobj || !mcell || !mgrad || !upstream || !grad_raw || B <= 0 || F <= 0 || K <= 0 || C <= 0) return YL_ERR_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int F2 = F * F;
-    const long n_cells = (long)B * 3 * F2;
-    YL_CUDA_TRY(cudaMemsetAsync(grad_raw, 0, sizeof(float) * (size_t)n_cells * (5 + C), st));
-    k_loss_bwd_obj<<<(unsigned)((n_cells + LS_THREADS - 1) / LS_THREADS), LS_THREADS, 0, st>>>(gobj, upstream, F2, C, n_cells, grad_raw);
-    YL_LAUNCH_CHECK();
-    const int n_gt = B * K;
-    k_loss_bwd_sparse<<<(n_gt + LS_THREADS / 32 - 1) / (LS_THREADS / 32), LS_THREADS, 0, st>>>(mcell, mgrad, upstream, F2, K, C, n_gt,
-                                                                                             grad_raw);
-    YL_LAUNCH_CHECK();
-    return YL_OK;
+    return yl_loss_backward_typed(gobj, mcell, mgrad, upstream, B, F, K, C, grad_raw, YL_DTYPE_F32, stream);
 }

@@ -5,7 +5,9 @@ forward(outputs, targets) restates the reference's loss arithmetic (yololoss.py:
 class can replace the reference's criterion as a whole, dense tensors and all.
 fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh) is SURVEY.md's "next" row N2: the same loss value and
 its gradient with respect to the raw head tensors from yl_loss_forward / yl_loss_backward, without materialising
-output / pred / target / masks; the padded labels are cast and uploaded once for the three scales (row N4).
+output / pred / target / masks; the padded labels are cast and uploaded once for the three scales (row N4).  The fused loss
+also takes fp16 / bf16 head tensors (autocast, apex O1/O2): widened exactly to fp32 inside the kernels, gradients in the
+head's dtype.
 """
 import numpy as np
 import torch
@@ -16,6 +18,21 @@ from . import _cabi
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
+
+
+# head tensor dtypes of the fused loss -> YL_DTYPE_* (include/yolo_head.h)
+_DTYPE_CODES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
+
+def _head_dtype_code(raws):
+    """YL_DTYPE_* of the fused loss's head tensors: float32, float16 or bfloat16 CUDA tensors, all of one dtype.  Raises
+    TypeError before any CUDA work."""
+    for r in raws:
+        if not isinstance(r, torch.Tensor) or not r.is_cuda or r.dtype not in _DTYPE_CODES:
+            raise TypeError("fused YOLO loss needs float32, float16 or bfloat16 CUDA head tensors; there is no CPU fallback")
+        if r.dtype != raws[0].dtype:
+            raise TypeError("fused YOLO loss head tensors must share one dtype, got %s and %s" % (raws[0].dtype, r.dtype))
+    return _DTYPE_CODES[raws[0].dtype]
 
 
 class _LabelUploader:
@@ -169,15 +186,20 @@ class YOLOLoss(nn.Module):
 
 
 class _FusedYoloLoss(torch.autograd.Function):
-    """N2: raw head tensors + padded labels -> the reference's YOLOLoss.forward value, gradient straight to the raw tensors."""
+    """N2: raw head tensors + padded labels -> the reference's YOLOLoss.forward value, gradient straight to the raw tensors
+    (in the heads' dtype: fp32, fp16 or bf16)."""
 
     @staticmethod
     def forward(ctx, labels, anchors, anchor_mask, ignore_thresh, n_classes, *raws):
         L = _cabi.lib()
+        C = int(n_classes)
+        dtype = _head_dtype_code(raws)
+        for r in raws:
+            if r.dim() != 4 or r.shape[1] != 3 * (5 + C) or r.shape[0] != labels.shape[0]:
+                raise TypeError("fused YOLO loss needs CUDA head tensors [B, 3*(5+C), F, F]; there is no CPU fallback")
         dev = raws[0].device
         lab = upload_labels(labels, dev)
         B, K = int(lab.shape[0]), int(lab.shape[1])
-        C = int(n_classes)
         anch = _cabi.floats([v for wh in anchors for v in wh])
         saved, keep = [], []
         with torch.cuda.device(dev):
@@ -185,8 +207,6 @@ class _FusedYoloLoss(torch.autograd.Function):
             status = torch.zeros(1, dtype=torch.int32, device=dev)
             calls = []
             for l, r in enumerate(raws):
-                if not r.is_cuda or r.dtype != torch.float32 or r.dim() != 4 or r.shape[1] != 3 * (5 + C) or r.shape[0] != B:
-                    raise TypeError("fused YOLO loss needs float32 CUDA head tensors [B, 3*(5+C), F, F]; there is no CPU fallback")
                 rc = r.detach().contiguous()
                 F = int(rc.shape[2])
                 gobj = torch.empty((B, 3, F, F), dtype=torch.float32, device=dev)
@@ -199,12 +219,13 @@ class _FusedYoloLoss(torch.autograd.Function):
             # every foreign kernel (contiguous copies, the fills of loss4 / status) is enqueued by now: the calls below are back
             # to back on the stream, so the second and later ones may be launched programmatically behind their predecessor
             for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):
-                fn = L.yl_loss_forward if i == 0 else L.yl_loss_forward_chained
-                _cabi.check(fn(rc.data_ptr(), lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(anchor_mask[l]),
+                fn = L.yl_loss_forward_typed if i == 0 else L.yl_loss_forward_chained_typed
+                _cabi.check(fn(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(anchor_mask[l]),
                                float(np.float32(ignore_thresh)), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
                                mcell.data_ptr(), mgrad.data_ptr(), status.data_ptr(), _stream()))
         ctx.save_for_backward(*saved)
         ctx.shapes = [tuple(r.shape) for r in raws]
+        ctx.dtype, ctx.dtype_code = raws[0].dtype, dtype
         ctx.K, ctx.C = K, C
         ctx.status = status
         ctx.loss4 = loss4
@@ -220,9 +241,9 @@ class _FusedYoloLoss(torch.autograd.Function):
             for l, shp in enumerate(ctx.shapes):
                 gobj, mcell, mgrad = saved[3 * l:3 * l + 3]
                 B, _, F, _ = shp
-                g = torch.empty(shp, dtype=torch.float32, device=up.device)
-                _cabi.check(L.yl_loss_backward(gobj.data_ptr(), mcell.data_ptr(), mgrad.data_ptr(), up.data_ptr(), B, F, ctx.K, ctx.C,
-                                               g.data_ptr(), _stream()))
+                g = torch.empty(shp, dtype=ctx.dtype, device=up.device)        # written in the head's dtype, no fp32 copy
+                _cabi.check(L.yl_loss_backward_typed(gobj.data_ptr(), mcell.data_ptr(), mgrad.data_ptr(), up.data_ptr(), B, F, ctx.K,
+                                                     ctx.C, g.data_ptr(), ctx.dtype_code, _stream()))
                 grads.append(g)
         return (None, None, None, None, None) + tuple(grads)
 
@@ -231,14 +252,24 @@ def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7):
     """N2 (SURVEY.md 8f): the value of `YOLOLoss(cfg, ignore_thresh)([YOLOLayer_l.train()(x_l)], {'padded_labels': labels})`
     (yolo/model/yololoss.py:373-443 on top of yololayer.py:122-145) computed from the three raw head tensors without
     materialising output / pred / target / masks; differentiable with respect to the head tensors.
-    Loss and gradient agree with the reference within 1e-5 / 2e-5 relative (not bit-exact: reduction order)."""
+    Loss and gradient agree with the reference within 1e-5 / 2e-5 relative (not bit-exact: reduction order).
+
+    The heads may be float32, float16 or bfloat16 CUDA tensors of one dtype (a model under torch.autocast or apex O1/O2); the
+    loss is always a float32 scalar.  A 16-bit head is widened exactly to fp32 inside the kernels, so the loss is that of
+    `[h.float() for h in head_outputs]` up to the order of the fp64 sums, and its gradient has the head's dtype: bit for bit
+    the fp32 path's gradient on the widened heads (with the same upstream gradient, e.g. a GradScaler's scale) rounded to
+    nearest-even, overflow to +-inf included.  This is not the reference's own half-precision arithmetic.  Mixed dtypes,
+    float64 and CPU heads raise TypeError before any CUDA work."""
     return _FusedYoloLoss.apply(padded_labels, cfg['ANCHORS'], cfg['ANCHOR_MASK'], ignore_thresh, cfg['N_CLASSES'], *head_outputs)
 
 
 def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0.7, layers=None):
     """The four sums (loss_xy, loss_wh, loss_obj, loss_cls; yololoss.py:421-427) over the given layers as a float64[4] device
-    tensor, no autograd.  `layers[i]` is the layer number of head_outputs[i] (default 0, 1, 2)."""
+    tensor, no autograd.  `layers[i]` is the layer number of head_outputs[i] (default 0, 1, 2).  The heads may be float32,
+    float16 or bfloat16 CUDA tensors of one dtype: a 16-bit head gives the components of its widened fp32 copy (up to the order
+    of the fp64 sums); mixed dtypes, float64 and CPU heads raise TypeError before any CUDA work."""
     L = _cabi.lib()
+    dtype = _head_dtype_code(head_outputs)
     dev = head_outputs[0].device
     lab = upload_labels(padded_labels, dev)
     B, K = int(lab.shape[0]), int(lab.shape[1])
@@ -259,8 +290,8 @@ def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0
             calls.append((rc, F, int(l), gobj, tcell, mcell, mgrad))
             keep += [rc, gobj, tcell, mcell, mgrad]
         for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):     # back to back: see _FusedYoloLoss.forward
-            fn = L.yl_loss_forward if i == 0 else L.yl_loss_forward_chained
-            _cabi.check(fn(rc.data_ptr(), lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(cfg['ANCHOR_MASK'][l]),
+            fn = L.yl_loss_forward_typed if i == 0 else L.yl_loss_forward_chained_typed
+            _cabi.check(fn(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(cfg['ANCHOR_MASK'][l]),
                            float(np.float32(ignore_thresh)), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
                            mcell.data_ptr(), mgrad.data_ptr(), None, _stream()))
     return loss4
