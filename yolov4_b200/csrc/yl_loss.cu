@@ -8,7 +8,9 @@
 //
 //   k_loss_match   per image: GT -> cell assignment (:249-265), then for every matched cell (last writer per cell, class
 //                  one-hots accumulated over colliding GTs, SURVEY.md 7-9) the xy / wh / cls terms of :417-427 and their
-//                  derivatives with respect to the raw logits, kept in a compact per-GT table.
+//                  derivatives with respect to the raw logits, kept in a compact per-GT table.  A class id sets channel
+//                  5 + cls with Python's negative-index wrap, as build_target does (class_channel): a negative id marks
+//                  another class, or overwrites the last GT's x / y / w / h target with 1 (channel 4 stays 1).
 //   k_loss_obj     per cell: decode the box from tx,ty,tw,th (5 of the 85 planes are read), ignore mask (:276-294),
 //                  objectness BCE (:425) and d/d(raw objectness).
 //   k_loss_bwd_*   grad_raw = upstream * (objectness plane from k_loss_obj, matched cells from the table); the rest of
@@ -28,16 +30,18 @@ namespace yl {
 
 constexpr int LS_THREADS = 256;
 
+// The clamps propagate NaN (nanmaxf, not fmaxf): a NaN probability gives a NaN term, as the max of ATen's CPU kernel does,
+// and as the NaN gradient of the same cell already says.
 __device__ __forceinline__ float bce_term(float x, float t)
 {
-    const float lx = fmaxf(spec_logf(x), -100.0f), l1x = fmaxf(spec_logf(__fsub_rn(1.0f, x)), -100.0f);
+    const float lx = nanmaxf(spec_logf(x), -100.0f), l1x = nanmaxf(spec_logf(__fsub_rn(1.0f, x)), -100.0f);
     return __fsub_rn(__fmul_rn(__fsub_rn(t, 1.0f), l1x), __fmul_rn(t, lx));
 }
 // bce_term for t = 1 (one) or t = 0: the other logarithm is clamped to [-100, 0] and multiplied by zero, so the term is
 // -max(log x, -100) resp. -max(log(1 - x), -100) -- the same value (NaN included) for one spec_logf instead of two.
 __device__ __forceinline__ float bce_term01(float x, bool one)
 {
-    const float l = fmaxf(spec_logf(one ? x : __fsub_rn(1.0f, x)), -100.0f);
+    const float l = nanmaxf(spec_logf(one ? x : __fsub_rn(1.0f, x)), -100.0f);
     return __fsub_rn(0.0f, l);
 }
 __device__ __forceinline__ float bce_grad(float x, float t)
@@ -102,28 +106,38 @@ k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F,
         if (lane == 0) mcell[(size_t)b * K + t] = cell;
         // GTs that share the cell (usually just this one): bit u of same[u >> 5]
         unsigned same[TG_MAXK / 32];
+        bool bad_class = false;
 #pragma unroll
         for (int w = 0; w < TG_MAXK / 32; ++w) {
             const int u = 32 * w + lane;
-            same[w] = (32 * w < n) ? __ballot_sync(0xFFFFFFFFu, u < n && tcell[u] == cell) : 0u;
+            const bool s = u < n && tcell[u] == cell;
+            same[w] = (32 * w < n) ? __ballot_sync(0xFFFFFFFFu, s) : 0u;
+            if (s) {
+                const int ku = class_channel(tcls[u], nch);
+                bad_class |= (ku < 0 || ku >= nch);
+            }
         }
+        if (bad_class && status) atomicExch(status, 1);                // the reference raises IndexError at :369
+        // The cell's last GT (this one) writes the xy / wh targets; its class channel overwrites one of them when its id
+        // wraps onto 0..3, and wrapping onto 4 (objectness, already 1) changes nothing.
+        const int kt = class_channel(tcls[t], nch);
         for (int kk = lane; kk < nk; kk += 32) {
             const int k = kk < 4 ? kk : kk + 1;
             const float v = widen(cp[(size_t)k * F2]);
             float g;
             if (kk < 2) {                                              // xy: weighted BCE (:421)
                 const float x = spec_sigmoidf(v);
-                const float tg = __fsub_rn(tb[t][kk], (float)(short)(int)tb[t][kk]);                                  // :346,349
+                const float tg = (kt == kk) ? 1.0f : __fsub_rn(tb[t][kk], (float)(short)(int)tb[t][kk]);              // :346,349
                 acc_xy += (double)__fmul_rn(bce_term(x, tg), w2);
                 g = __fmul_rn(__fmul_rn(__fmul_rn(bce_grad(x, tg), w2), x), __fsub_rn(1.0f, x));
             } else if (kk < 4) {                                       // wh: MSE / 2 on the scaled raw logits (:423)
                 const float anc = (kk == 2) ? A.maw[tanc[t]] : A.mah[tanc[t]];
-                const float tg = spec_logf(__fadd_rn(__fdiv_rn(kk == 2 ? tw : th, anc), 1e-16f));                     // :362,365
+                const float tg = (kt == kk) ? 1.0f : spec_logf(__fadd_rn(__fdiv_rn(kk == 2 ? tw : th, anc), 1e-16f)); // :362,365
                 const float d = __fsub_rn(__fmul_rn(v, sc), __fmul_rn(tg, sc));
                 acc_wh += 0.5 * (double)d * (double)d;
                 g = __fmul_rn(d, sc);
             } else {                                                   // classes: BCE against the union of the cell's one-hots (:427)
-                const int kc = kk - 4;
+                const int kc = kk + 1;                                 // channel 5 + class
                 float tg = 0.0f;
 #pragma unroll
                 for (int w = 0; w < TG_MAXK / 32; ++w) {
@@ -131,9 +145,7 @@ k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F,
                     while (m) {
                         const int u = 32 * w + __ffs(m) - 1;
                         m &= m - 1u;
-                        const int cu = (int)(short)(int)tcls[u];                                                      // :369
-                        if (cu == kc) tg = 1.0f;
-                        if ((cu < 0 || cu >= C) && status) atomicExch(status, 1);   // a class id that would index outside 5..5+C
+                        if (class_channel(tcls[u], nch) == kc) tg = 1.0f;                                             // :369
                     }
                 }
                 const float x = spec_sigmoidf(v);

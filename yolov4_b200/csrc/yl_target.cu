@@ -4,7 +4,9 @@
 //   k_target_scatter   per image: GT <-> 9-anchor IoU argmax (:249-265) and the assignment of
 //                      obj_mask / tgt_mask / tgt_scale / target at the matched cells (:304-369),
 //                      resolving same-cell collisions the way the reference's sequential loop does:
-//                      scalar fields last-writer-wins, class one-hots accumulate (SURVEY.md 7-9).
+//                      scalar fields last-writer-wins, class one-hots accumulate (SURVEY.md 7-9).  A class id writes
+//                      channel 5 + cls with Python's negative-index wrap (class_channel): a negative id lands on another
+//                      class or on the box targets 0..3 / objectness 4.
 // The dense zero background of target / tgt_mask / tgt_scale (:156-167, 99.9 % of the 16 MB/image this path writes) is
 // stored by k_target_objmask itself, 128 bits at a time, before it computes its cells' IoUs: the pass runs at the pace
 // of the HBM writes and the IoU arithmetic hides underneath instead of following three memsets.
@@ -142,10 +144,11 @@ k_target_scatter(const __grid_constant__ TargetParams P)
                 tg[3] = spec_logf(__fadd_rn(__fdiv_rn(th, an.h[an.mask[a]]), 1e-16f));        // :365
             }
             tg[4] = 1.0f;                                                                     // :367
-            int kc = 5 + (int)(short)(int)tcls[t];                                            // :369
-            if (kc < 0) kc += nch;
+            const int kc = class_channel(tcls[t], nch);                                       // :369
+            // An overridden GT's write to channels 0..4 is a no-op or overwritten by the cell's last GT in the reference's
+            // order; skipping it keeps it from racing with that GT's writes (another warp, possibly another CTA).
             if (kc < 0 || kc >= nch) { if (status) atomicExch(status, 1); }
-            else tg[kc] = 1.0f;
+            else if (!overridden || kc >= 5) tg[kc] = 1.0f;
         }
     }
 }

@@ -41,6 +41,15 @@ __device__ __forceinline__ bool bounded(float v) { return fabsf(v) <= 1e18f; }  
 
 struct AnchorSet { float w[9], h[9]; int mask[3]; };
 
+// Channel of a GT's class one-hot in its cell's 5+C target row, target[..., 5 + cls] = 1 (:369): int16 truncation of the
+// class id, then Python's negative-index wrap, so negative ids land on channels nch-1..0 (0..4: the box / objectness
+// targets).  Valid when 0 <= channel < nch; the reference raises IndexError otherwise.
+__device__ __forceinline__ int class_channel(float cls, int nch)
+{
+    const int k = 5 + (int)(short)(int)cls;
+    return k < 0 ? k + nch : k;
+}
+
 // GT t of an image -> the cell it is assigned to on this layer, or -1 (yololoss.py:249-265, :206-207, :257): IoU of
 // (0,0,w,h) against the nine (0,0,aw,ah) reference anchors, xyxy=True form; first max wins, NaN counts as the maximum
 // (torch.argmax); the GT belongs to the layer when the best anchor is one of the layer's three; int16 truncation of the
