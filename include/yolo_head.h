@@ -174,6 +174,23 @@ int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, fl
  * Image groups (img_first / img_count) use only their own images' slices of the workspace. */
 int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
               float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream);
+/* yl_nms_ex with DIoU-NMS (Zheng et al., AAAI 2020; the DIoU-NMS of the YOLOv4 paper).  The candidates, their order, the rows,
+ * their order in the output, max_det and the capacity protocol are those of yl_nms_ex (per class, or agnostic with
+ * agnostic = 1); only the suppression decision changes.  A candidate a is dropped by an earlier kept box b (both x1,y1,x2,y2)
+ * when, every operation one fp32 rounding in this order and max / min propagating NaN:
+ *   iou = the literal NaN-propagating IoU of utils.py:71-77 (the decision of yl_nms)
+ *   dx  = (a.x1 + a.x2) * 0.5 - (b.x1 + b.x2) * 0.5        dy = (a.y1 + a.y2) * 0.5 - (b.y1 + b.y2) * 0.5
+ *   cw  = max(a.x2, b.x2) - min(a.x1, b.x1)                 ch = max(a.y2, b.y2) - min(a.y1, b.y1)
+ *   pen = (dx*dx + dy*dy) / (cw*cw + ch*ch)
+ *   suppress  <=>  (iou - pen) >= nms_thre
+ * ">=" is the paper's rule and the reference's rule for IoU (darknet's diounms uses ">" and an exponent beta_nms, which this
+ * call does not have).  pen >= 0 or NaN, so a pair the IoU rule keeps apart is never suppressed here: a NaN penalty (c^2 = 0,
+ * inf / inf) decides "keep", and a degenerate box (NaN, zero or negative extent) never suppresses anything at nms_thre > 0,
+ * itself included.  With nms_thre <= 0, boxes that do not overlap can suppress each other, as they do under IoU.
+ *   diou   0 = yl_nms_ex (same launches, same bytes); 1 = DIoU-NMS; anything else returns YL_ERR_ARG before any CUDA call.
+ * The workspace is that of yl_nms_ex (yl_post_workspace_bytes_ex with the same agnostic). */
+int yl_nms_ex2(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic, int diou,
+               float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream);
 /* Workspace bytes for yl_nms_ex: agnostic = 0 is yl_post_workspace_bytes(); 1 adds 8 bytes per candidate slot
  * (B * C * cap_seg) of scratch for images whose survivors exceed shared memory; anything else returns 0. */
 size_t yl_post_workspace_bytes_ex(int B, long M, int C, int cap_seg, int agnostic);
@@ -303,6 +320,12 @@ int yl_detect_host_topk(yl_context *ctx, const float *const *raw_host, float con
  * yl_post_workspace_bytes_ex(..., 1). */
 int yl_detect_host_ex(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det, int agnostic,
                       float *out_rows_host, int *counts_host);
+/* yl_detect_host_ex with DIoU-NMS (yl_nms_ex2): a candidate a is dropped by an earlier kept box b when
+ * fl(iou - pen) >= nms_thre, pen = (dx*dx + dy*dy) / (cw*cw + ch*ch) with the centre distances dx, dy and the enclosing box's
+ * extents cw, ch, each operation one fp32 rounding as stated for yl_nms_ex2.  diou = 0 is yl_detect_host_ex, 1 is DIoU-NMS,
+ * anything else returns YL_ERR_ARG before any CUDA call. */
+int yl_detect_host_ex2(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det, int agnostic,
+                       int diou, float *out_rows_host, int *counts_host);
 
 /* ---------------------------------------------------------------------------------------------------------
  * (e) Multi-GPU: the final exchange of the image-sharded path            (SURVEY.md 8(e); no reference counterpart: the

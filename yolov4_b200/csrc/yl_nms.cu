@@ -11,6 +11,7 @@
 //                       out_rows[b] = (x1,y1,x2,y2,obj,cls_conf,cls) and the per-image counts.
 //   k_select_topk       per-image detection cap (max_det), between the NMS tiers and the gather.
 //   k_segment_nms_agnostic  class-agnostic NMS, one CTA per image, in place of the two NMS tiers (yl_nms_ex).
+// The three NMS kernels take a template flag DIOU: the DIoU-NMS pair decision in place of IoU >= thr (yl_nms_ex2).
 //
 // Candidate record (written by the filter kernels, yl_filter.cu): two uint4,
 //   A = {score bits, box row, cls_conf bits, obj_conf bits}    B = {x1, y1, x2, y2}
@@ -27,9 +28,25 @@ constexpr int NMS_THREADS = 128;
 constexpr int SMEM_R = kSmemR;
 constexpr int CHUNK = 64;
 
+// DIoU penalty (Zheng et al., AAAI 2020) of candidate a against kept box b, pen = num / den: squared distance of the box
+// centres over the squared diagonal of the smallest box enclosing both, every operation one fp32 rounding in this order,
+// max / min propagating NaN.  pen is >= 0 or NaN, so fl(iou - pen) >= thr implies fl(iou) >= thr: every conservative IoU
+// pruning stays exact.  num and den are returned apart so that the boxes need not stay live until the division.
+__device__ __forceinline__ float2 diou_terms(const float4 &a, const float4 &b)
+{
+    const float dx = __fsub_rn(__fmul_rn(__fadd_rn(a.x, a.z), 0.5f), __fmul_rn(__fadd_rn(b.x, b.z), 0.5f));
+    const float dy = __fsub_rn(__fmul_rn(__fadd_rn(a.y, a.w), 0.5f), __fmul_rn(__fadd_rn(b.y, b.w), 0.5f));
+    const float cw = __fsub_rn(nanmaxf(a.z, b.z), nanminf(a.x, b.x));
+    const float ch = __fsub_rn(nanmaxf(a.w, b.w), nanminf(a.y, b.y));
+    return make_float2(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fadd_rn(__fmul_rn(cw, cw), __fmul_rn(ch, ch)));
+}
+
 // IoU >= thr decision, bit-equal to utils.py:71-77 (fp32, separate roundings, (area_a + area_b) - inter, IEEE divide).
 // Fast path (thr > 0, boxes sanitised so that NaN coordinates can never overlap): a pair whose intersection
 // is empty has iou = 0 or NaN, neither of which is >= thr, so only overlapping pairs pay for the division.
+// DIOU: the decision fl(iou - fl(num / den)) >= thr (diou_terms).  Every early `return false` holds for it too; the `return
+// true` shortcut does not, so such a pair takes the exact quotient and the penalty.
+template <bool DIOU = false>
 __device__ __forceinline__ bool suppresses_pos(const float4 &a, float area_a, const float4 &b, float area_b, float thr)
 {
     const float tlx = fmaxf(a.x, b.x), tly = fmaxf(a.y, b.y);
@@ -41,6 +58,7 @@ __device__ __forceinline__ bool suppresses_pos(const float4 &a, float area_a, co
         const float amin = fminf(area_a, area_b), amax = fmaxf(area_a, area_b);
         if (amax < 3.0e38f && amin < 0.999f * thr * amax) return false;
     }
+    const float2 pen = DIOU ? diou_terms(a, b) : make_float2(0.0f, 0.0f);
     const float inter = __fmul_rn(__fsub_rn(brx, tlx), __fsub_rn(bry, tly));
     const float uni = __fsub_rn(__fadd_rn(area_a, area_b), inter);
     // fl(inter/uni) >= thr is decided without the division when inter is not within 0.1% of thr*uni (the quotient's
@@ -48,12 +66,14 @@ __device__ __forceinline__ bool suppresses_pos(const float4 &a, float area_a, co
     if (uni > 0.0f && uni < 3.0e38f) {
         const float tu = thr * uni;
         if (inter < 0.999f * tu) return false;
-        if (inter > 1.001f * tu && inter < 3.0e38f) return true;
+        if (!DIOU && inter > 1.001f * tu && inter < 3.0e38f) return true;
     }
+    if (DIOU) return __fsub_rn(__fdiv_rn(inter, uni), __fdiv_rn(pen.x, pen.y)) >= thr;
     return __fdiv_rn(inter, uni) >= thr;
 }
 
 // General path (thr <= 0 or unsanitised boxes): literal NaN-propagating formula.
+template <bool DIOU = false>
 __device__ __forceinline__ bool suppresses_any(const float4 &a, float area_a, const float4 &b, float area_b, float thr)
 {
     const float tlx = nanmaxf(a.x, b.x), tly = nanmaxf(a.y, b.y);
@@ -61,6 +81,10 @@ __device__ __forceinline__ bool suppresses_any(const float4 &a, float area_a, co
     const float en = (tlx < brx && tly < bry) ? 1.0f : 0.0f;
     const float inter = __fmul_rn(__fmul_rn(__fsub_rn(brx, tlx), __fsub_rn(bry, tly)), en);
     const float iou = __fdiv_rn(inter, __fsub_rn(__fadd_rn(area_a, area_b), inter));
+    if (DIOU) {
+        const float2 pen = diou_terms(a, b);
+        return __fsub_rn(iou, __fdiv_rn(pen.x, pen.y)) >= thr;
+    }
     return iou >= thr;
 }
 
@@ -190,6 +214,8 @@ __device__ __forceinline__ int coord_bin(float v, float lo, float scale)
     return min(max(q, 0), NBIN - 1);
 }
 
+// DIOU selects the DIoU decision for the exact tests of step 5; the bin tables stay exact for it (DIoU >= thr needs IoU >= thr).
+template <bool DIOU>
 __global__ void __launch_bounds__(SMALL_THREADS, YL_NMS_MINB)
 k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_count, unsigned *__restrict__ kept_count,
                    int C, int cap_seg, float thr, int area_k, int seg_first,
@@ -462,7 +488,7 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
                 const unsigned e = S.a.queue[wq][q];
                 const int j = e >> 8, i = e & 255;
                 const float4 bj = S.box[j], bi = S.box[i];
-                if (suppresses_pos(bj, box_area(bj), bi, box_area(bi), thr)) {
+                if (suppresses_pos<DIOU>(bj, box_area(bj), bi, box_area(bi), thr)) {
                     atomicOr(&S.b.T[j][i >> 5], 1u << (i & 31));
                     atomicOr(&S.dirty[j >> 5], 1u << (j & 31));
                     found = true;
@@ -581,8 +607,8 @@ __device__ void bitonic_sort(Store &s, int n)
 //   (2) the 64x64 intra-chunk suppression matrix is built as one 64-bit row per member
 //   (3) warp 0 resolves the chunk serially with the rows in registers
 //   (4) survivors are appended to the kept list (compacted in place: a kept box never moves to a higher index)
-// kept_of[q] = sorted position of the q-th kept box.  Returns the number kept.
-template <bool POS, class Store, int NT = NMS_THREADS>
+// kept_of[q] = sorted position of the q-th kept box.  Returns the number kept.  DIOU selects the DIoU pair decision.
+template <bool POS, bool DIOU, class Store, int NT = NMS_THREADS>
 __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, unsigned *kept_g,
                           unsigned *sh_supp /*[2]*/, unsigned long long *sh_rows /*[64]*/, int *sh_nk)
 {
@@ -606,7 +632,7 @@ __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, un
                     const int kq = kept_s ? (int)kept_s[q] : (int)kept_g[q];
                     const float4 bk = s.get_box(kq);
                     const float ak = s.get_area(kq);
-                    dead = POS ? suppresses_pos(bi, ai, bk, ak, thr) : suppresses_any(bi, ai, bk, ak, thr);
+                    dead = POS ? suppresses_pos<DIOU>(bi, ai, bk, ak, thr) : suppresses_any<DIOU>(bi, ai, bk, ak, thr);
                 }
                 if (dead) atomicOr(&sh_supp[i >> 5], 1u << (i & 31));
             }
@@ -616,8 +642,8 @@ __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, un
             const int i = pr / CHUNK, j = pr - i * CHUNK;
             if (j > i && j < cn) {
                 const float4 bi = s.get_box(c0 + i), bj = s.get_box(c0 + j);
-                const bool sup = POS ? suppresses_pos(bj, s.get_area(c0 + j), bi, s.get_area(c0 + i), thr)
-                                     : suppresses_any(bj, s.get_area(c0 + j), bi, s.get_area(c0 + i), thr);
+                const bool sup = POS ? suppresses_pos<DIOU>(bj, s.get_area(c0 + j), bi, s.get_area(c0 + i), thr)
+                                     : suppresses_any<DIOU>(bj, s.get_area(c0 + j), bi, s.get_area(c0 + i), thr);
                 if (sup) atomicOr(&sh_rows[i], 1ull << j);
             }
         }
@@ -646,6 +672,7 @@ __device__ int greedy_nms(Store &s, int n, float thr, unsigned short *kept_s, un
 }
 
 // Persistent CTAs walk the list of segments the small tier passed on.
+template <bool DIOU>
 __global__ void __launch_bounds__(NMS_THREADS)
 k_segment_nms_big(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_count, unsigned *__restrict__ kept_count,
                   int C, int cap_seg, float thr, const unsigned *__restrict__ big_count, const unsigned *__restrict__ big_list,
@@ -683,8 +710,8 @@ k_segment_nms_big(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_cou
             __syncthreads();
             SmemStore s{sh_key, sh_idx, sh_ubox, pos};
             bitonic_sort(s, n);
-            const int nk = pos ? greedy_nms<true>(s, n, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk)
-                               : greedy_nms<false>(s, n, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk);
+            const int nk = pos ? greedy_nms<true, DIOU>(s, n, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk)
+                               : greedy_nms<false, DIOU>(s, n, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk);
             for (int q = tid; q < nk; q += NMS_THREADS) {
                 const int e = sh_idx[sh_kept[q]];
                 const uint2 co = sh_uco[e];
@@ -701,8 +728,8 @@ k_segment_nms_big(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_cou
             GlobalStore s{rec, pos};
             bitonic_sort(s, n);
             unsigned *kept_g = kept_scratch + (size_t)seg * cap_seg;
-            const int nk = pos ? greedy_nms<true>(s, n, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk)
-                               : greedy_nms<false>(s, n, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk);
+            const int nk = pos ? greedy_nms<true, DIOU>(s, n, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk)
+                               : greedy_nms<false, DIOU>(s, n, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk);
             // rows replace records in place: kept_g[q] >= q and a row (28 B) is shorter than a record (32 B), so the
             // rows of a chunk never reach a record a later chunk still has to read; go through registers chunk by chunk
             for (int q0 = 0; q0 < nk; q0 += NMS_THREADS) {
@@ -975,6 +1002,9 @@ __device__ __forceinline__ unsigned agn_block_scan(bool f, unsigned *sh_w /*[AGN
     return before + __popc(m & ((1u << lane) - 1u));
 }
 
+// DIOU: the DIoU decision, in the greedy pass and in the self test of the first-copy reduction.  The reduction stays exact:
+// copies of a box have the same bits, so a decision against one copy is the decision against every copy.
+template <bool DIOU>
 __global__ void __launch_bounds__(AGN_THREADS, 1)
 k_segment_nms_agnostic(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_count, unsigned *__restrict__ kept_count,
                        int C, int cap_seg, float thr, unsigned *__restrict__ tab_key_all, unsigned *__restrict__ tab_cls_all,
@@ -1050,11 +1080,11 @@ k_segment_nms_agnostic(uint4 *__restrict__ cand, const unsigned *__restrict__ se
         if (score_desc_bits(a.x) == __ldcg(&tab_key[a.y])) atomicMin(&tab_cls[a.y], (unsigned)c);
     }
     __syncthreads();
-    // a copy survives when it is the box's first copy or when the literal self-IoU of its box is below thr
+    // a copy survives when it is the box's first copy or when its box does not suppress itself (the literal self decision)
     auto survives = [&](const uint4 &a, const float4 &bx, int c) -> bool {
         if (score_desc_bits(a.x) == __ldcg(&tab_key[a.y]) && (unsigned)c == __ldcg(&tab_cls[a.y])) return true;
         const float ar = box_area(bx);
-        return !suppresses_any(bx, ar, bx, ar, thr);
+        return !suppresses_any<DIOU>(bx, ar, bx, ar, thr);
     };
     for (unsigned i = tid; i < n; i += AGN_THREADS) {
         int c;
@@ -1079,8 +1109,8 @@ k_segment_nms_agnostic(uint4 *__restrict__ cand, const unsigned *__restrict__ se
         // ---- 2. shared-memory path.  Every read of the image's records is done: rows may overwrite them from here ----
         SmemStore s{sh_key, sh_idx, sh_box, pos};
         bitonic_sort<SmemStore, AGN_THREADS>(s, (int)ns);
-        const int nk = pos ? greedy_nms<true, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk)
-                           : greedy_nms<false, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk);
+        const int nk = pos ? greedy_nms<true, DIOU, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk)
+                           : greedy_nms<false, DIOU, SmemStore, AGN_THREADS>(s, (int)ns, thr, sh_kept, nullptr, sh_supp, sh_rows, &sh_nk);
         // rank within the class: each warp takes a contiguous slice of the kept list; per-class counts per warp, a prefix over
         // the warps, then ranks inside the slice from peer masks
         const int q0 = (int)(((long)nk * warp) / (AGN_THREADS / 32)), q1 = (int)(((long)nk * (warp + 1)) / (AGN_THREADS / 32));
@@ -1164,8 +1194,8 @@ k_segment_nms_agnostic(uint4 *__restrict__ cand, const unsigned *__restrict__ se
     }
     __syncthreads();
     MergedStore ms{img, order, pos};
-    const int nk = pos ? greedy_nms<true, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk)
-                       : greedy_nms<false, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk);
+    const int nk = pos ? greedy_nms<true, DIOU, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk)
+                       : greedy_nms<false, DIOU, MergedStore, AGN_THREADS>(ms, (int)ns, thr, nullptr, kept_g, sh_supp, sh_rows, &sh_nk);
     // mark the kept records (the key word is free now), then compact every segment in place
     for (unsigned i = tid; i < ns; i += AGN_THREADS) img[2 * (size_t)order[i]].x = 0u;
     __syncthreads();
@@ -1228,10 +1258,12 @@ extern "C" size_t yl_post_workspace_bytes_ex(int B, long M, int C, int cap_seg, 
     return (base == 0 || !agnostic) ? base : base + agn_scratch_bytes(B, C, cap_seg);
 }
 
-extern "C" int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
-                         float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
+extern "C" int yl_nms_ex2(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
+                          int diou, float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count,
+                          yl_stream_t stream)
 {
     if (agnostic != 0 && agnostic != 1) return YL_ERR_ARG;
+    if (diou != 0 && diou != 1) return YL_ERR_ARG;
     if (!ws || !out_rows || !meta || B <= 0 || M <= 0 || C <= 0 || cap_seg <= 0 || cap_out <= 0) return YL_ERR_ARG;
     if (img_first < 0 || img_count < 0 || img_first + img_count > B) return YL_ERR_ARG;
     if (max_det < 0 || max_det > cap_out) return YL_ERR_ARG;
@@ -1253,17 +1285,21 @@ extern "C" int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int ca
     // each kernel may become resident while its predecessor drains (PDL); it waits before reading the predecessor's output.
     // The first one follows the emit / dense filter kernel of yl_filter_* on the same stream.
     const bool pdl = pdl_enabled();
+    // the same launches with either pair decision: only the instantiation differs
     if (agnostic) {
+        const auto k_agn = diou ? k_segment_nms_agnostic<true> : k_segment_nms_agnostic<false>;
         // per device, so set on every call (a host-side attribute: allowed during stream capture)
-        YL_CUDA_TRY(cudaFuncSetAttribute(k_segment_nms_agnostic, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AGN_SMEM_BYTES));
-        YL_CUDA_TRY(launch_after(k_segment_nms_agnostic, dim3(img_count), dim3(AGN_THREADS), AGN_SMEM_BYTES, st, pdl, cand,
+        YL_CUDA_TRY(cudaFuncSetAttribute(k_agn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)AGN_SMEM_BYTES));
+        YL_CUDA_TRY(launch_after(k_agn, dim3(img_count), dim3(AGN_THREADS), AGN_SMEM_BYTES, st, pdl, cand,
                                  (const unsigned *)seg_count, kept_count, C, cap_seg, nms_thre, (unsigned *)(w + L.off_obj),
                                  (unsigned *)(w + L.off_flags), L.M4, (unsigned *)(w + L.total), img_first));
     } else {
-        YL_CUDA_TRY(launch_after(k_segment_nms_bins, dim3(nseg), dim3(SMALL_THREADS), 0, st, pdl, cand, seg_count, kept_count, C, cap_seg,
+        const auto k_bins = diou ? k_segment_nms_bins<true> : k_segment_nms_bins<false>;
+        const auto k_big = diou ? k_segment_nms_big<true> : k_segment_nms_big<false>;
+        YL_CUDA_TRY(launch_after(k_bins, dim3(nseg), dim3(SMALL_THREADS), 0, st, pdl, cand, seg_count, kept_count, C, cap_seg,
                                  nms_thre, area_bin_gap(nms_thre), seg_first, big_count, big_list));
         const int grid_big = nseg < 148 * 2 ? nseg : 148 * 2;
-        YL_CUDA_TRY(launch_after(k_segment_nms_big, dim3(grid_big), dim3(NMS_THREADS), 0, st, pdl, cand, (const unsigned *)seg_count, kept_count,
+        YL_CUDA_TRY(launch_after(k_big, dim3(grid_big), dim3(NMS_THREADS), 0, st, pdl, cand, (const unsigned *)seg_count, kept_count,
                                  C, cap_seg, nms_thre, (const unsigned *)big_count, (const unsigned *)big_list, kept_scratch));
     }
     if (max_det > 0) {
@@ -1274,6 +1310,13 @@ extern "C" int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int ca
     YL_CUDA_TRY(launch_after(k_gather_rows, dim3(nseg), dim3(GATHER_THREADS), 0, st, pdl, (const uint4 *)cand, (const unsigned *)seg_count,
                              (const unsigned *)kept_count, C, cap_seg, B, out_rows, cap_out, meta, seg_first));
     return YL_OK;
+}
+
+extern "C" int yl_nms_ex(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det, int agnostic,
+                         float *out_rows, long cap_out, int *meta, int *uncapped, int img_first, int img_count, yl_stream_t stream)
+{
+    return yl_nms_ex2(ws, ws_bytes, B, M, C, cap_seg, nms_thre, max_det, agnostic, 0, out_rows, cap_out, meta, uncapped, img_first,
+                      img_count, stream);
 }
 
 extern "C" int yl_nms_topk(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, float nms_thre, int max_det,

@@ -88,6 +88,13 @@ def _check_agnostic(agnostic):
     return agnostic
 
 
+def _check_diou(diou):
+    """A bool; checked before any CUDA work."""
+    if not isinstance(diou, bool):
+        raise TypeError("diou must be a bool, got %r" % (diou,))
+    return diou
+
+
 def _round4(n):
     return (n + 3) // 4 * 4
 
@@ -106,12 +113,13 @@ def _split(rows, meta_host, B, out_device, out_dtype):
     return out
 
 
-def _run(front_end, device, B, M, C, nms_thre, max_det=None, agnostic=False):
+def _run(front_end, device, B, M, C, nms_thre, max_det=None, agnostic=False, diou=False):
     """Runs front end + NMS, growing cap_seg / cap_out and re-running when the device reports an overflow.  With a cap the
-    output holds max_det rows per image (rounded up to a multiple of 4), which no image can exceed; the capacities a capped
-    or agnostic call settles on are kept apart from those of plain calls."""
+    output holds max_det rows per image (rounded up to a multiple of 4), which no image can exceed; the capacities a capped,
+    agnostic or DIoU call settles on are kept apart from those of plain calls."""
     L = _cabi.lib()
-    hint_key = (B, M, C) if max_det is None and not agnostic else (B, M, C, max_det, agnostic)
+    plain = max_det is None and not agnostic and not diou
+    hint_key = (B, M, C) if plain else (B, M, C, max_det, agnostic, diou)
     cap_seg, cap_out = _cap_hint.get(hint_key, (_DEFAULT_CAP_SEG, _DEFAULT_CAP_OUT))
     if max_det is not None:
         cap_out = _round4(max_det)
@@ -122,8 +130,8 @@ def _run(front_end, device, B, M, C, nms_thre, max_det=None, agnostic=False):
         meta = torch.empty((3 * B,), dtype=torch.int32, device=device)
         _cabi.check(L.yl_post_reset(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _stream()))
         front_end(ws, cap_seg)
-        _cabi.check(L.yl_nms_ex(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), max_det or 0, int(agnostic), rows.data_ptr(),
-                                cap_out, meta.data_ptr(), None, 0, B, _stream()))
+        _cabi.check(L.yl_nms_ex2(ws.ptr(), ws.nbytes, B, M, C, cap_seg, _f32(nms_thre), max_det or 0, int(agnostic), int(diou),
+                                 rows.data_ptr(), cap_out, meta.data_ptr(), None, 0, B, _stream()))
         mh = meta.cpu().numpy()                      # the one D2H sync the list-of-tensors contract requires
         max_seg, max_rows = int(mh[B:2 * B].max()), int(mh[:B].max())
         if max_seg > cap_seg:
@@ -138,7 +146,7 @@ def _run(front_end, device, B, M, C, nms_thre, max_det=None, agnostic=False):
         return rows, mh
 
 
-def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_det=None, agnostic=False):
+def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_det=None, agnostic=False, diou=False):
     """Same contract as the reference's postprocess (yolo/util/utils.py:92).
 
     prediction: [B, M, 5+C] decoded (cx, cy, w, h, obj, cls...), fp32, on a CUDA device (a CPU tensor, as
@@ -151,9 +159,11 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
     max_det (keyword only, not part of the reference signature): keep at most this many detections per image, those with the
     highest obj_conf * cls_conf (equal scores keep the order above), still listed classes ascending then score descending.
     agnostic (keyword only, not part of the reference signature): class-agnostic NMS, see detect_raw.
+    diou (keyword only, not part of the reference signature): DIoU-NMS, see detect_raw.
     """
     max_det = _check_max_det(max_det)
     agnostic = _check_agnostic(agnostic)
+    diou = _check_diou(diou)
     if prediction.dim() != 3 or prediction.shape[2] < 6:
         raise ValueError("prediction must be [B, M, 5+C]")
     if prediction.dtype != torch.float32:
@@ -171,7 +181,7 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_dense(pred.data_ptr(), B, M, C, num_classes, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                           cap_seg, 0, B, _stream()))
-        rows, mh = _run(front, pred.device, B, M, C, nms_thre, max_det, agnostic)
+        rows, mh = _run(front, pred.device, B, M, C, nms_thre, max_det, agnostic, diou)
     return _split(rows, mh, B, in_device, prediction.dtype)
 
 
@@ -198,7 +208,7 @@ def _check_raws(head_outputs, num_classes):
 
 
 def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None,
-               agnostic=False):
+               agnostic=False, diou=False):
     """Fused YOLOLayer eval decode (yololayer.py:88-166) + postprocess (utils.py:92-223).
 
     head_outputs: the three raw head conv outputs [B, 3*(5+C), F_l, F_l] (stride 8, 16, 32; yolov4.py:235-251).
@@ -220,9 +230,18 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     candidate, whatever the classes.  A box then keeps at most one label, its best-scoring passing class (a degenerate box --
     NaN, zero or negative extent, overflowing area -- never suppresses itself and keeps all its labels).  The kept rows are
     listed as usual, classes ascending then score descending; max_det applies to them.  Default False: per-class NMS.
+
+    diou: DIoU-NMS (Zheng et al., AAAI 2020; the DIoU-NMS of the YOLOv4 paper).  Candidates, order, rows and max_det are as
+    without it, per class or agnostic; only the suppression decision changes.  A candidate a is dropped by an earlier kept box
+    b when fl32(iou - pen) >= nms_thre, with the literal IoU above and pen = (dx*dx + dy*dy) / (cw*cw + ch*ch): dx, dy the
+    distances of the box centres ((x1 + x2) * 0.5), cw, ch the extents of the smallest box enclosing both, every operation
+    one fp32 rounding, max / min propagating NaN.  A NaN penalty keeps the pair apart, and pen >= 0, so DIoU never suppresses
+    a pair IoU keeps apart: boxes far apart that overlap enough for IoU survive as separate detections.  darknet's diounms
+    compares with > and an exponent beta_nms; this is the paper's >= with no exponent.  Default False: IoU.
     """
     max_det = _check_max_det(max_det)
     agnostic = _check_agnostic(agnostic)
+    diou = _check_diou(diou)
     raws, B, Fs, dt = _check_raws(head_outputs, num_classes)
     C = int(num_classes)
     M = sum(3 * f * f for f in Fs)
@@ -236,7 +255,7 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
         def front(ws, cap_seg):
             _cabi.check(L.yl_filter_raw_typed(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes,
                                               M, cap_seg, 0, B, 3, _stream()))
-        rows, mh = _run(front, dev, B, M, C, nms_thre, max_det, agnostic)
+        rows, mh = _run(front, dev, B, M, C, nms_thre, max_det, agnostic, diou)
     return _split(rows, mh, B, dev, torch.float32)
 
 
@@ -254,13 +273,14 @@ class HeadPostprocessor:
     of 4, so the output (and a DetectionExchange built with hp.cap_out) is sized by the cap.  uncapped is a device int32 [B]
     with every image's uncapped count, refreshed by every run and replay: meta[b] < uncapped[b] means image b was capped.
     Without a cap uncapped is the view meta[:B].  agnostic selects class-agnostic NMS as in detect_raw (uncapped then counts
-    the agnostic rows).
+    the agnostic rows), and diou DIoU-NMS as in detect_raw.
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
-                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None, agnostic=False):
+                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None, agnostic=False, diou=False):
         self.max_det = _check_max_det(max_det)
         self.agnostic = _check_agnostic(agnostic)
+        self.diou = _check_diou(diou)
         if cap_out is None:
             cap_out = _DEFAULT_CAP_OUT if self.max_det is None else _round4(self.max_det)
         if self.max_det is not None and self.max_det > int(cap_out):
@@ -303,9 +323,9 @@ class HeadPostprocessor:
                                               self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7 if fold_reset else 3,
                                               main.cuda_stream))
             self.side.wait_stream(main)
-            _cabi.check(L.yl_nms_ex(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
-                                    int(self.agnostic), self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
-                                    None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, self.side.cuda_stream))
+            _cabi.check(L.yl_nms_ex2(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
+                                     int(self.agnostic), int(self.diou), self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),
+                                     None if self.max_det is None else self.uncapped.data_ptr(), i0, i1 - i0, self.side.cuda_stream))
         main.wait_stream(self.side)
         return self.rows, self.meta
 
