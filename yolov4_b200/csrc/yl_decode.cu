@@ -16,12 +16,12 @@ constexpr int DD_THREADS = 256;    // 4 channel rows x 64 boxes per pass
 __global__ void __launch_bounds__(DD_THREADS)
 k_decode_dense(const float *__restrict__ raw, int Fw, int F2, int C, float stride,
                float aw0, float ah0, float aw1, float ah1, float aw2, float ah2,
-               float *__restrict__ out, long rows_per_image, long row_offset)
+               float *__restrict__ out, long rows_per_image, long row_offset, int ba0)
 {
     extern __shared__ __align__(16) float tile[];   // [DD_TP][nch]: the output layout itself (odd nch, e.g. 85: conflict-free stores)
     const int nch = 5 + C;
     const int nchp = nch;
-    const int ba = blockIdx.y;
+    const int ba = ba0 + (int)blockIdx.y;
     const int b = ba / 3, a = ba - 3 * b;
     const int p0 = blockIdx.x * DD_TP;
     const int np = min(DD_TP, F2 - p0);
@@ -196,16 +196,22 @@ extern "C" int yl_decode_dense(const float *raw, int B, int F, int C, const floa
 {
     if (!raw || !ag || !out || B <= 0 || F <= 0 || C <= 0 || rows_per_image < 3L * F * F + row_offset || row_offset < 0)
         return YL_ERR_ARG;
+    if (3L * B > 0x7FFFFFFFL) return YL_ERR_ARG;
     const int F2 = F * F;
     const size_t smem = sizeof(float) * DD_TP * (5 + C);
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_decode_dense, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return YL_ERR_CUDA_BASE + (int)e;
     }
-    dim3 grid((F2 + DD_TP - 1) / DD_TP, B * 3);
-    k_decode_dense<<<grid, DD_THREADS, smem, (cudaStream_t)stream>>>(raw, F, F2, C, stride, ag[0], ag[1], ag[2], ag[3],
-                                                                     ag[4], ag[5], out, rows_per_image, row_offset);
-    YL_LAUNCH_CHECK();
+    // gridDim.y is at most 65535: larger batches go out in slices of (image, anchor) pairs, one launch when B*3 fits
+    constexpr int kMaxGridY = 65535;
+    const long pairs = 3L * B;
+    for (long ba0 = 0; ba0 < pairs; ba0 += kMaxGridY) {
+        dim3 grid((F2 + DD_TP - 1) / DD_TP, (unsigned)min((long)kMaxGridY, pairs - ba0));
+        k_decode_dense<<<grid, DD_THREADS, smem, (cudaStream_t)stream>>>(raw, F, F2, C, stride, ag[0], ag[1], ag[2], ag[3],
+                                                                         ag[4], ag[5], out, rows_per_image, row_offset, (int)ba0);
+        YL_LAUNCH_CHECK();
+    }
     return YL_OK;
 }
 
