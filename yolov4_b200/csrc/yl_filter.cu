@@ -836,14 +836,15 @@ __device__ __forceinline__ void dense_row(const float (&e)[NJ], int nch, int C, 
         anyn |= pass[j] && idx < 5 + num_classes;
         has_nan |= (idx >= 5 && idx < 5 + num_classes) && (e[j] != e[j]);
     }
-    if (obj >= 0.0f) {
-        // Row pre-filter obj * max_{c < num_classes} cls >= thr (utils.py:139-148).  For obj >= 0, fl(obj*x) is monotone in x,
-        // so without NaNs the row passes exactly when one of its first num_classes classes passes the per-class test:
-        // no max reduction for the ~99 % of rows that produce nothing.
+    if (obj > 0.0f && obj < kInf) {
+        // Row pre-filter obj * max_{c < num_classes} cls >= thr (utils.py:139-148).  For a finite obj > 0, fl(obj*x) is monotone
+        // in x and never NaN for a non-NaN x, so without NaNs the row passes exactly when one of its first num_classes classes
+        // passes the per-class test: no max reduction for the ~99 % of rows that produce nothing.  (+-0 and +inf are not:
+        // 0 * inf and inf * 0 are NaN, so the max can fail where a smaller class passes.)
         if (!__any_sync(0xFFFFFFFFu, anyn)) return;
         if (__any_sync(0xFFFFFFFFu, has_nan)) return;                 // torch.max propagates NaN: NaN >= thr is False
     } else {
-        // negative / NaN objectness (not a sigmoid output): literal form, max with torch.max NaN propagation
+        // +-0, +inf, negative or NaN objectness (not a finite sigmoid output): literal form, max with torch.max NaN propagation
         float mx = -kInf;
 #pragma unroll
         for (int j = 0; j < NJ; ++j) {

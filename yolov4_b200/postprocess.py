@@ -156,6 +156,7 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
     Differences from the reference, none observable by its callers: `prediction[:, :, :4]` is not overwritten
     in place with the corner form (utils.py:126), and score ties are ordered (score desc, box index desc),
     the order of a stable argsort, where NumPy's default sort leaves them unspecified (utils.py:58).
+    num_classes limits the row pre-filter to the first num_classes classes; a value above C means C, as the reference's slice.
     max_det (keyword only, not part of the reference signature): keep at most this many detections per image, those with the
     highest obj_conf * cls_conf (equal scores keep the order above), still listed classes ascending then score descending.
     agnostic (keyword only, not part of the reference signature): class-agnostic NMS, see detect_raw.
@@ -175,7 +176,7 @@ def postprocess(prediction, num_classes, conf_thre=0.7, nms_thre=0.45, *, max_de
     C = nch - 5
     if B == 0:
         return []
-    num_classes = int(num_classes)
+    num_classes = min(int(num_classes), C)           # the reference's slice image_pred[:, 5:5 + num_classes] clamps
     L = _cabi.lib()
     with torch.cuda.device(pred.device):
         def front(ws, cap_seg):
