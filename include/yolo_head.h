@@ -290,6 +290,28 @@ int yl_loss_forward_chained_typed(const void *raw, int dtype, const float *label
 int yl_loss_backward_typed(const float *gobj, const int *mcell, const float *mgrad, const float *upstream,
                            int B, int F, int K, int C, void *grad_raw, int dtype, yl_stream_t stream);
 
+/* IoU box regression in the fused loss (YOLOv4's CIoU, darknet's iou_loss = giou / diou / ciou).  yl_loss_forward_ex is the
+ * forward call of all of the above: yl_loss_forward[_typed] is it with iou_loss = YL_IOU_LOSS_NONE, iou_normalizer = 1,
+ * chained = 0, and yl_loss_forward_chained[_typed] the same with chained = 1 (chained = 1: the PDL launch and its rule above).
+ *   iou_loss NONE   the loss above, bit for bit
+ *   GIOU/DIOU/CIOU  the xy BCE and wh MSE of every matched cell are replaced by iou_normalizer * L(p, g): torchvision's
+ *            generalized_ / distance_ / complete_box_iou_loss (eps = 1e-7) of the train-mode predicted box p (grid units, the
+ *            fp32 bits of the decode) and the cell's last matched GT g (label / stride), on the xyxy corners x +- w / 2.  No
+ *            tgt_scale weighting.  loss4[0] accumulates the box term, loss4[1] receives nothing, loss4[2] / loss4[3] and the
+ *            objectness / class gradients are those of YL_IOU_LOSS_NONE.  mgrad[..., 0:4] holds iou_normalizer * d L / d raw
+ *            (CIoU's alpha held constant, ties of the min / max split evenly; fp32, see DESIGN.md section 1 for the bound);
+ *            a NaN term gives NaN in the cell's four entries.
+ * An unknown iou_loss, a negative, NaN or infinite iou_normalizer, or an unknown dtype returns YL_ERR_ARG before any CUDA
+ * call.  The saved tables, the aliasing rule and yl_loss_backward[_typed] are unchanged. */
+#define YL_IOU_LOSS_NONE 0
+#define YL_IOU_LOSS_GIOU 1
+#define YL_IOU_LOSS_DIOU 2
+#define YL_IOU_LOSS_CIOU 3
+int yl_loss_forward_ex(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                       const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_normalizer,
+                       int chained, double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                       yl_stream_t stream);
+
 /* ---------------------------------------------------------------------------------------------------------
  * Host-buffer entry (what a non-Python caller binds; also the bench's end-to-end leg): raw head tensors in
  * HOST memory -> detections in HOST memory.  The context owns device staging buffers, workspace, streams and

@@ -20,6 +20,11 @@
 // fp32 image) and the fp32 arithmetic below applies unchanged; the backward kernels form the same fp32 product and round it once
 // into the head's element type, so a 16-bit gradient is the fp32 path's gradient on the widened head, rounded to nearest-even.
 //
+// IoU box regression (iou_loss = GIoU / DIoU / CIoU, k_loss_match<T, IOU>, yl_loss_forward_ex): the xy BCE and wh MSE of every
+// matched cell are replaced by iou_normalizer * torchvision's box-IoU loss of the decoded prediction and the cell's last GT, in
+// grid units (DESIGN.md sections 1 and 5.9).  Lanes 0..3 evaluate the term redundantly and keep their own channel's derivative;
+// k_loss_obj, the class terms and the backward kernels do not change.  The IOU = 0 instantiations are the plain loss, unchanged.
+//
 // Per-term arithmetic is fp32 like the reference's (ATen binary_cross_entropy: (t-1) max(log(1-x), -100) - t max(log x, -100),
 // backward (x-t)/max((1-x) x, 1e-12); mse_loss); sums are accumulated in fp64.  Parity: loss and gradient within 1e-5 /
 // 2e-5 relative of the reference (tests/golden/loss.npz), not bit-exact (the reference's reduction order is unspecified).
@@ -49,6 +54,113 @@ __device__ __forceinline__ float bce_grad(float x, float t)
     return __fdiv_rn(__fsub_rn(x, t), fmaxf(__fmul_rn(__fsub_rn(1.0f, x), x), 1e-12f));
 }
 
+// ---- IoU box losses (iou_loss = giou / diou / ciou): torchvision's generalized_ / distance_ / complete_box_iou_loss with
+// eps = 1e-7 on the xyxy corners x +- w / 2 of the predicted box p and the GT g (grid units), and d loss / d (px, py, pw, ph) of
+// that float64 expression: alpha of CIoU is a constant (torchvision computes it under no_grad) and an exact tie of
+// torch.maximum / torch.minimum gives half the gradient to each side.
+constexpr float IOU_EPS = 1e-7f;
+
+// NaN-propagating min / max of fp64 edges (torch.minimum / maximum propagate NaN)
+__device__ __forceinline__ double edge_min(double a, double b) { return (a != a) ? a : ((b != b) ? b : (a < b ? a : b)); }
+__device__ __forceinline__ double edge_max(double a, double b) { return (a != a) ? a : ((b != b) ? b : (a > b ? a : b)); }
+// 1 / x within 1 ulp (MUFU.RCP; a subnormal x counts as 0 and gives inf, +inf gives 0, NaN stays NaN).  The IoU term is a
+// tolerance contract, and unlike __fdiv_rn this has no slow-path call, whose register save would spill.
+__device__ __forceinline__ float rcp_approx(float x)
+{
+    float r;
+    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
+// the first operand's share of the gradient of max(a, b) (or of min(b, a)): 1, 1/2 at a tie, 0
+__device__ __forceinline__ float share_gt(double a, double b) { return a > b ? 1.0f : (a == b ? 0.5f : 0.0f); }
+
+// One axis of the box pair: the prediction's edges relative to the GT's centre.  The fp64 difference of two fp32 values is
+// exact and every edge is within 2^-53 of its real value, so the min / max decisions (ties included) are the float64 spec's,
+// and the widths and the centre distance below are each ONE fp32 rounding away from the exact value, whether the boxes sit
+// in cell 0 or cell 75 and however small they are.
+struct IouAxis { float d, iw, cw, di, dip, dc, dcp; bool ov; };
+__device__ __forceinline__ IouAxis iou_axis(float pc, float pw, float gc, float gw)
+{
+    const double d = (double)pc - (double)gc, hp = 0.5 * (double)pw, hg = 0.5 * (double)gw;
+    const double l = d - hp, r = d + hp;
+    const double iw = edge_min(r, hg) - edge_max(l, -hg), cw = edge_max(r, hg) - edge_min(l, -hg);
+    IouAxis x;
+    x.d = (float)(d + (hp - hp) + (hg - hg));                              // the spec's (x1 + x2) / 2 is NaN for an infinite width
+    x.ov = iw > 0.0;                                                       // torchvision: overlap strictly positive
+    x.iw = (float)iw;
+    x.cw = (float)cw;
+    const float aR = share_gt(hg, r), aL = share_gt(l, -hg);               // p's share in min(right edges), max(left edges)
+    const float bR = share_gt(r, hg), bL = share_gt(-hg, l);               // p's share in max(right edges), min(left edges)
+    x.di = __fsub_rn(aR, aL);                                              // d iw / d pc, d iw / d pw
+    x.dip = __fmul_rn(__fadd_rn(aR, aL), 0.5f);
+    x.dc = __fsub_rn(bR, bL);                                              // d cw / d pc, d cw / d pw
+    x.dcp = __fmul_rn(__fadd_rn(bR, bL), 0.5f);
+    return x;
+}
+
+// L(p, g) and d L / d (px, py, pw, ph) in d.  IOU: 1 GIoU, 2 DIoU, 3 CIoU.  A NaN term gives NaN in all four derivatives.
+template <int IOU>
+__device__ __forceinline__ float iou_box_loss(float px, float py, float pw, float ph, float gx, float gy, float gw, float gh,
+                                              float (&d)[4])
+{
+    const IouAxis X = iou_axis(px, pw, gx, gw), Y = iou_axis(py, ph, gy, gh);
+    const bool ov = X.ov && Y.ov;
+    const float I = ov ? __fmul_rn(X.iw, Y.iw) : 0.0f;
+    const float ap = __fmul_rn(pw, ph), ag = __fmul_rn(gw, gh);
+    const float U = __fsub_rn(__fadd_rn(ap, ag), I), Ue = __fadd_rn(U, IOU_EPS);
+    const float rUe = rcp_approx(Ue), iou = __fmul_rn(I, rUe);
+    // 1 - iou as ((ap - I) + (ag - I) + eps) / Ue: no cancellation near iou = 1 (exactly eps / Ue for p == g); an infinite
+    // area makes that inf / inf, where 1 - iou is exact instead
+    const float omi = isinf(Ue) ? __fsub_rn(1.0f, iou)
+                                : __fmul_rn(__fadd_rn(__fadd_rn(__fsub_rn(ap, I), __fsub_rn(ag, I)), IOU_EPS), rUe);
+    // d I / d p (zero without overlap); d U = (0, 0, ph, pw) - d I; d (1 - iou) = (iou d U - d I) / Ue
+    const float kx = ov ? Y.iw : 0.0f, ky = ov ? X.iw : 0.0f;
+    const float dI[4] = {__fmul_rn(kx, X.di), __fmul_rn(ky, Y.di), __fmul_rn(kx, X.dip), __fmul_rn(ky, Y.dip)};
+    const float dU[4] = {__fsub_rn(0.0f, dI[0]), __fsub_rn(0.0f, dI[1]), __fsub_rn(ph, dI[2]), __fsub_rn(pw, dI[3])};
+#pragma unroll
+    for (int k = 0; k < 4; ++k) d[k] = __fmul_rn(__fsub_rn(__fmul_rn(iou, dU[k]), dI[k]), rUe);
+    float L = omi;
+    if (IOU == 1) {                                                        // GIoU: + (C - U) / (C + eps)
+        const float C = __fmul_rn(X.cw, Y.cw), Ce = __fadd_rn(C, IOU_EPS);
+        L = __fadd_rn(L, __fmul_rn(__fsub_rn(C, U), rcp_approx(Ce)));
+        const float dC[4] = {__fmul_rn(Y.cw, X.dc), __fmul_rn(X.cw, Y.dc), __fmul_rn(Y.cw, X.dcp), __fmul_rn(X.cw, Y.dcp)};
+        const float rCe = rcp_approx(Ce), q = __fmul_rn(Ue, rCe);     // d = (dC (U + eps) / Ce - dU) / Ce
+#pragma unroll
+        for (int k = 0; k < 4; ++k) d[k] = __fadd_rn(d[k], __fmul_rn(__fsub_rn(__fmul_rn(dC[k], q), dU[k]), rCe));
+    } else {                                                               // DIoU / CIoU: + rho^2 / (cw^2 + ch^2 + eps)
+        const float rho2 = __fadd_rn(__fmul_rn(X.d, X.d), __fmul_rn(Y.d, Y.d));
+        const float D = __fadd_rn(__fadd_rn(__fmul_rn(X.cw, X.cw), __fmul_rn(Y.cw, Y.cw)), IOU_EPS);
+        const float rD = rcp_approx(D), P = __fmul_rn(rho2, rD);
+        L = __fadd_rn(L, P);
+        const float tcx = __fmul_rn(2.0f, X.cw), tcy = __fmul_rn(2.0f, Y.cw);
+        const float dD[4] = {__fmul_rn(tcx, X.dc), __fmul_rn(tcy, Y.dc), __fmul_rn(tcx, X.dcp), __fmul_rn(tcy, Y.dcp)};
+        const float dr[4] = {__fmul_rn(2.0f, X.d), __fmul_rn(2.0f, Y.d), 0.0f, 0.0f};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) d[k] = __fadd_rn(d[k], __fmul_rn(__fsub_rn(dr[k], __fmul_rn(P, dD[k])), rD));
+        if (IOU == 3) {                                                    // CIoU: + alpha v, alpha constant
+            const float r = __fmul_rn(pw, rcp_approx(ph));
+            const float da = __fsub_rn(atanf(__fmul_rn(gw, rcp_approx(gh))), atanf(r));
+            const float v = __fmul_rn(0.405284735f, __fmul_rn(da, da));     // 4 / pi^2
+            const float alpha = __fmul_rn(v, rcp_approx(__fadd_rn(__fadd_rn(omi, v), IOU_EPS)));
+            L = __fadd_rn(L, __fmul_rn(alpha, v));
+            // d atan(pw / ph) = (ph d pw - pw d ph) / (pw^2 + ph^2), through the ratio t = min / max of the two extents (|t| <= 1),
+            // so that nothing overflows or underflows for extents in [1e-30, 1e30];  d v = -(8 / pi^2) da d atan(pw / ph)
+            const bool wide = fabsf(pw) > fabsf(ph);
+            const float inv = rcp_approx(wide ? pw : ph), t = __fmul_rn(wide ? ph : pw, inv);
+            const float ik = __fmul_rn(inv, rcp_approx(__fadd_rn(1.0f, __fmul_rn(t, t))));
+            const float dik = __fmul_rn(ik, t);
+            const float c = __fmul_rn(alpha, __fmul_rn(-0.810569469f, da));  // 8 / pi^2
+            d[2] = __fadd_rn(d[2], __fmul_rn(c, wide ? dik : ik));
+            d[3] = __fsub_rn(d[3], __fmul_rn(c, wide ? ik : dik));
+        }
+    }
+    if (L != L) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) d[k] = L;
+    }
+    return L;
+}
+
 __device__ __forceinline__ double warp_sum(double v)
 {
 #pragma unroll
@@ -63,11 +175,16 @@ __device__ __forceinline__ float narrow(float x, float *) { return x; }
 __device__ __forceinline__ __half narrow(float x, __half *) { return __float2half_rn(x); }
 __device__ __forceinline__ __nv_bfloat16 narrow(float x, __nv_bfloat16 *) { return __float2bfloat16_rn(x); }
 
-template <typename T>
-__global__ void __launch_bounds__(LS_THREADS)
+// IOU (YL_IOU_LOSS_*): 0 is the reference's xy BCE / wh MSE box term; 1..3 replace it by iou_norm * L(p, g) of the matched
+// cell (iou_box_loss), with p decoded from the cell's four box logits exactly as k_loss_obj decodes it and g its last GT.
+// iou_norm is the last parameter so that the IOU = 0 instantiations keep the parameter layout (and code) they always had.  The
+// IoU instantiations ask for one resident CTA per SM at least (in place of ptxas's occupancy target), which lets them hold the
+// box term's ~80 live values without spilling; the grid has 8 B CTAs of which a few hundred fit on 148 SMs at any count.
+template <typename T, int IOU>
+__global__ void __launch_bounds__(LS_THREADS, IOU == 0 ? 0 : 1)
 k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
              double *__restrict__ loss4, int *__restrict__ tcell_all, int *__restrict__ mcell, float *__restrict__ mgrad,
-             int *__restrict__ status)
+             int *__restrict__ status, float iou_norm)
 {
     __shared__ float tb[TG_MAXK][4];
     __shared__ float tcls[TG_MAXK];
@@ -122,6 +239,22 @@ k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F,
         // wraps onto 0..3, and wrapping onto 4 (objectness, already 1) changes nothing.
         const int kt = class_channel(tcls[t], nch);
         for (int kk = lane; kk < nk; kk += 32) {
+            if constexpr (IOU != 0) {
+                if (kk < 4) {                                          // IoU term: lanes 0..3 each evaluate it, keep their channel
+                    const float t0 = widen(cp[0]), t1 = widen(cp[(size_t)F2]), t2 = widen(cp[2 * (size_t)F2]), t3 = widen(cp[3 * (size_t)F2]);
+                    const int j = r / F, i = r - j * F;
+                    const float sx = spec_sigmoidf(t0), sy = spec_sigmoidf(t1);
+                    const float pw = __fmul_rn(spec_expf(t2), A.maw[a]), ph = __fmul_rn(spec_expf(t3), A.mah[a]);
+                    float dl[4];
+                    const float term = iou_box_loss<IOU>(__fadd_rn(sx, (float)i), __fadd_rn(sy, (float)j), pw, ph,
+                                                         tb[t][0], tb[t][1], tb[t][2], tb[t][3], dl);
+                    if (kk == 0) acc_xy += (double)__fmul_rn(iou_norm, term);
+                    const float dn = __fmul_rn(iou_norm, kk == 0 ? dl[0] : kk == 1 ? dl[1] : kk == 2 ? dl[2] : dl[3]);
+                    const float s = kk == 0 ? sx : sy;                 // x, y: through s (1 - s); w, h: through pw, ph
+                    gout[kk] = kk < 2 ? __fmul_rn(__fmul_rn(dn, s), __fsub_rn(1.0f, s)) : __fmul_rn(dn, kk == 2 ? pw : ph);
+                    continue;
+                }
+            }
             const int k = kk < 4 ? kk : kk + 1;
             const float v = widen(cp[(size_t)k * F2]);
             float g;
@@ -287,7 +420,7 @@ using namespace yl;
 
 template <typename T>
 static int loss_forward_impl(const T *raw, const float *labels, int B, int F, int K, int C, int layer_no,
-                             const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                             const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_norm,
                              double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                              int chained, yl_stream_t stream)
 {
@@ -304,8 +437,11 @@ static int loss_forward_impl(const T *raw, const float *labels, int B, int F, in
     // own k_loss_obj (chained != 0): behind a foreign kernel (the producer of raw or labels, the fill of loss4) it is a
     // normal launch, fully ordered after everything earlier on the stream.
     const bool pdl = pdl_enabled();
-    YL_CUDA_TRY(launch_after(k_loss_match<T>, dim3(B, 8), dim3(LS_THREADS), 0, st, pdl && chained != 0, raw, labels, F, K, C, stride, A,
-                             loss4, tcell_all, mcell, mgrad, status));
+    auto match = iou_loss == YL_IOU_LOSS_GIOU ? k_loss_match<T, YL_IOU_LOSS_GIOU>
+               : iou_loss == YL_IOU_LOSS_DIOU ? k_loss_match<T, YL_IOU_LOSS_DIOU>
+               : iou_loss == YL_IOU_LOSS_CIOU ? k_loss_match<T, YL_IOU_LOSS_CIOU> : k_loss_match<T, YL_IOU_LOSS_NONE>;
+    YL_CUDA_TRY(launch_after(match, dim3(B, 8), dim3(LS_THREADS), 0, st, pdl && chained != 0, raw, labels, F, K, C, stride, A,
+                             loss4, tcell_all, mcell, mgrad, status, iou_norm));
     dim3 grid((3 * F * F + LS_THREADS - 1) / LS_THREADS, B);
     YL_CUDA_TRY(launch_after(k_loss_obj<T>, grid, dim3(LS_THREADS), 0, st, pdl, raw, labels, F, K, C, stride, A, ignore_thre,
                              (const int *)tcell_all, loss4, gobj));
@@ -313,23 +449,33 @@ static int loss_forward_impl(const T *raw, const float *labels, int B, int F, in
 }
 
 static int loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
-                              const float *anchors_px, const int *anchor_mask3, float ignore_thre,
+                              const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_norm,
                               double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                               int chained, yl_stream_t stream)
 {
+    if (iou_loss < YL_IOU_LOSS_NONE || iou_loss > YL_IOU_LOSS_CIOU || !(iou_norm >= 0.0f) || isinf(iou_norm)) return YL_ERR_ARG;
     switch (dtype) {
     case YL_DTYPE_F32:
-        return loss_forward_impl((const float *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4,
-                                 gobj, tcell_all, mcell, mgrad, status, chained, stream);
+        return loss_forward_impl((const float *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
+                                 iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     case YL_DTYPE_F16:
-        return loss_forward_impl((const __half *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4,
-                                 gobj, tcell_all, mcell, mgrad, status, chained, stream);
+        return loss_forward_impl((const __half *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
+                                 iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     case YL_DTYPE_BF16:
         return loss_forward_impl((const __nv_bfloat16 *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
-                                 loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+                                 iou_loss, iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     default:
         return YL_ERR_ARG;
     }
+}
+
+extern "C" int yl_loss_forward_ex(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                                  const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss,
+                                  float iou_normalizer, int chained, double *loss4, float *gobj, int *tcell_all, int *mcell,
+                                  float *mgrad, int *status, yl_stream_t stream)
+{
+    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
+                              iou_normalizer, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
 }
 
 extern "C" int yl_loss_forward(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -337,8 +483,8 @@ extern "C" int yl_loss_forward(const float *raw, const float *labels, int B, int
                                double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                yl_stream_t stream)
 {
-    return loss_forward_typed(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
-                              tcell_all, mcell, mgrad, status, 0, stream);
+    return yl_loss_forward_ex(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
+                              YL_IOU_LOSS_NONE, 1.0f, 0, loss4, gobj, tcell_all, mcell, mgrad, status, stream);
 }
 
 extern "C" int yl_loss_forward_chained(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -346,8 +492,8 @@ extern "C" int yl_loss_forward_chained(const float *raw, const float *labels, in
                                        double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                        yl_stream_t stream)
 {
-    return loss_forward_typed(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
-                              tcell_all, mcell, mgrad, status, 1, stream);
+    return yl_loss_forward_ex(raw, YL_DTYPE_F32, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
+                              YL_IOU_LOSS_NONE, 1.0f, 1, loss4, gobj, tcell_all, mcell, mgrad, status, stream);
 }
 
 extern "C" int yl_loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -355,8 +501,8 @@ extern "C" int yl_loss_forward_typed(const void *raw, int dtype, const float *la
                                      double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                      yl_stream_t stream)
 {
-    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
-                              tcell_all, mcell, mgrad, status, 0, stream);
+    return yl_loss_forward_ex(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
+                              YL_IOU_LOSS_NONE, 1.0f, 0, loss4, gobj, tcell_all, mcell, mgrad, status, stream);
 }
 
 extern "C" int yl_loss_forward_chained_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C,
@@ -364,8 +510,8 @@ extern "C" int yl_loss_forward_chained_typed(const void *raw, int dtype, const f
                                              double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                                              yl_stream_t stream)
 {
-    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, loss4, gobj,
-                              tcell_all, mcell, mgrad, status, 1, stream);
+    return yl_loss_forward_ex(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
+                              YL_IOU_LOSS_NONE, 1.0f, 1, loss4, gobj, tcell_all, mcell, mgrad, status, stream);
 }
 
 template <typename T>

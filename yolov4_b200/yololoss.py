@@ -185,12 +185,30 @@ class YOLOLoss(nn.Module):
         return total
 
 
+# iou_loss= of the fused loss -> YL_IOU_LOSS_* (include/yolo_head.h)
+_IOU_LOSS_CODES = {None: 0, "giou": 1, "diou": 2, "ciou": 3}
+
+
+def _iou_args(iou_loss, iou_normalizer):
+    """(YL_IOU_LOSS_* code, fp32 normalizer) of the fused loss's box-term keywords; raises before any CUDA work."""
+    if not (iou_loss is None or isinstance(iou_loss, str)) or iou_loss not in _IOU_LOSS_CODES:
+        raise ValueError("iou_loss must be None, 'giou', 'diou' or 'ciou', got %r" % (iou_loss,))
+    if isinstance(iou_normalizer, (bool, np.bool_)) or not isinstance(iou_normalizer, (int, float, np.integer, np.floating)):
+        raise TypeError("iou_normalizer must be a real number, got %r" % (iou_normalizer,))
+    norm = float(iou_normalizer)
+    if not np.isfinite(norm) or norm < 0.0 or norm > float(np.finfo(np.float32).max):
+        raise ValueError("iou_normalizer must be finite and >= 0, got %r" % (iou_normalizer,))
+    if iou_loss is None and norm != 1.0:
+        raise ValueError("iou_normalizer weights the IoU box term only: it needs iou_loss='giou', 'diou' or 'ciou'")
+    return _IOU_LOSS_CODES[iou_loss], float(np.float32(norm))
+
+
 class _FusedYoloLoss(torch.autograd.Function):
     """N2: raw head tensors + padded labels -> the reference's YOLOLoss.forward value, gradient straight to the raw tensors
     (in the heads' dtype: fp32, fp16 or bf16)."""
 
     @staticmethod
-    def forward(ctx, labels, anchors, anchor_mask, ignore_thresh, n_classes, *raws):
+    def forward(ctx, labels, anchors, anchor_mask, ignore_thresh, n_classes, iou_code, iou_norm, *raws):
         L = _cabi.lib()
         C = int(n_classes)
         dtype = _head_dtype_code(raws)
@@ -219,10 +237,10 @@ class _FusedYoloLoss(torch.autograd.Function):
             # every foreign kernel (contiguous copies, the fills of loss4 / status) is enqueued by now: the calls below are back
             # to back on the stream, so the second and later ones may be launched programmatically behind their predecessor
             for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):
-                fn = L.yl_loss_forward_typed if i == 0 else L.yl_loss_forward_chained_typed
-                _cabi.check(fn(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(anchor_mask[l]),
-                               float(np.float32(ignore_thresh)), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
-                               mcell.data_ptr(), mgrad.data_ptr(), status.data_ptr(), _stream()))
+                _cabi.check(L.yl_loss_forward_ex(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
+                                                 _cabi.ints(anchor_mask[l]), float(np.float32(ignore_thresh)), iou_code,
+                                                 iou_norm, int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
+                                                 mcell.data_ptr(), mgrad.data_ptr(), status.data_ptr(), _stream()))
         ctx.save_for_backward(*saved)
         ctx.shapes = [tuple(r.shape) for r in raws]
         ctx.dtype, ctx.dtype_code = raws[0].dtype, dtype
@@ -245,10 +263,10 @@ class _FusedYoloLoss(torch.autograd.Function):
                 _cabi.check(L.yl_loss_backward_typed(gobj.data_ptr(), mcell.data_ptr(), mgrad.data_ptr(), up.data_ptr(), B, F, ctx.K,
                                                      ctx.C, g.data_ptr(), ctx.dtype_code, _stream()))
                 grads.append(g)
-        return (None, None, None, None, None) + tuple(grads)
+        return (None, None, None, None, None, None, None) + tuple(grads)
 
 
-def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7):
+def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7, iou_loss=None, iou_normalizer=1.0):
     """N2 (SURVEY.md 8f): the value of `YOLOLoss(cfg, ignore_thresh)([YOLOLayer_l.train()(x_l)], {'padded_labels': labels})`
     (yolo/model/yololoss.py:373-443 on top of yololayer.py:122-145) computed from the three raw head tensors without
     materialising output / pred / target / masks; differentiable with respect to the head tensors.
@@ -259,15 +277,26 @@ def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7):
     `[h.float() for h in head_outputs]` up to the order of the fp64 sums, and its gradient has the head's dtype: bit for bit
     the fp32 path's gradient on the widened heads (with the same upstream gradient, e.g. a GradScaler's scale) rounded to
     nearest-even, overflow to +-inf included.  This is not the reference's own half-precision arithmetic.  Mixed dtypes,
-    float64 and CPU heads raise TypeError before any CUDA work."""
-    return _FusedYoloLoss.apply(padded_labels, cfg['ANCHORS'], cfg['ANCHOR_MASK'], ignore_thresh, cfg['N_CLASSES'], *head_outputs)
+    float64 and CPU heads raise TypeError before any CUDA work.
+
+    iou_loss='giou' / 'diou' / 'ciou' (YOLOv4's CIoU box regression, darknet's iou_loss option) replaces the xy BCE and wh MSE
+    of every matched cell by iou_normalizer * torchvision's generalized_ / distance_ / complete_box_iou_loss (eps 1e-7) of the
+    train-mode predicted box and the cell's last GT, in grid units, without tgt_scale weighting; objectness and class terms
+    are unchanged (DESIGN.md section 1).  iou_normalizer (a finite real >= 0) weights the box term only; with iou_loss=None
+    it must stay 1.  A bad keyword raises ValueError (TypeError for a bool normalizer) before any CUDA work."""
+    iou_code, iou_norm = _iou_args(iou_loss, iou_normalizer)
+    return _FusedYoloLoss.apply(padded_labels, cfg['ANCHORS'], cfg['ANCHOR_MASK'], ignore_thresh, cfg['N_CLASSES'], iou_code,
+                                iou_norm, *head_outputs)
 
 
-def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0.7, layers=None):
+def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0.7, layers=None, iou_loss=None,
+                               iou_normalizer=1.0):
     """The four sums (loss_xy, loss_wh, loss_obj, loss_cls; yololoss.py:421-427) over the given layers as a float64[4] device
     tensor, no autograd.  `layers[i]` is the layer number of head_outputs[i] (default 0, 1, 2).  The heads may be float32,
     float16 or bfloat16 CUDA tensors of one dtype: a 16-bit head gives the components of its widened fp32 copy (up to the order
-    of the fp64 sums); mixed dtypes, float64 and CPU heads raise TypeError before any CUDA work."""
+    of the fp64 sums); mixed dtypes, float64 and CPU heads raise TypeError before any CUDA work.  iou_loss / iou_normalizer as
+    for fused_yolo_loss: with an IoU box term, component 0 is that term and component 1 is 0."""
+    iou_code, iou_norm = _iou_args(iou_loss, iou_normalizer)
     L = _cabi.lib()
     dtype = _head_dtype_code(head_outputs)
     dev = head_outputs[0].device
@@ -290,8 +319,8 @@ def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0
             calls.append((rc, F, int(l), gobj, tcell, mcell, mgrad))
             keep += [rc, gobj, tcell, mcell, mgrad]
         for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):     # back to back: see _FusedYoloLoss.forward
-            fn = L.yl_loss_forward_typed if i == 0 else L.yl_loss_forward_chained_typed
-            _cabi.check(fn(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch, _cabi.ints(cfg['ANCHOR_MASK'][l]),
-                           float(np.float32(ignore_thresh)), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
-                           mcell.data_ptr(), mgrad.data_ptr(), None, _stream()))
+            _cabi.check(L.yl_loss_forward_ex(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
+                                             _cabi.ints(cfg['ANCHOR_MASK'][l]), float(np.float32(ignore_thresh)), iou_code,
+                                             iou_norm, int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
+                                             mcell.data_ptr(), mgrad.data_ptr(), None, _stream()))
     return loss4
