@@ -109,7 +109,9 @@ size_t yl_post_workspace_bytes(int B, long M, int C, int cap_seg);
 int yl_post_reset(void *ws, size_t ws_bytes, int B, long M, int C, int cap_seg, yl_stream_t stream);
 
 /* raw[l] = [B, 3*(5+C), F[l], F[l]], l = 0..n_layers-1 (n_layers <= 3), strides 8/16/32 (yololayer.py:54);
- * anchors_px[18] and anchor_mask[9] are cfg MODEL.ANCHORS / ANCHOR_MASK.  M must equal sum 3*F[l]^2.
+ * anchors_px[18] and anchor_mask[9] are cfg MODEL.ANCHORS / ANCHOR_MASK.  M must equal sum 3*F[l]^2.  Any grid sizes F[l] >= 1
+ * work (odd and even, in any mix), at any element-aligned base and any batch size (above 21845 images the kernels are launched
+ * in slices of images).
  * img_first/img_count select a contiguous image range (used to pipeline image groups on several streams). */
 int yl_filter_raw(const float *const *raw, const int *F, int n_layers, int B, int C,
                   const float *anchors_px, const int *anchor_mask, float conf_thre,

@@ -23,7 +23,8 @@ n_cases = int(sys.argv[1]) if len(sys.argv) > 1 else 40
 rng = np.random.RandomState(int(sys.argv[2]) if len(sys.argv) > 2 else 0)
 bad = 0
 for it in range(n_cases):
-    img = int(rng.choice([64, 96, 160, 224, 320, 416]))
+    # 104, 152, 200 and 600 are multiples of 8 but not of 32: an odd grid below an even one (600: 75, 37, 18)
+    img = int(rng.choice([64, 96, 160, 224, 320, 416, 104, 152, 200, 600]))
     C = int(rng.choice([1, 3, 20, 33, 80, 100]))
     B = int(rng.randint(1, 5))
     conf = float(rng.choice([1e-4, 1e-3, 0.01, 0.05, 0.2, 0.5]))

@@ -1088,27 +1088,43 @@ extern "C" int yl_post_reset(void *ws, size_t ws_bytes, int B, long M, int C, in
     return YL_OK;
 }
 
+// gridDim.y (image, anchor) of k_flag_raw / k_emit_flagged is at most 65535.
+constexpr int kSliceImages = 65535 / 3;
+
 // The register-staged flag kernel (unless the caller has already streamed the scales with k_flag_tma) and the emit kernel for
-// element type T.
+// element type T over images [P.img_first, P.img_first + img_count), tiles CTAs along x.  A batch of more than kSliceImages
+// images goes out in slices of that many, one launch per kernel and slice, each told its first image; up to that size each
+// kernel is one launch with the same grid.  Only the first flag slice zeroes the counters (P.reset_words), and every emit
+// slice follows the last flag slice on the stream.  pdl: the first emit launch may overlap its predecessor's tail, which is
+// allowed only when that predecessor is the flag launch whose tables it reads (so not after a sliced flag pass).
 template <typename T>
-static int launch_flag_emit(const RawParams &P, dim3 grid, bool flag, bool emit, bool pdl, int NW, cudaStream_t st)
+static int launch_flag_emit(const RawParams &P, int tiles, int img_count, bool flag, bool emit, bool pdl, int NW, cudaStream_t st)
 {
-    if (flag) {
+    for (int i0 = 0; flag && i0 < img_count; i0 += kSliceImages) {
+        RawParams Q = P;
+        Q.img_first += i0;
+        if (i0 > 0) Q.reset_words = 0;
+        const dim3 grid(tiles, 3 * min(kSliceImages, img_count - i0));
         switch (NW) {
-        case 1: k_flag_raw<T, 1><<<grid, K1_THREADS, 0, st>>>(P); break;
-        case 2: k_flag_raw<T, 2><<<grid, K1_THREADS, 0, st>>>(P); break;
-        case 3: k_flag_raw<T, 3><<<grid, K1_THREADS, 0, st>>>(P); break;
-        default: k_flag_raw<T, 4><<<grid, K1_THREADS, 0, st>>>(P); break;
+        case 1: k_flag_raw<T, 1><<<grid, K1_THREADS, 0, st>>>(Q); break;
+        case 2: k_flag_raw<T, 2><<<grid, K1_THREADS, 0, st>>>(Q); break;
+        case 3: k_flag_raw<T, 3><<<grid, K1_THREADS, 0, st>>>(Q); break;
+        default: k_flag_raw<T, 4><<<grid, K1_THREADS, 0, st>>>(Q); break;
         }
         YL_LAUNCH_CHECK();
     }
-    if (emit) {
+    if (flag && img_count > kSliceImages) pdl = false;
+    for (int i0 = 0; emit && i0 < img_count; i0 += kSliceImages) {
+        RawParams Q = P;
+        Q.img_first += i0;
+        const dim3 grid(tiles, 3 * min(kSliceImages, img_count - i0));
+        const bool pdl_i = pdl && i0 == 0;
         cudaError_t le;
         switch (NW) {
-        case 1: le = launch_after(k_emit_flagged<T, 1>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
-        case 2: le = launch_after(k_emit_flagged<T, 2>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
-        case 3: le = launch_after(k_emit_flagged<T, 3>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
-        default: le = launch_after(k_emit_flagged<T, 4>, grid, dim3(K1_THREADS), 0, st, pdl, P); break;
+        case 1: le = launch_after(k_emit_flagged<T, 1>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
+        case 2: le = launch_after(k_emit_flagged<T, 2>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
+        case 3: le = launch_after(k_emit_flagged<T, 3>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
+        default: le = launch_after(k_emit_flagged<T, 4>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
         }
         if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
     }
@@ -1162,9 +1178,11 @@ static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int 
             Ly.ah[a] = (float)((double)anchors_px[2 * q + 1] / (double)Ly.stride);
         }
         // 128-bit loads / bulk copies need 16-byte aligned planes: F^2 % 4 == 0 and an aligned base (19x19, 13x13 fall back).
-        // 16-bit planes are read with 64-bit loads where F^2 % 4 == 0 and the base is 8-byte aligned; their tables are then
-        // stored as uint4, so the scale's rows of them must start 16-byte aligned as well.
-        if (f32) Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 16 == 0)) ? 4 : 1;
+        // 16-bit planes are read with 64-bit loads where F^2 % 4 == 0 and the base is 8-byte aligned.  Either way the flag and
+        // objectness tables of a vector scale are stored and loaded as uint4 / float4 at row b*M4 + row_off + a*F^2 + p, so the
+        // scale's rows must start 16-byte aligned as well: a lower scale with an odd grid (e.g. 75x75 below 38x38) makes row_off
+        // odd, and the scale then takes the scalar path.
+        if (f32) Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 16 == 0) && row_off % 4 == 0) ? 4 : 1;
         else Ly.vec = ((Ly.F2 % 4 == 0) && (((uintptr_t)raw[l]) % 8 == 0) && row_off % 4 == 0) ? 4 : 1;
         Ly.tma = (Ly.vec == 4 && n_cc >= FT_STAGES) ? 1 : 0;              // k_flag_tma's ring needs FT_STAGES class chunks
         Ly.tile_boxes = 0; Ly.tiles = 0;
@@ -1210,7 +1228,6 @@ static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int 
     }
 
     // ---- streaming flag kernel ----
-    const dim3 grid(tiles_ldg, img_count * 3);
     if ((stages & 1) && persistent) {
         const int nba = img_count * 3;
         unsigned *tile_counter = (unsigned *)(w + L.off_tile_count) + img_first;
@@ -1245,9 +1262,9 @@ static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int 
     const bool flag_ldg = (stages & 1) && !persistent;
     const bool pdl = pdl_enabled() && (stages & 1);                         // the emit kernel directly follows the flag kernel
     switch (dtype) {
-    case YL_DTYPE_F16: return launch_flag_emit<__half>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
-    case YL_DTYPE_BF16: return launch_flag_emit<__nv_bfloat16>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
-    default: return launch_flag_emit<float>(Pl, grid, flag_ldg, stages & 2, pdl, NW, st);
+    case YL_DTYPE_F16: return launch_flag_emit<__half>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
+    case YL_DTYPE_BF16: return launch_flag_emit<__nv_bfloat16>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
+    default: return launch_flag_emit<float>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
     }
 }
 
