@@ -63,6 +63,15 @@ int yl_selftest_rcp(unsigned long long *bad_dev, yl_stream_t stream);
  * --------------------------------------------------------------------------------------------------------- */
 int yl_decode_dense(const float *raw, int B, int F, int C, const float *anch_grid, float stride,
                     float *out, long rows_per_image, long row_offset, yl_stream_t stream);
+/* yl_decode_dense with YOLOv4's grid-sensitivity decode (darknet's scale_x_y; DESIGN.md section 1).  With s = scale_x_y and
+ * beta = fl32(-0.5 * (s - 1)) evaluated in float64, the box centre of cell (i, j) is
+ *   cx = fl(fl(fl(sigmoid(tx) * s) + beta) + i),  bx = fl(cx * stride)           (cy, by likewise with j)
+ * every operation one fp32 rounding in this order; w, h, objectness and classes are unchanged, and nothing is clamped (a centre
+ * may leave its cell).  s = 1 is yl_decode_dense (the same launch, the same bytes; yl_decode_dense is this call with 1), s = 2
+ * is the 2 sigmoid - 0.5 centre of YOLOv5 / Scaled-YOLOv4.  A NaN, infinite or non-positive s returns YL_ERR_ARG before any
+ * CUDA call. */
+int yl_decode_dense_ex(const float *raw, int B, int F, int C, const float *anch_grid, float stride, float scale_x_y,
+                       float *out, long rows_per_image, long row_offset, yl_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * A3  YOLOLayer.forward, train branch                      replaces yolo/model/yololayer.py:122-145
@@ -135,6 +144,14 @@ int yl_filter_raw_stage(const float *const *raw, const int *F, int n_layers, int
 int yl_filter_raw_typed(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
                         const float *anchors_px, const int *anchor_mask, float conf_thre, void *ws, size_t ws_bytes,
                         long M, int cap_seg, int img_first, int img_count, int stages, yl_stream_t stream);
+
+/* yl_filter_raw_typed with YOLOv4's grid-sensitivity decode: scale_x_y[l] is head l's scale (the centre of yl_decode_dense_ex),
+ * NULL = every scale 1.  Only the boxes of the candidates change; which (box, class) pairs pass the threshold does not depend
+ * on the box.  NULL, or every scale exactly 1, is yl_filter_raw_typed (the same launches, the same bytes; yl_filter_raw_typed
+ * is this call with NULL).  A NaN, infinite or non-positive scale returns YL_ERR_ARG before any CUDA call. */
+int yl_filter_raw_ex(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
+                     const float *anchors_px, const int *anchor_mask, float conf_thre, const float *scale_x_y /* [n_layers] */,
+                     void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count, int stages, yl_stream_t stream);
 
 /* pred [B, M, 5+C] decoded (cx,cy,w,h,obj,cls...), not modified (the reference's in-place xyxy overwrite,
  * utils.py:126, is an unobserved side effect).  num_classes <= C limits the row pre-filter (utils.py:139). */
@@ -313,6 +330,17 @@ int yl_loss_forward_ex(const void *raw, int dtype, const float *labels, int B, i
                        const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_normalizer,
                        int chained, double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                        yl_stream_t stream);
+/* yl_loss_forward_ex with YOLOv4's grid-sensitivity decode of the layer (darknet's scale_x_y, which yolov4.cfg pairs with
+ * iou_loss = ciou).  The train-mode predicted box p of the ignore test and of the IoU box term takes the centre
+ * fl(fl(fl(sigmoid(tx) * s) + beta) + i) (beta as for yl_decode_dense_ex; cy likewise), and d px / d tx = s sigmoid (1 - sigmoid):
+ * mgrad[..., 0:2] = fl(fl(fl(iou_normalizer * d L / d px) * s) * sigmoid) * (1 - sigmoid).  w / h, the objectness and class
+ * terms and yl_loss_backward[_typed] are unchanged.  s = 1 is yl_loss_forward_ex (the same launches, the same bytes;
+ * yl_loss_forward_ex is this call with 1).  A NaN, infinite or non-positive s, or s != 1 with YL_IOU_LOSS_NONE (the BCE xy
+ * term has no scaled form), returns YL_ERR_ARG before any CUDA call. */
+int yl_loss_forward_ex2(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                        const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_normalizer,
+                        float scale_x_y, int chained, double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad,
+                        int *status, yl_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Host-buffer entry (what a non-Python caller binds; also the bench's end-to-end leg): raw head tensors in
@@ -350,6 +378,11 @@ int yl_detect_host_ex(yl_context *ctx, const float *const *raw_host, float conf_
  * anything else returns YL_ERR_ARG before any CUDA call. */
 int yl_detect_host_ex2(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det, int agnostic,
                        int diou, float *out_rows_host, int *counts_host);
+/* yl_detect_host_ex2 with YOLOv4's grid-sensitivity decode (yl_filter_raw_ex): scale_x_y[l] is head l's scale, NULL = every
+ * scale 1 (yl_detect_host_ex2 is this call with NULL).  A NaN, infinite or non-positive scale returns YL_ERR_ARG before any
+ * CUDA call. */
+int yl_detect_host_ex3(yl_context *ctx, const float *const *raw_host, float conf_thre, float nms_thre, int max_det, int agnostic,
+                       int diou, const float *scale_x_y /* [n_layers] */, float *out_rows_host, int *counts_host);
 
 /* ---------------------------------------------------------------------------------------------------------
  * (e) Multi-GPU: the final exchange of the image-sharded path            (SURVEY.md 8(e); no reference counterpart: the

@@ -51,6 +51,8 @@ def lib():
     L.yl_selftest_rcp.argtypes = [_p, _p]
     L.yl_decode_dense.restype = _i
     L.yl_decode_dense.argtypes = [_p, _i, _i, _i, _p, _f, _p, _l, _l, _p]
+    L.yl_decode_dense_ex.restype = _i
+    L.yl_decode_dense_ex.argtypes = [_p, _i, _i, _i, _p, _f, _f, _p, _l, _l, _p]
     L.yl_decode_train.restype = _i
     L.yl_decode_train.argtypes = [_p, _i, _i, _i, _p, _p, _p, _p]
     L.yl_decode_train_backward.restype = _i
@@ -67,6 +69,8 @@ def lib():
     L.yl_filter_raw_stage.argtypes = [_p, _p, _i, _i, _i, _p, _p, _f, _p, _sz, _l, _i, _i, _i, _i, _p]
     L.yl_filter_raw_typed.restype = _i
     L.yl_filter_raw_typed.argtypes = [_p, _i, _p, _i, _i, _i, _p, _p, _f, _p, _sz, _l, _i, _i, _i, _i, _p]
+    L.yl_filter_raw_ex.restype = _i
+    L.yl_filter_raw_ex.argtypes = [_p, _i, _p, _i, _i, _i, _p, _p, _f, _p, _p, _sz, _l, _i, _i, _i, _i, _p]
     L.yl_filter_dense.restype = _i
     L.yl_filter_dense.argtypes = [_p, _i, _l, _i, _i, _f, _p, _sz, _i, _i, _i, _p]
     L.yl_nms.restype = _i
@@ -99,6 +103,8 @@ def lib():
     L.yl_loss_forward_chained_typed.argtypes = L.yl_loss_forward_typed.argtypes
     L.yl_loss_forward_ex.restype = _i
     L.yl_loss_forward_ex.argtypes = [_p, _i, _p, _i, _i, _i, _i, _i, _p, _p, _f, _i, _f, _i, _p, _p, _p, _p, _p, _p, _p]
+    L.yl_loss_forward_ex2.restype = _i
+    L.yl_loss_forward_ex2.argtypes = [_p, _i, _p, _i, _i, _i, _i, _i, _p, _p, _f, _i, _f, _f, _i, _p, _p, _p, _p, _p, _p, _p]
     L.yl_loss_backward_typed.restype = _i
     L.yl_loss_backward_typed.argtypes = [_p, _p, _p, _p, _i, _i, _i, _i, _p, _i, _p]
     L.yl_context_create.restype = _i
@@ -115,6 +121,8 @@ def lib():
     L.yl_detect_host_ex.argtypes = [_p, _p, _f, _f, _i, _i, _p, _p]
     L.yl_detect_host_ex2.restype = _i
     L.yl_detect_host_ex2.argtypes = [_p, _p, _f, _f, _i, _i, _i, _p, _p]
+    L.yl_detect_host_ex3.restype = _i
+    L.yl_detect_host_ex3.argtypes = [_p, _p, _f, _f, _i, _i, _i, _p, _p, _p]
     L.yl_xchg_create.restype = _i
     L.yl_xchg_create.argtypes = [ctypes.POINTER(_p), _i, _i, _i, _i, _l, _i]
     L.yl_xchg_window_bytes.restype = _sz
@@ -147,10 +155,10 @@ def lib():
 
 
 EXPORTS = [
-    "yl_abi_version", "yl_source_hash", "yl_error_string", "yl_selftest_rcp", "yl_decode_dense", "yl_decode_train", "yl_decode_train_backward", "yl_decode_train_backward_raw",
-    "yl_post_workspace_bytes", "yl_post_reset", "yl_filter_raw", "yl_filter_raw_stage", "yl_filter_raw_typed", "yl_filter_dense", "yl_nms", "yl_nms_topk", "yl_nms_ex", "yl_nms_ex2", "yl_post_workspace_bytes_ex", "yl_build_target", "yl_build_target3", "yl_coco_rows", "yl_coco_rows_padded",
-    "yl_loss_forward", "yl_loss_forward_chained", "yl_loss_backward", "yl_loss_forward_typed", "yl_loss_forward_chained_typed", "yl_loss_backward_typed", "yl_loss_forward_ex",
-    "yl_context_create", "yl_context_create_typed", "yl_context_destroy", "yl_detect_host", "yl_detect_host_topk", "yl_detect_host_ex", "yl_detect_host_ex2",
+    "yl_abi_version", "yl_source_hash", "yl_error_string", "yl_selftest_rcp", "yl_decode_dense", "yl_decode_dense_ex", "yl_decode_train", "yl_decode_train_backward", "yl_decode_train_backward_raw",
+    "yl_post_workspace_bytes", "yl_post_reset", "yl_filter_raw", "yl_filter_raw_stage", "yl_filter_raw_typed", "yl_filter_raw_ex", "yl_filter_dense", "yl_nms", "yl_nms_topk", "yl_nms_ex", "yl_nms_ex2", "yl_post_workspace_bytes_ex", "yl_build_target", "yl_build_target3", "yl_coco_rows", "yl_coco_rows_padded",
+    "yl_loss_forward", "yl_loss_forward_chained", "yl_loss_backward", "yl_loss_forward_typed", "yl_loss_forward_chained_typed", "yl_loss_backward_typed", "yl_loss_forward_ex", "yl_loss_forward_ex2",
+    "yl_context_create", "yl_context_create_typed", "yl_context_destroy", "yl_detect_host", "yl_detect_host_topk", "yl_detect_host_ex", "yl_detect_host_ex2", "yl_detect_host_ex3",
     "yl_xchg_create", "yl_xchg_create_external", "yl_xchg_window_bytes", "yl_xchg_destroy", "yl_xchg_handle_bytes", "yl_xchg_local_handle", "yl_xchg_connect", "yl_xchg_push",
     "yl_xchg_wait", "yl_xchg_release", "yl_xchg_rows", "yl_xchg_counts", "yl_xchg_status",
 ]

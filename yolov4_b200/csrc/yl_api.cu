@@ -143,13 +143,15 @@ extern "C" int yl_context_create(yl_context **out, int device, int B, const int 
     return yl_context_create_typed(out, device, B, F, n_layers, C, YL_DTYPE_F32, anchors_px, anchor_mask, cap_seg, cap_out);
 }
 
-extern "C" int yl_detect_host_ex2(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
-                                  int agnostic, int diou, float *out_rows_host, int *counts_host)
+extern "C" int yl_detect_host_ex3(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
+                                  int agnostic, int diou, const float *scale_x_y, float *out_rows_host, int *counts_host)
 {
     if (!c || !raw_host || !out_rows_host || !counts_host) return YL_ERR_ARG;
     if (max_det < 0 || max_det > c->cap_out) return YL_ERR_ARG;
     if (agnostic != 0 && agnostic != 1) return YL_ERR_ARG;
     if (diou != 0 && diou != 1) return YL_ERR_ARG;
+    for (int l = 0; scale_x_y && l < c->n_layers; ++l)
+        if (!yl::scale_xy_valid(scale_x_y[l])) return YL_ERR_ARG;
     YL_CUDA_TRY(cudaSetDevice(c->device));
     const int B = c->B, C = c->C, G = c->n_groups;
     const size_t need = yl_post_workspace_bytes_ex(B, c->M, C, c->cap_seg, agnostic);
@@ -176,8 +178,8 @@ extern "C" int yl_detect_host_ex2(yl_context *c, const float *const *raw_host, f
         }
         YL_CUDA_TRY(cudaEventRecord(c->ev_copied[g], c->s_copy));
         YL_CUDA_TRY(cudaStreamWaitEvent(c->s_comp, c->ev_copied[g], 0));
-        rc = yl_filter_raw_typed((const void *const *)c->d_raw, c->dtype, c->F, c->n_layers, B, C, c->anchors, c->mask, conf_thre,
-                                 c->ws, c->ws_bytes, c->M, c->cap_seg, i0, i1 - i0, 3, c->s_comp);
+        rc = yl_filter_raw_ex((const void *const *)c->d_raw, c->dtype, c->F, c->n_layers, B, C, c->anchors, c->mask, conf_thre,
+                              scale_x_y, c->ws, c->ws_bytes, c->M, c->cap_seg, i0, i1 - i0, 3, c->s_comp);
         if (rc != YL_OK) return rc;
         rc = yl_nms_ex2(c->ws, c->ws_bytes, B, c->M, C, c->cap_seg, nms_thre, max_det, agnostic, diou, c->d_rows, c->cap_out,
                         c->d_meta, nullptr, i0, i1 - i0, c->s_comp);
@@ -209,10 +211,16 @@ extern "C" int yl_detect_host_ex2(yl_context *c, const float *const *raw_host, f
     return status;
 }
 
+extern "C" int yl_detect_host_ex2(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
+                                  int agnostic, int diou, float *out_rows_host, int *counts_host)
+{
+    return yl_detect_host_ex3(c, raw_host, conf_thre, nms_thre, max_det, agnostic, diou, nullptr, out_rows_host, counts_host);
+}
+
 extern "C" int yl_detect_host_ex(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,
                                  int agnostic, float *out_rows_host, int *counts_host)
 {
-    return yl_detect_host_ex2(c, raw_host, conf_thre, nms_thre, max_det, agnostic, 0, out_rows_host, counts_host);
+    return yl_detect_host_ex3(c, raw_host, conf_thre, nms_thre, max_det, agnostic, 0, nullptr, out_rows_host, counts_host);
 }
 
 extern "C" int yl_detect_host_topk(yl_context *c, const float *const *raw_host, float conf_thre, float nms_thre, int max_det,

@@ -13,10 +13,13 @@ namespace yl {
 constexpr int DD_TP = 64;          // boxes per tile
 constexpr int DD_THREADS = 256;    // 4 channel rows x 64 boxes per pass
 
+// SXY: the centres take the grid-sensitivity decode fl(fl(fl(sigmoid(t) * sxy) + beta) + cell) (scale_x_y, DESIGN.md section 1);
+// otherwise sxy / beta are not read.
+template <bool SXY>
 __global__ void __launch_bounds__(DD_THREADS)
 k_decode_dense(const float *__restrict__ raw, int Fw, int F2, int C, float stride,
                float aw0, float ah0, float aw1, float ah1, float aw2, float ah2,
-               float *__restrict__ out, long rows_per_image, long row_offset, int ba0)
+               float *__restrict__ out, long rows_per_image, long row_offset, int ba0, float sxy, float beta)
 {
     extern __shared__ __align__(16) float tile[];   // [DD_TP][nch]: the output layout itself (odd nch, e.g. 85: conflict-free stores)
     const int nch = 5 + C;
@@ -52,6 +55,9 @@ k_decode_dense(const float *__restrict__ raw, int Fw, int F2, int C, float strid
             spec_sigmoid_batch<8>(t, sg);                              // one range test for the batch
             if (kr >= 2) sg[0] = spec_expf(t[0]);                       // tw / th
             float v0;
+            if constexpr (SXY) {
+                if (kr < 2) sg[0] = __fadd_rn(__fmul_rn(sg[0], sxy), beta);
+            }
             if (kr == 0) v0 = __fmul_rn(__fadd_rn(sg[0], (float)gx), stride);
             else if (kr == 1) v0 = __fmul_rn(__fadd_rn(sg[0], (float)gy), stride);
             else if (kr == 2) v0 = __fmul_rn(__fmul_rn(sg[0], aw), stride);
@@ -191,16 +197,20 @@ k_decode_train_bwd(const float *__restrict__ src, const float *__restrict__ grad
 
 using namespace yl;
 
-extern "C" int yl_decode_dense(const float *raw, int B, int F, int C, const float *ag, float stride,
-                               float *out, long rows_per_image, long row_offset, yl_stream_t stream)
+extern "C" int yl_decode_dense_ex(const float *raw, int B, int F, int C, const float *ag, float stride, float scale_x_y,
+                                  float *out, long rows_per_image, long row_offset, yl_stream_t stream)
 {
     if (!raw || !ag || !out || B <= 0 || F <= 0 || C <= 0 || rows_per_image < 3L * F * F + row_offset || row_offset < 0)
         return YL_ERR_ARG;
-    if (3L * B > 0x7FFFFFFFL) return YL_ERR_ARG;
+    if (3L * B > 0x7FFFFFFFL || !scale_xy_valid(scale_x_y)) return YL_ERR_ARG;
     const int F2 = F * F;
     const size_t smem = sizeof(float) * DD_TP * (5 + C);
+    // a scale of exactly 1 is the unscaled kernel (the same launch and bytes as yl_decode_dense)
+    const bool scaled = scale_x_y != 1.0f;
+    const float beta = scale_xy_beta(scale_x_y);
+    auto kernel = scaled ? k_decode_dense<true> : k_decode_dense<false>;
     if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(k_decode_dense, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return YL_ERR_CUDA_BASE + (int)e;
     }
     // gridDim.y is at most 65535: larger batches go out in slices of (image, anchor) pairs, one launch when B*3 fits
@@ -208,11 +218,17 @@ extern "C" int yl_decode_dense(const float *raw, int B, int F, int C, const floa
     const long pairs = 3L * B;
     for (long ba0 = 0; ba0 < pairs; ba0 += kMaxGridY) {
         dim3 grid((F2 + DD_TP - 1) / DD_TP, (unsigned)min((long)kMaxGridY, pairs - ba0));
-        k_decode_dense<<<grid, DD_THREADS, smem, (cudaStream_t)stream>>>(raw, F, F2, C, stride, ag[0], ag[1], ag[2], ag[3],
-                                                                         ag[4], ag[5], out, rows_per_image, row_offset, (int)ba0);
+        kernel<<<grid, DD_THREADS, smem, (cudaStream_t)stream>>>(raw, F, F2, C, stride, ag[0], ag[1], ag[2], ag[3], ag[4], ag[5], out,
+                                                                 rows_per_image, row_offset, (int)ba0, scale_x_y, beta);
         YL_LAUNCH_CHECK();
     }
     return YL_OK;
+}
+
+extern "C" int yl_decode_dense(const float *raw, int B, int F, int C, const float *ag, float stride,
+                               float *out, long rows_per_image, long row_offset, yl_stream_t stream)
+{
+    return yl_decode_dense_ex(raw, B, F, C, ag, stride, 1.0f, out, rows_per_image, row_offset, stream);
 }
 
 extern "C" int yl_decode_train(const float *raw, int B, int F, int C, const float *ag,

@@ -112,11 +112,25 @@ struct EmitWarp {
     float4 box[128];                   // decoded corners of the box slots that have a surviving pair
 };
 
-__device__ __forceinline__ float4 decode_box_v(float tx, float ty, float tw, float th, int Fw, int p, float aw, float ah, float stride)
+// Per-scale grid-sensitivity decode (scale_x_y, DESIGN.md section 1): centre = fl(fl(fl(sigmoid(t) * s) + beta) + cell), beta =
+// -(s - 1) / 2.  A kernel parameter of its own after RawParams, so that the flag kernels and RawParams keep their layout.
+struct ScaleXY { float s[3], beta[3]; };
+
+// Grid-unit centre of one box: sigmoid(t) + cell, or with SXY the scaled form above.
+template <bool SXY>
+__device__ __forceinline__ float centre(float sg, int cell, float sxy, float beta)
+{
+    if constexpr (SXY) return __fadd_rn(__fadd_rn(__fmul_rn(sg, sxy), beta), (float)cell);
+    else return __fadd_rn(sg, (float)cell);
+}
+
+template <bool SXY>
+__device__ __forceinline__ float4 decode_box_v(float tx, float ty, float tw, float th, int Fw, int p, float aw, float ah, float stride,
+                                               float sxy, float beta)
 {
     const int gy = p / Fw, gx = p - gy * Fw;
-    const float bx = __fmul_rn(__fadd_rn(spec_sigmoidf(tx), (float)gx), stride);
-    const float by = __fmul_rn(__fadd_rn(spec_sigmoidf(ty), (float)gy), stride);
+    const float bx = __fmul_rn(centre<SXY>(spec_sigmoidf(tx), gx, sxy, beta), stride);
+    const float by = __fmul_rn(centre<SXY>(spec_sigmoidf(ty), gy, sxy, beta), stride);
     const float bw = __fmul_rn(__fmul_rn(spec_expf(tw), aw), stride);
     const float bh = __fmul_rn(__fmul_rn(spec_expf(th), ah), stride);
     const float hw = __fmul_rn(bw, 0.5f), hh = __fmul_rn(bh, 0.5f);
@@ -124,11 +138,11 @@ __device__ __forceinline__ float4 decode_box_v(float tx, float ty, float tw, flo
 }
 
 // Decode one box (yololayer.py:150-162) and convert to corners (utils.py:117-126).
-template <typename T>
-__device__ __forceinline__ float4 decode_box(const T *bp, int F2, int Fw, int p, float aw, float ah, float stride)
+template <typename T, bool SXY>
+__device__ __forceinline__ float4 decode_box(const T *bp, int F2, int Fw, int p, float aw, float ah, float stride, float sxy, float beta)
 {
     const float tx = widen(bp[0]), ty = widen(bp[(size_t)F2]), tw = widen(bp[2 * (size_t)F2]), th = widen(bp[3 * (size_t)F2]);
-    return decode_box_v(tx, ty, tw, th, Fw, p, aw, ah, stride);
+    return decode_box_v<SXY>(tx, ty, tw, th, Fw, p, aw, ah, stride, sxy, beta);
 }
 
 // Exact pass over one batch of `total` queued (box slot, class) pairs of a warp tile.  All lanes take part:
@@ -150,9 +164,9 @@ __device__ __forceinline__ int nth_slot(const unsigned (&w)[4], const int (&c)[4
     return 32 * j + (int)__fns(wsel, 0, i - cs + 1);
 }
 
-template <typename T, int VEC>
+template <typename T, int VEC, bool SXY>
 __device__ __forceinline__ void emit_batch(const RawParams &P, const RawLayer &Ly, EmitWarp &E, const float *sobj,
-                                           const T *wbase, int b, int a, int wp0, int total)
+                                           const T *wbase, int b, int a, int wp0, int total, float sxy, float beta)
 {
     const int lane = threadIdx.x & 31;
     const int C = P.C, F2 = Ly.F2;
@@ -202,11 +216,11 @@ __device__ __forceinline__ void emit_batch(const RawParams &P, const RawLayer &L
     }
     __syncwarp();
     if (sbs >= 0 && (((E.any[sbs >> 5] & ~E.nan[sbs >> 5]) >> (sbs & 31)) & 1u))
-        E.box[sbs] = decode_box_v(tx, ty, tw, th, Ly.Fw, wp0 + sbs, Ly.aw[a], Ly.ah[a], Ly.stride);
+        E.box[sbs] = decode_box_v<SXY>(tx, ty, tw, th, Ly.Fw, wp0 + sbs, Ly.aw[a], Ly.ah[a], Ly.stride, sxy, beta);
     for (int i = lane + 32; i < nflag; i += 32) {                    // more than 32 flagged boxes in the batch (dense inputs)
         const int bs = nth_slot(fw, fc, i);
         if (((E.any[bs >> 5] & ~E.nan[bs >> 5]) >> (bs & 31)) & 1u)
-            E.box[bs] = decode_box(wbase + bs, F2, Ly.Fw, wp0 + bs, Ly.aw[a], Ly.ah[a], Ly.stride);
+            E.box[bs] = decode_box<T, SXY>(wbase + bs, F2, Ly.Fw, wp0 + bs, Ly.aw[a], Ly.ah[a], Ly.stride, sxy, beta);
     }
     __syncwarp();
     for (int q0 = 0; q0 < total; q0 += 128) {
@@ -300,9 +314,10 @@ __device__ __forceinline__ void queue_pairs(const unsigned (&bits)[VEC][NW], con
 // position a warp prefix sum gives it, and the queue is resolved as one batch.  Dense tiles fall back to expanding the
 // flag words box by box and resolving the queue in batches of whole boxes.  sobj must already hold
 // sigmoid(objectness) per box slot.
-template <typename T, int VEC, int NW>
+template <typename T, int VEC, int NW, bool SXY>
 __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &Ly, int ba, int wp0,
-                                           const float (&lth)[VEC], unsigned (&bits)[VEC][NW], EmitWarp &E, const float *sobj)
+                                           const float (&lth)[VEC], unsigned (&bits)[VEC][NW], EmitWarp &E, const float *sobj,
+                                           float sxy, float beta)
 {
     const unsigned FULL = 0xFFFFFFFFu;
     const int lane = threadIdx.x & 31;
@@ -316,7 +331,7 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
     __syncwarp();
     if (total <= K1_QCAP) {
         queue_pairs<VEC, NW>(bits, anyv, first, E.ent, E.flg);
-        emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, total);
+        emit_batch<T, VEC, SXY>(P, Ly, E, sobj, wbase, b, a, wp0, total, sxy, beta);
         return;
     }
     unsigned flagged[VEC];
@@ -333,7 +348,7 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
             int n = 0;
 #pragma unroll
             for (int w = 0; w < NW; ++w) { m[w] = __shfl_sync(FULL, bits[v][w], L); n += __popc(m[w]); }
-            if (qb + n > K1_QCAP) { emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb); qb = 0; __syncwarp(); }
+            if (qb + n > K1_QCAP) { emit_batch<T, VEC, SXY>(P, Ly, E, sobj, wbase, b, a, wp0, qb, sxy, beta); qb = 0; __syncwarp(); }
             const int bs = L * VEC + v;
             if (lane == 0) E.flg[bs >> 5] |= 1u << (bs & 31);
             const unsigned hdr = (unsigned)bs << 8;
@@ -344,7 +359,7 @@ __device__ __forceinline__ void emit_pairs(const RawParams &P, const RawLayer &L
             }
         }
     }
-    if (qb) emit_batch<T, VEC>(P, Ly, E, sobj, wbase, b, a, wp0, qb);
+    if (qb) emit_batch<T, VEC, SXY>(P, Ly, E, sobj, wbase, b, a, wp0, qb, sxy, beta);
 }
 
 // One tile = K1_THREADS*VEC consecutive boxes of one (image, anchor).  Phase 1 (the flag kernels) streams the class
@@ -493,8 +508,8 @@ k_flag_raw(const __grid_constant__ RawParams P)
     else flag_tile<T, 1, NW>(P, P.layer[l], tile, ba);
 }
 
-template <typename T, int VEC, int NW>
-__device__ __forceinline__ void emit_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba, LdgSmem &sm)
+template <typename T, int VEC, int NW, bool SXY>
+__device__ __forceinline__ void emit_tile(const RawParams &P, const RawLayer &Ly, int tile, int ba, LdgSmem &sm, float sxy, float beta)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int p0 = (tile * K1_THREADS + threadIdx.x) * VEC;
@@ -529,15 +544,14 @@ __device__ __forceinline__ void emit_tile(const RawParams &P, const RawLayer &Ly
     if (!__any_sync(0xFFFFFFFFu, any != 0u)) return;                 // warp-uniform: nothing flagged in these 32*VEC boxes
     if (VEC == 4) *reinterpret_cast<float4 *>(&sm.sobj[warp][lane * 4]) = o;
     else sm.sobj[warp][lane] = o.x;
-    emit_pairs<T, VEC, NW>(P, Ly, ba, (tile * K1_THREADS + warp * 32) * VEC, lth, bits, sm.e[warp], sm.sobj[warp]);
+    emit_pairs<T, VEC, NW, SXY>(P, Ly, ba, (tile * K1_THREADS + warp * 32) * VEC, lth, bits, sm.e[warp], sm.sobj[warp], sxy, beta);
 }
 
 #ifndef YL_EMIT_MINB
 #define YL_EMIT_MINB 8
 #endif
-template <typename T, int NW>
-__global__ void __launch_bounds__(K1_THREADS, YL_EMIT_MINB)
-k_emit_flagged(const __grid_constant__ RawParams P)
+template <typename T, int NW, bool SXY>
+__device__ __forceinline__ void emit_flagged(const RawParams &P, const ScaleXY &S)
 {
     __shared__ LdgSmem sm;
     pdl_trigger();
@@ -548,8 +562,23 @@ k_emit_flagged(const __grid_constant__ RawParams P)
     int tile = (int)gridDim.x - 1 - (int)blockIdx.x;
     int l = 0;
     while (l < P.n_layers - 1 && tile >= P.layer[l].tiles) { tile -= P.layer[l].tiles; ++l; }
-    if (P.layer[l].vec == 4) emit_tile<T, 4, NW>(P, P.layer[l], tile, ba, sm);
-    else emit_tile<T, 1, NW>(P, P.layer[l], tile, ba, sm);
+    if (P.layer[l].vec == 4) emit_tile<T, 4, NW, SXY>(P, P.layer[l], tile, ba, sm, S.s[l], S.beta[l]);
+    else emit_tile<T, 1, NW, SXY>(P, P.layer[l], tile, ba, sm, S.s[l], S.beta[l]);
+}
+
+// Two overloads of one kernel: the plain decode, and the grid-sensitivity decode with the per-scale scale_x_y of S.
+template <typename T, int NW>
+__global__ void __launch_bounds__(K1_THREADS, YL_EMIT_MINB)
+k_emit_flagged(const __grid_constant__ RawParams P)
+{
+    emit_flagged<T, NW, false>(P, ScaleXY{});
+}
+
+template <typename T, int NW>
+__global__ void __launch_bounds__(K1_THREADS, YL_EMIT_MINB)
+k_emit_flagged(const __grid_constant__ RawParams P, const __grid_constant__ ScaleXY S)
+{
+    emit_flagged<T, NW, true>(P, S);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1097,8 +1126,10 @@ constexpr int kSliceImages = 65535 / 3;
 // kernel is one launch with the same grid.  Only the first flag slice zeroes the counters (P.reset_words), and every emit
 // slice follows the last flag slice on the stream.  pdl: the first emit launch may overlap its predecessor's tail, which is
 // allowed only when that predecessor is the flag launch whose tables it reads (so not after a sliced flag pass).
+// sxy: the per-scale scale_x_y of the emit kernel, or nullptr for the unscaled decode.
 template <typename T>
-static int launch_flag_emit(const RawParams &P, int tiles, int img_count, bool flag, bool emit, bool pdl, int NW, cudaStream_t st)
+static int launch_flag_emit(const RawParams &P, const ScaleXY *sxy, int tiles, int img_count, bool flag, bool emit, bool pdl, int NW,
+                            cudaStream_t st)
 {
     for (int i0 = 0; flag && i0 < img_count; i0 += kSliceImages) {
         RawParams Q = P;
@@ -1120,25 +1151,43 @@ static int launch_flag_emit(const RawParams &P, int tiles, int img_count, bool f
         const dim3 grid(tiles, 3 * min(kSliceImages, img_count - i0));
         const bool pdl_i = pdl && i0 == 0;
         cudaError_t le;
+        void (*plain)(RawParams);
+        void (*scaled)(RawParams, ScaleXY);
+#define YL_EMIT_CASE(NW_)                                                                                                    \
+        plain = k_emit_flagged<T, NW_>;                                                                                      \
+        scaled = k_emit_flagged<T, NW_>;                                                                                     \
+        le = sxy ? launch_after(scaled, grid, dim3(K1_THREADS), 0, st, pdl_i, Q, *sxy)                                       \
+                 : launch_after(plain, grid, dim3(K1_THREADS), 0, st, pdl_i, Q);
         switch (NW) {
-        case 1: le = launch_after(k_emit_flagged<T, 1>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
-        case 2: le = launch_after(k_emit_flagged<T, 2>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
-        case 3: le = launch_after(k_emit_flagged<T, 3>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
-        default: le = launch_after(k_emit_flagged<T, 4>, grid, dim3(K1_THREADS), 0, st, pdl_i, Q); break;
+        case 1: YL_EMIT_CASE(1) break;
+        case 2: YL_EMIT_CASE(2) break;
+        case 3: YL_EMIT_CASE(3) break;
+        default: YL_EMIT_CASE(4) break;
         }
+#undef YL_EMIT_CASE
         if (le != cudaSuccess) return YL_ERR_CUDA_BASE + (int)le;
     }
     return YL_OK;
 }
 
 static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
-                           const float *anchors_px, const int *anchor_mask, float conf_thre,
+                           const float *anchors_px, const int *anchor_mask, float conf_thre, const float *scale_x_y,
                            void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                            yl_stream_t stream, int stages)
 {
     if (dtype != YL_DTYPE_F32 && dtype != YL_DTYPE_F16 && dtype != YL_DTYPE_BF16) return YL_ERR_ARG;
     if (!raw || !F || !anchors_px || !anchor_mask || !ws) return YL_ERR_ARG;
     if (n_layers < 1 || n_layers > 3 || B <= 0 || C <= 0 || cap_seg <= 0) return YL_ERR_ARG;
+    // scale_x_y: NULL or every scale exactly 1 is the unscaled emit kernel (the same launches and bytes as without it)
+    ScaleXY sxy;
+    bool scaled = false;
+    for (int l = 0; l < 3; ++l) {
+        const float s = (scale_x_y && l < n_layers) ? scale_x_y[l] : 1.0f;
+        if (!scale_xy_valid(s)) return YL_ERR_ARG;
+        sxy.s[l] = s;
+        sxy.beta[l] = scale_xy_beta(s);
+        scaled |= s != 1.0f;
+    }
     if (img_first < 0 || img_count < 0 || img_first + img_count > B) return YL_ERR_ARG;
     if (C > YL_MAX_CLASSES) return YL_ERR_CLASSES;
     long m_sum = 0;
@@ -1262,10 +1311,21 @@ static int filter_raw_impl(const void *const *raw, int dtype, const int *F, int 
     const bool flag_ldg = (stages & 1) && !persistent;
     const bool pdl = pdl_enabled() && (stages & 1);                         // the emit kernel directly follows the flag kernel
     switch (dtype) {
-    case YL_DTYPE_F16: return launch_flag_emit<__half>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
-    case YL_DTYPE_BF16: return launch_flag_emit<__nv_bfloat16>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
-    default: return launch_flag_emit<float>(Pl, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
+    case YL_DTYPE_F16: return launch_flag_emit<__half>(Pl, scaled ? &sxy : nullptr, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
+    case YL_DTYPE_BF16:
+        return launch_flag_emit<__nv_bfloat16>(Pl, scaled ? &sxy : nullptr, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
+    default: return launch_flag_emit<float>(Pl, scaled ? &sxy : nullptr, tiles_ldg, img_count, flag_ldg, stages & 2, pdl, NW, st);
     }
+}
+
+extern "C" int yl_filter_raw_ex(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
+                                const float *anchors_px, const int *anchor_mask, float conf_thre, const float *scale_x_y,
+                                void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
+                                int stages, yl_stream_t stream)
+{
+    if (stages < 1 || stages > 7 || (stages & 3) == 0) return YL_ERR_ARG;
+    return filter_raw_impl(raw, dtype, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, scale_x_y, ws, ws_bytes, M, cap_seg,
+                           img_first, img_count, stream, stages);
 }
 
 extern "C" int yl_filter_raw_typed(const void *const *raw, int dtype, const int *F, int n_layers, int B, int C,
@@ -1273,9 +1333,8 @@ extern "C" int yl_filter_raw_typed(const void *const *raw, int dtype, const int 
                                    void *ws, size_t ws_bytes, long M, int cap_seg, int img_first, int img_count,
                                    int stages, yl_stream_t stream)
 {
-    if (stages < 1 || stages > 7 || (stages & 3) == 0) return YL_ERR_ARG;
-    return filter_raw_impl(raw, dtype, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, ws, ws_bytes, M, cap_seg, img_first,
-                           img_count, stream, stages);
+    return yl_filter_raw_ex(raw, dtype, F, n_layers, B, C, anchors_px, anchor_mask, conf_thre, nullptr, ws, ws_bytes, M, cap_seg,
+                            img_first, img_count, stages, stream);
 }
 
 extern "C" int yl_filter_raw(const float *const *raw, const int *F, int n_layers, int B, int C,

@@ -184,7 +184,7 @@ template <typename T, int IOU>
 __global__ void __launch_bounds__(LS_THREADS, IOU == 0 ? 0 : 1)
 k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
              double *__restrict__ loss4, int *__restrict__ tcell_all, int *__restrict__ mcell, float *__restrict__ mgrad,
-             int *__restrict__ status, float iou_norm)
+             int *__restrict__ status, float iou_norm, float sxy, float beta)
 {
     __shared__ float tb[TG_MAXK][4];
     __shared__ float tcls[TG_MAXK];
@@ -246,12 +246,14 @@ k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F,
                     const float sx = spec_sigmoidf(t0), sy = spec_sigmoidf(t1);
                     const float pw = __fmul_rn(spec_expf(t2), A.maw[a]), ph = __fmul_rn(spec_expf(t3), A.mah[a]);
                     float dl[4];
-                    const float term = iou_box_loss<IOU>(__fadd_rn(sx, (float)i), __fadd_rn(sy, (float)j), pw, ph,
+                    // scale_x_y: centre fl(fl(fl(s * sxy) + beta) + cell); sxy = 1, beta = -0 is fl(s + cell), bit for bit
+                    const float term = iou_box_loss<IOU>(__fadd_rn(__fadd_rn(__fmul_rn(sx, sxy), beta), (float)i),
+                                                         __fadd_rn(__fadd_rn(__fmul_rn(sy, sxy), beta), (float)j), pw, ph,
                                                          tb[t][0], tb[t][1], tb[t][2], tb[t][3], dl);
                     if (kk == 0) acc_xy += (double)__fmul_rn(iou_norm, term);
                     const float dn = __fmul_rn(iou_norm, kk == 0 ? dl[0] : kk == 1 ? dl[1] : kk == 2 ? dl[2] : dl[3]);
-                    const float s = kk == 0 ? sx : sy;                 // x, y: through s (1 - s); w, h: through pw, ph
-                    gout[kk] = kk < 2 ? __fmul_rn(__fmul_rn(dn, s), __fsub_rn(1.0f, s)) : __fmul_rn(dn, kk == 2 ? pw : ph);
+                    const float s = kk == 0 ? sx : sy;                 // x, y: through sxy s (1 - s); w, h: through pw, ph
+                    gout[kk] = kk < 2 ? __fmul_rn(__fmul_rn(__fmul_rn(dn, sxy), s), __fsub_rn(1.0f, s)) : __fmul_rn(dn, kk == 2 ? pw : ph);
                     continue;
                 }
             }
@@ -299,10 +301,12 @@ k_loss_match(const T *__restrict__ raw, const float *__restrict__ labels, int F,
     pdl_wait();
 }
 
-template <typename T>
+// SXY: the ignore test's predicted centre takes the grid-sensitivity decode (scale_x_y); otherwise sxy / beta are not read.
+template <typename T, bool SXY>
 __global__ void __launch_bounds__(LS_THREADS)
 k_loss_obj(const T *__restrict__ raw, const float *__restrict__ labels, int F, int K, int C, float stride, LossAnchors A,
-           float ignore_thre, const int *__restrict__ tcell_all, double *__restrict__ loss4, float *__restrict__ gobj)
+           float ignore_thre, const int *__restrict__ tcell_all, double *__restrict__ loss4, float *__restrict__ gobj, float sxy,
+           float beta)
 {
     __shared__ __align__(16) float tb[TG_MAXK][4];
     __shared__ __align__(16) float tc[TG_MAXK][4];
@@ -334,6 +338,10 @@ k_loss_obj(const T *__restrict__ raw, const float *__restrict__ labels, int F, i
             float sx, sy, ew, eh;
             spec_sigmoid2(t0, t1, sx, sy);                             // packed fp32x2 forms: the same bits as the scalar calls
             spec_exp2(t2, t3, ew, eh);
+            if constexpr (SXY) {
+                sx = __fadd_rn(__fmul_rn(sx, sxy), beta);
+                sy = __fadd_rn(__fmul_rn(sy, sxy), beta);
+            }
             const float ax = __fadd_rn(sx, (float)i), ay = __fadd_rn(sy, (float)j);
             const float aw = __fmul_rn(ew, A.maw[a]), ah = __fmul_rn(eh, A.mah[a]);
             ignored = iou_max_above(ax, ay, aw, ah, n, tb, tc, tarea, tns, sh_ns, ignore_thre);
@@ -421,7 +429,7 @@ using namespace yl;
 template <typename T>
 static int loss_forward_impl(const T *raw, const float *labels, int B, int F, int K, int C, int layer_no,
                              const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_norm,
-                             double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                             float sxy, double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                              int chained, yl_stream_t stream)
 {
     if (!raw || !labels || !anchors_px || !anchor_mask3 || !loss4 || !gobj || !tcell_all || !mcell || !mgrad) return YL_ERR_ARG;
@@ -440,33 +448,46 @@ static int loss_forward_impl(const T *raw, const float *labels, int B, int F, in
     auto match = iou_loss == YL_IOU_LOSS_GIOU ? k_loss_match<T, YL_IOU_LOSS_GIOU>
                : iou_loss == YL_IOU_LOSS_DIOU ? k_loss_match<T, YL_IOU_LOSS_DIOU>
                : iou_loss == YL_IOU_LOSS_CIOU ? k_loss_match<T, YL_IOU_LOSS_CIOU> : k_loss_match<T, YL_IOU_LOSS_NONE>;
+    const float beta = scale_xy_beta(sxy);
     YL_CUDA_TRY(launch_after(match, dim3(B, 8), dim3(LS_THREADS), 0, st, pdl && chained != 0, raw, labels, F, K, C, stride, A,
-                             loss4, tcell_all, mcell, mgrad, status, iou_norm));
+                             loss4, tcell_all, mcell, mgrad, status, iou_norm, sxy, beta));
     dim3 grid((3 * F * F + LS_THREADS - 1) / LS_THREADS, B);
-    YL_CUDA_TRY(launch_after(k_loss_obj<T>, grid, dim3(LS_THREADS), 0, st, pdl, raw, labels, F, K, C, stride, A, ignore_thre,
-                             (const int *)tcell_all, loss4, gobj));
+    // a scale of exactly 1 is the unscaled objectness kernel (the same launches and bytes as without scale_x_y)
+    YL_CUDA_TRY(launch_after(sxy != 1.0f ? k_loss_obj<T, true> : k_loss_obj<T, false>, grid, dim3(LS_THREADS), 0, st, pdl, raw,
+                             labels, F, K, C, stride, A, ignore_thre, (const int *)tcell_all, loss4, gobj, sxy, beta));
     return YL_OK;
 }
 
 static int loss_forward_typed(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
                               const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss, float iou_norm,
-                              double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
+                              float sxy, double *loss4, float *gobj, int *tcell_all, int *mcell, float *mgrad, int *status,
                               int chained, yl_stream_t stream)
 {
     if (iou_loss < YL_IOU_LOSS_NONE || iou_loss > YL_IOU_LOSS_CIOU || !(iou_norm >= 0.0f) || isinf(iou_norm)) return YL_ERR_ARG;
+    // scale_x_y moves the predicted centre of the IoU box term; the BCE xy term has no scaled counterpart
+    if (!scale_xy_valid(sxy) || (sxy != 1.0f && iou_loss == YL_IOU_LOSS_NONE)) return YL_ERR_ARG;
     switch (dtype) {
     case YL_DTYPE_F32:
         return loss_forward_impl((const float *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
-                                 iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+                                 iou_norm, sxy, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     case YL_DTYPE_F16:
         return loss_forward_impl((const __half *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
-                                 iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+                                 iou_norm, sxy, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     case YL_DTYPE_BF16:
         return loss_forward_impl((const __nv_bfloat16 *)raw, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre,
-                                 iou_loss, iou_norm, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+                                 iou_loss, iou_norm, sxy, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
     default:
         return YL_ERR_ARG;
     }
+}
+
+extern "C" int yl_loss_forward_ex2(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
+                                   const float *anchors_px, const int *anchor_mask3, float ignore_thre, int iou_loss,
+                                   float iou_normalizer, float scale_x_y, int chained, double *loss4, float *gobj, int *tcell_all,
+                                   int *mcell, float *mgrad, int *status, yl_stream_t stream)
+{
+    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
+                              iou_normalizer, scale_x_y, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
 }
 
 extern "C" int yl_loss_forward_ex(const void *raw, int dtype, const float *labels, int B, int F, int K, int C, int layer_no,
@@ -474,8 +495,8 @@ extern "C" int yl_loss_forward_ex(const void *raw, int dtype, const float *label
                                   float iou_normalizer, int chained, double *loss4, float *gobj, int *tcell_all, int *mcell,
                                   float *mgrad, int *status, yl_stream_t stream)
 {
-    return loss_forward_typed(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
-                              iou_normalizer, loss4, gobj, tcell_all, mcell, mgrad, status, chained, stream);
+    return yl_loss_forward_ex2(raw, dtype, labels, B, F, K, C, layer_no, anchors_px, anchor_mask3, ignore_thre, iou_loss,
+                               iou_normalizer, 1.0f, chained, loss4, gobj, tcell_all, mcell, mgrad, status, stream);
 }
 
 extern "C" int yl_loss_forward(const float *raw, const float *labels, int B, int F, int K, int C, int layer_no,

@@ -95,6 +95,32 @@ def _check_diou(diou):
     return diou
 
 
+def _scale_value(v):
+    """One scale_x_y value as the fp32 the kernels use: a real number, finite and > 0 in fp32."""
+    if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)):
+        raise TypeError("scale_x_y values must be real numbers, got %r" % (v,))
+    with np.errstate(over="ignore"):
+        f = np.float32(v)
+    if not np.isfinite(f) or not f > 0:
+        raise ValueError("scale_x_y values must be finite and > 0 (in float32), got %r" % (v,))
+    return float(f)
+
+
+def _check_scale_x_y(scale_x_y, n_heads):
+    """scale_x_y for n_heads head tensors: None, one real number for every head, or a sequence of one real number per head in
+    head order.  Returns None when every scale is 1 (the unscaled decode, bit for bit) and otherwise a list of n_heads fp32
+    values.  Raises TypeError / ValueError before any CUDA work."""
+    if scale_x_y is None:
+        return None
+    if isinstance(scale_x_y, (str, bytes)) or not hasattr(scale_x_y, "__len__"):
+        vals = [_scale_value(scale_x_y)] * n_heads
+    else:
+        vals = [_scale_value(v) for v in scale_x_y]
+        if len(vals) != n_heads:
+            raise ValueError("scale_x_y needs one value per head tensor (%d), got %d" % (n_heads, len(vals)))
+    return None if all(v == 1.0 for v in vals) else vals
+
+
 def _round4(n):
     return (n + 3) // 4 * 4
 
@@ -209,7 +235,7 @@ def _check_raws(head_outputs, num_classes):
 
 
 def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None,
-               agnostic=False, diou=False):
+               agnostic=False, diou=False, scale_x_y=None):
     """Fused YOLOLayer eval decode (yololayer.py:88-166) + postprocess (utils.py:92-223).
 
     head_outputs: the three raw head conv outputs [B, 3*(5+C), F_l, F_l] (stride 8, 16, 32; yolov4.py:235-251).
@@ -239,10 +265,19 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     one fp32 rounding, max / min propagating NaN.  A NaN penalty keeps the pair apart, and pen >= 0, so DIoU never suppresses
     a pair IoU keeps apart: boxes far apart that overlap enough for IoU survive as separate detections.  darknet's diounms
     compares with > and an exponent beta_nms; this is the paper's >= with no exponent.  Default False: IoU.
+
+    scale_x_y: YOLOv4's grid-sensitivity decode (darknet's scale_x_y; yolov4.cfg sets 1.2, 1.1, 1.05 for the stride 8, 16,
+    32 heads).  With s the head's scale and beta = fl32(-0.5 * (s - 1)) (evaluated in float64), a box centre of cell i is
+    fl(fl(fl(sigmoid(tx) * s) + beta) + i) grid units before the stride, every operation one fp32 rounding; nothing is
+    clamped.  One real number applies to every head, a sequence gives one value per head tensor in head order.  Only the boxes
+    change: the scores, and so which pairs pass conf_thre, do not depend on the scale.  None (the default), 1.0 or all ones is
+    the plain decode, bit for bit.  A bool or non-real raises TypeError; a non-finite or non-positive value or a wrong length
+    raises ValueError, before any CUDA work.
     """
     max_det = _check_max_det(max_det)
     agnostic = _check_agnostic(agnostic)
     diou = _check_diou(diou)
+    sxy = _check_scale_x_y(scale_x_y, len(head_outputs))
     raws, B, Fs, dt = _check_raws(head_outputs, num_classes)
     C = int(num_classes)
     M = sum(3 * f * f for f in Fs)
@@ -252,10 +287,11 @@ def detect_raw(head_outputs, num_classes, conf_thre=0.7, nms_thre=0.45, anchors=
     mask = _cabi.ints([v for m in anchor_mask for v in m])
     rp = _cabi.ptrs([r.data_ptr() for r in raws])
     fs = _cabi.ints(Fs)
+    sp = None if sxy is None else _cabi.floats(sxy)
     with torch.cuda.device(dev):
         def front(ws, cap_seg):
-            _cabi.check(L.yl_filter_raw_typed(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), ws.ptr(), ws.nbytes,
-                                              M, cap_seg, 0, B, 3, _stream()))
+            _cabi.check(L.yl_filter_raw_ex(rp, dt, fs, len(raws), B, C, anch, mask, _f32(conf_thre), sp, ws.ptr(), ws.nbytes,
+                                           M, cap_seg, 0, B, 3, _stream()))
         rows, mh = _run(front, dev, B, M, C, nms_thre, max_det, agnostic, diou)
     return _split(rows, mh, B, dev, torch.float32)
 
@@ -274,14 +310,18 @@ class HeadPostprocessor:
     of 4, so the output (and a DetectionExchange built with hp.cap_out) is sized by the cap.  uncapped is a device int32 [B]
     with every image's uncapped count, refreshed by every run and replay: meta[b] < uncapped[b] means image b was capped.
     Without a cap uncapped is the view meta[:B].  agnostic selects class-agnostic NMS as in detect_raw (uncapped then counts
-    the agnostic rows), and diou DIoU-NMS as in detect_raw.
+    the agnostic rows), and diou DIoU-NMS as in detect_raw.  scale_x_y (one number, or one per grid size) is the
+    grid-sensitivity decode of detect_raw, fixed at construction for run / capture / replay.
     """
 
     def __init__(self, batch, grid_sizes, num_classes, conf_thre, nms_thre, device=None, cap_seg=_DEFAULT_CAP_SEG,
-                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None, agnostic=False, diou=False):
+                 cap_out=None, n_groups=1, anchors=ANCHORS_PX, anchor_mask=ANCHOR_MASK, max_det=None, agnostic=False, diou=False,
+                 scale_x_y=None):
         self.max_det = _check_max_det(max_det)
         self.agnostic = _check_agnostic(agnostic)
         self.diou = _check_diou(diou)
+        self.scale_x_y = _check_scale_x_y(scale_x_y, len(grid_sizes))
+        self._sxy = None if self.scale_x_y is None else _cabi.floats(self.scale_x_y)
         if cap_out is None:
             cap_out = _DEFAULT_CAP_OUT if self.max_det is None else _round4(self.max_det)
         if self.max_det is not None and self.max_det > int(cap_out):
@@ -320,9 +360,9 @@ class HeadPostprocessor:
             _cabi.check(L.yl_post_reset(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, main.cuda_stream))
         for g in range(G):
             i0, i1 = B * g // G, B * (g + 1) // G
-            _cabi.check(L.yl_filter_raw_typed(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf,
-                                              self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7 if fold_reset else 3,
-                                              main.cuda_stream))
+            _cabi.check(L.yl_filter_raw_ex(rp, dt, self.fs, len(self.Fs), B, C, self.anch, self.mask, self.conf, self._sxy,
+                                           self.ws.ptr(), self.ws.nbytes, M, self.cap_seg, i0, i1 - i0, 7 if fold_reset else 3,
+                                           main.cuda_stream))
             self.side.wait_stream(main)
             _cabi.check(L.yl_nms_ex2(self.ws.ptr(), self.ws.nbytes, B, M, C, self.cap_seg, self.nms, self.max_det or 0,
                                      int(self.agnostic), int(self.diou), self.rows.data_ptr(), self.cap_out, self.meta.data_ptr(),

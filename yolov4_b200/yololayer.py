@@ -11,6 +11,7 @@ import torch
 from torch import nn
 
 from . import _cabi
+from .postprocess import _check_scale_x_y, _scale_value
 
 
 def _stream():
@@ -55,8 +56,14 @@ class _DecodeTrain(torch.autograd.Function):
 class YOLOLayer(nn.Module):
     strides = [8, 16, 32]
 
-    def __init__(self, cfg, layer_no, device=None):
+    def __init__(self, cfg, layer_no, device=None, *, scale_x_y=None):
+        """scale_x_y (keyword only, not part of the reference signature): YOLOv4's grid-sensitivity decode of this head, one
+        real number s (darknet's scale_x_y).  The eval output's centres become fl(fl(fl(fl(sigmoid(t) * s) + beta) + cell)
+        * stride), beta = fl32(-0.5 * (s - 1)); None or 1 is the reference's decode, bit for bit.  The train branch feeds the
+        reference's BCE loss, which has no scaled form: in training mode a scale other than 1 raises ValueError (train with
+        fused_yolo_loss(..., iou_loss=..., scale_x_y=...)).  A plain attribute, so the state_dict stays empty."""
         super().__init__()
+        self.scale_x_y = 1.0 if scale_x_y is None else _scale_value(scale_x_y)
         self.stride = self.strides[layer_no]
         self.layer_no = layer_no
         self.anchors = cfg['ANCHORS']
@@ -80,6 +87,9 @@ class YOLOLayer(nn.Module):
         B, _, F, _ = output.shape
         n_ch = 5 + self.n_classes
         if self.training:
+            if self.scale_x_y != 1.0:
+                raise ValueError("YOLOLayer with scale_x_y=%r has no train branch (the reference's BCE xy loss has no scaled "
+                                 "form): train with fused_yolo_loss(..., iou_loss=..., scale_x_y=...)" % (self.scale_x_y,))
             out_planar, pred_planar = _DecodeTrain.apply(output, self._anch, self.n_classes)
             return dict({
                 'layer_no': self.layer_no,
@@ -89,14 +99,17 @@ class YOLOLayer(nn.Module):
         raw = output.detach().contiguous()
         res = torch.empty((B, self.n_anchors * F * F, n_ch), dtype=raw.dtype, device=raw.device)
         with torch.cuda.device(raw.device):
-            _cabi.check(_cabi.lib().yl_decode_dense(raw.data_ptr(), B, F, self.n_classes, self._anch, float(self.stride),
-                                                    res.data_ptr(), self.n_anchors * F * F, 0, _stream()))
+            _cabi.check(_cabi.lib().yl_decode_dense_ex(raw.data_ptr(), B, F, self.n_classes, self._anch, float(self.stride),
+                                                       self.scale_x_y, res.data_ptr(), self.n_anchors * F * F, 0, _stream()))
         return res
 
 
-def decode_dense_cat(head_outputs, cfg):
+def decode_dense_cat(head_outputs, cfg, *, scale_x_y=None):
     """The three eval-mode YOLOLayer outputs written straight into one [B, sum 3F^2, 5+C] tensor: the value of
-    `torch.cat((x1, x2, x3), 1)` at yolov4.py:324 without the three intermediate tensors and the cat copy."""
+    `torch.cat((x1, x2, x3), 1)` at yolov4.py:324 without the three intermediate tensors and the cat copy.
+    scale_x_y: None, one real number or one per head tensor in head order, the grid-sensitivity decode of
+    YOLOLayer(..., scale_x_y=s) (detect_raw states it); checked before any CUDA work."""
+    sxy = _check_scale_x_y(scale_x_y, len(head_outputs)) or [1.0] * len(head_outputs)
     C = int(cfg['N_CLASSES'])
     B = int(head_outputs[0].shape[0])
     Fs = [int(r.shape[2]) for r in head_outputs]
@@ -111,6 +124,7 @@ def decode_dense_cat(head_outputs, cfg):
             s = YOLOLayer.strides[l]
             anch = _cabi.floats([v / s for i in cfg['ANCHOR_MASK'][l] for v in cfg['ANCHORS'][i]])
             raw = r.detach().contiguous()
-            _cabi.check(_cabi.lib().yl_decode_dense(raw.data_ptr(), B, Fs[l], C, anch, float(s), out.data_ptr(), M, off, _stream()))
+            _cabi.check(_cabi.lib().yl_decode_dense_ex(raw.data_ptr(), B, Fs[l], C, anch, float(s), sxy[l], out.data_ptr(), M, off,
+                                                       _stream()))
             off += 3 * Fs[l] * Fs[l]
     return out

@@ -14,6 +14,7 @@ import torch
 from torch import nn
 
 from . import _cabi
+from .postprocess import _check_scale_x_y
 
 
 def _stream():
@@ -203,12 +204,21 @@ def _iou_args(iou_loss, iou_normalizer):
     return _IOU_LOSS_CODES[iou_loss], float(np.float32(norm))
 
 
+def _scale_args(scale_x_y, n_heads, iou_code):
+    """One fp32 scale_x_y per head tensor (all 1.0 without scales); raises before any CUDA work."""
+    sxy = _check_scale_x_y(scale_x_y, n_heads)
+    if sxy is not None and iou_code == 0:
+        raise ValueError("scale_x_y moves the predicted centre of the IoU box term: it needs iou_loss='giou', 'diou' or 'ciou' "
+                         "(the BCE xy term has no scaled form)")
+    return sxy or [1.0] * n_heads
+
+
 class _FusedYoloLoss(torch.autograd.Function):
     """N2: raw head tensors + padded labels -> the reference's YOLOLoss.forward value, gradient straight to the raw tensors
     (in the heads' dtype: fp32, fp16 or bf16)."""
 
     @staticmethod
-    def forward(ctx, labels, anchors, anchor_mask, ignore_thresh, n_classes, iou_code, iou_norm, *raws):
+    def forward(ctx, labels, anchors, anchor_mask, ignore_thresh, n_classes, iou_code, iou_norm, sxy, *raws):
         L = _cabi.lib()
         C = int(n_classes)
         dtype = _head_dtype_code(raws)
@@ -237,10 +247,10 @@ class _FusedYoloLoss(torch.autograd.Function):
             # every foreign kernel (contiguous copies, the fills of loss4 / status) is enqueued by now: the calls below are back
             # to back on the stream, so the second and later ones may be launched programmatically behind their predecessor
             for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):
-                _cabi.check(L.yl_loss_forward_ex(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
-                                                 _cabi.ints(anchor_mask[l]), float(np.float32(ignore_thresh)), iou_code,
-                                                 iou_norm, int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
-                                                 mcell.data_ptr(), mgrad.data_ptr(), status.data_ptr(), _stream()))
+                _cabi.check(L.yl_loss_forward_ex2(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
+                                                  _cabi.ints(anchor_mask[l]), float(np.float32(ignore_thresh)), iou_code,
+                                                  iou_norm, sxy[i], int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
+                                                  mcell.data_ptr(), mgrad.data_ptr(), status.data_ptr(), _stream()))
         ctx.save_for_backward(*saved)
         ctx.shapes = [tuple(r.shape) for r in raws]
         ctx.dtype, ctx.dtype_code = raws[0].dtype, dtype
@@ -263,10 +273,10 @@ class _FusedYoloLoss(torch.autograd.Function):
                 _cabi.check(L.yl_loss_backward_typed(gobj.data_ptr(), mcell.data_ptr(), mgrad.data_ptr(), up.data_ptr(), B, F, ctx.K,
                                                      ctx.C, g.data_ptr(), ctx.dtype_code, _stream()))
                 grads.append(g)
-        return (None, None, None, None, None, None, None) + tuple(grads)
+        return (None, None, None, None, None, None, None, None) + tuple(grads)
 
 
-def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7, iou_loss=None, iou_normalizer=1.0):
+def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7, iou_loss=None, iou_normalizer=1.0, scale_x_y=None):
     """N2 (SURVEY.md 8f): the value of `YOLOLoss(cfg, ignore_thresh)([YOLOLayer_l.train()(x_l)], {'padded_labels': labels})`
     (yolo/model/yololoss.py:373-443 on top of yololayer.py:122-145) computed from the three raw head tensors without
     materialising output / pred / target / masks; differentiable with respect to the head tensors.
@@ -283,20 +293,31 @@ def fused_yolo_loss(head_outputs, padded_labels, cfg, ignore_thresh=0.7, iou_los
     of every matched cell by iou_normalizer * torchvision's generalized_ / distance_ / complete_box_iou_loss (eps 1e-7) of the
     train-mode predicted box and the cell's last GT, in grid units, without tgt_scale weighting; objectness and class terms
     are unchanged (DESIGN.md section 1).  iou_normalizer (a finite real >= 0) weights the box term only; with iou_loss=None
-    it must stay 1.  A bad keyword raises ValueError (TypeError for a bool normalizer) before any CUDA work."""
+    it must stay 1.  A bad keyword raises ValueError (TypeError for a bool normalizer) before any CUDA work.
+
+    scale_x_y (YOLOv4's grid-sensitivity decode, darknet's scale_x_y; yolov4.cfg pairs 1.2 / 1.1 / 1.05 with iou_loss='ciou'):
+    None, one real number for every head, or one per head tensor in head order.  The train-mode predicted box of the IoU box
+    term and of the ignore test takes the centre fl(fl(fl(sigmoid(t) * s) + beta) + cell), beta = fl32(-0.5 * (s - 1)), and
+    d centre / d t = s * sigmoid * (1 - sigmoid); w / h, objectness and class terms are unchanged.  None or all ones is the
+    loss without it, bit for bit.  A scale other than 1 needs an IoU box term (iou_loss=None raises ValueError: the BCE xy
+    term has no scaled form); a bool or non-real raises TypeError, a non-finite or non-positive value or a wrong length
+    ValueError, before any CUDA work."""
     iou_code, iou_norm = _iou_args(iou_loss, iou_normalizer)
+    sxy = _scale_args(scale_x_y, len(head_outputs), iou_code)
     return _FusedYoloLoss.apply(padded_labels, cfg['ANCHORS'], cfg['ANCHOR_MASK'], ignore_thresh, cfg['N_CLASSES'], iou_code,
-                                iou_norm, *head_outputs)
+                                iou_norm, sxy, *head_outputs)
 
 
 def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0.7, layers=None, iou_loss=None,
-                               iou_normalizer=1.0):
+                               iou_normalizer=1.0, scale_x_y=None):
     """The four sums (loss_xy, loss_wh, loss_obj, loss_cls; yololoss.py:421-427) over the given layers as a float64[4] device
     tensor, no autograd.  `layers[i]` is the layer number of head_outputs[i] (default 0, 1, 2).  The heads may be float32,
     float16 or bfloat16 CUDA tensors of one dtype: a 16-bit head gives the components of its widened fp32 copy (up to the order
     of the fp64 sums); mixed dtypes, float64 and CPU heads raise TypeError before any CUDA work.  iou_loss / iou_normalizer as
-    for fused_yolo_loss: with an IoU box term, component 0 is that term and component 1 is 0."""
+    for fused_yolo_loss: with an IoU box term, component 0 is that term and component 1 is 0.  scale_x_y as for
+    fused_yolo_loss, one value per head tensor (not per layer number)."""
     iou_code, iou_norm = _iou_args(iou_loss, iou_normalizer)
+    sxy = _scale_args(scale_x_y, len(head_outputs), iou_code)
     L = _cabi.lib()
     dtype = _head_dtype_code(head_outputs)
     dev = head_outputs[0].device
@@ -319,8 +340,8 @@ def fused_yolo_loss_components(head_outputs, padded_labels, cfg, ignore_thresh=0
             calls.append((rc, F, int(l), gobj, tcell, mcell, mgrad))
             keep += [rc, gobj, tcell, mcell, mgrad]
         for i, (rc, F, l, gobj, tcell, mcell, mgrad) in enumerate(calls):     # back to back: see _FusedYoloLoss.forward
-            _cabi.check(L.yl_loss_forward_ex(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
-                                             _cabi.ints(cfg['ANCHOR_MASK'][l]), float(np.float32(ignore_thresh)), iou_code,
-                                             iou_norm, int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
-                                             mcell.data_ptr(), mgrad.data_ptr(), None, _stream()))
+            _cabi.check(L.yl_loss_forward_ex2(rc.data_ptr(), dtype, lab.data_ptr(), B, F, K, C, l, anch,
+                                              _cabi.ints(cfg['ANCHOR_MASK'][l]), float(np.float32(ignore_thresh)), iou_code,
+                                              iou_norm, sxy[i], int(i > 0), loss4.data_ptr(), gobj.data_ptr(), tcell.data_ptr(),
+                                              mcell.data_ptr(), mgrad.data_ptr(), None, _stream()))
     return loss4
