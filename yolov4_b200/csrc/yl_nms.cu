@@ -112,9 +112,9 @@ __device__ __forceinline__ void store_row(float *o, const float4 &box, unsigned 
 
 // ---------------------------------------------------------------------------------------------------------------
 // Small tier (the common case: ~150 candidates per (image,class) at conf 1e-4).  Everything in ~21 KB of shared memory.
-//   1. rank sort on the 32-bit score key (LDS.128 per four keys, one compare + predicated add per key); if two records
-//      tie on the score the ranks collide, which is detected, and the segment is ranked again on the unique 64-bit key
-//      (score, row);
+//   1. rank by bucket sort: the 32-bit score keys are spread over RB buckets by their offset from the segment's smallest
+//      key (monotone, so a bucket's records come after every record of lower buckets); a record's rank is its bucket's
+//      first position plus the number of smaller unique 64-bit keys (score desc, row desc) in its own bucket;
 //   2. candidate pairs by table lookup instead of an all-pairs loop: boxes are binned on x1, x2, y1, y2 (NBIN bins over
 //      the segment's coordinate range) and on log2(area) (4 bins per octave); six prefix tables hold, per bin, the set
 //      (bitmask over sorted positions) of boxes that CANNOT overlap / reach the IoU threshold with a box of that bin:
@@ -147,17 +147,49 @@ constexpr int QCAP_W = YL_NMS_QCAP;                     // queued pairs per warp
 #ifndef YL_NMS_MINB
 #define YL_NMS_MINB 10
 #endif
-#ifndef YL_NMS_SPLIT_RANK
-#define YL_NMS_SPLIT_RANK 1
-#endif
+constexpr int RB_LOG2 = 7, RB = 1 << RB_LOG2;           // rank buckets
 constexpr int AREA_BIN_OFF = (127 + 4) << 2;            // float bits >> 21 of 16.0f: areas below 16 px^2 share bin 0
+
+// Phase probe (tools/nms_phase_probe.py; never defined in the library build).  YL_NMS_PROBE: thread 0 of every CTA adds the
+// clock64() cycles of each phase (closed by a barrier) to yl_nms_probe_acc[phase] and counts segments, queued
+// pairs, rows with a suppressor and kept rows in the slots after the phases.  YL_NMS_PROBE_STOP=k: the CTA returns after phase
+// k (the results are then wrong; only the kernel's time means something).
+#if defined(YL_NMS_PROBE) || defined(YL_NMS_PROBE_STOP)
+__device__ unsigned long long yl_nms_probe_acc[16];
+extern "C" int yl_nms_probe_read(unsigned long long *host, int reset)
+{
+    cudaError_t e = cudaMemcpyFromSymbol(host, yl_nms_probe_acc, sizeof(yl_nms_probe_acc));
+    if (e == cudaSuccess && reset) {
+        static const unsigned long long zero[16] = {};
+        e = cudaMemcpyToSymbol(yl_nms_probe_acc, zero, sizeof(zero));
+    }
+    return (int)e;
+}
+#endif
+#ifdef YL_NMS_PROBE
+#define NMS_PHASE(k)                                                                                                    \
+    do {                                                                                                               \
+        __syncthreads();                                                                                               \
+        if (threadIdx.x == 0) {                                                                                        \
+            const long long t_ = clock64();                                                                            \
+            atomicAdd(&yl_nms_probe_acc[k], (unsigned long long)(t_ - probe_t));                                       \
+            probe_t = t_;                                                                                              \
+        }                                                                                                              \
+    } while (0)
+#define NMS_COUNT(k, v) do { if (threadIdx.x == 0) atomicAdd(&yl_nms_probe_acc[k], (unsigned long long)(v)); } while (0)
+#elif defined(YL_NMS_PROBE_STOP)
+#define NMS_PHASE(k) do { if ((k) == YL_NMS_PROBE_STOP) return; } while (0)
+#define NMS_COUNT(k, v) do {} while (0)
+#else
+#define NMS_PHASE(k) do {} while (0)
+#define NMS_COUNT(k, v) do {} while (0)
+#endif
 
 struct alignas(16) BinsSmem {
     union {
         struct {
-            unsigned key[SMALL_R + 4];                  // score key per record (record order), padded for the 4-wide loop
-            unsigned pad_[4];
-            unsigned long long k64[SMALL_R + 2];        // tie fallback: (score key, ~row)
+            unsigned long long key[SMALL_R];            // (score key, ~row), grouped by bucket
+            unsigned base[RB + 1];                      // records per bucket, then the bucket's first position
         } s;
         unsigned short queue[SMALL_WARPS][QCAP_W];      // (j << 8) | i candidate pairs, one queue per warp
     } a;
@@ -169,43 +201,11 @@ struct alignas(16) BinsSmem {
         unsigned T[SMALL_R][SMALL_W];                   // transposed suppression matrix
         float stage[SMALL_R * 7];                       // finished rows
     } b;
-    unsigned char owner[SMALL_R];
     float red[2][SMALL_WARPS];
+    unsigned kred[2][SMALL_WARPS];
     unsigned qn[SMALL_WARPS];
     unsigned dirty[SMALL_W], keptw[SMALL_W], pref[SMALL_W + 1];
 };
-
-// Number of keys below `key`; keys beyond n are padded with 0xFFFFFFFF up to a multiple of four.
-__device__ __forceinline__ int rank32(const unsigned *sh_key, int n, unsigned key)
-{
-    int r0 = 0, r1 = 0, r2 = 0, r3 = 0;                        // four independent counters: no serial chain through the adds
-    const uint4 *k4 = reinterpret_cast<const uint4 *>(sh_key);
-    const int n4 = (n + 3) >> 2;
-#pragma unroll 4
-    for (int j = 0; j < n4; ++j) {
-        const uint4 k = k4[j];
-        asm("{\n\t.reg .pred p, q, r, s;\n\t"
-            "setp.lt.u32 p, %4, %8;\n\tsetp.lt.u32 q, %5, %8;\n\tsetp.lt.u32 r, %6, %8;\n\tsetp.lt.u32 s, %7, %8;\n\t"
-            "@p add.s32 %0, %0, 1;\n\t@q add.s32 %1, %1, 1;\n\t@r add.s32 %2, %2, 1;\n\t@s add.s32 %3, %3, 1;\n\t}"
-            : "+r"(r0), "+r"(r1), "+r"(r2), "+r"(r3) : "r"(k.x), "r"(k.y), "r"(k.z), "r"(k.w), "r"(key));
-    }
-    return (r0 + r1) + (r2 + r3);
-}
-
-// Number of keys below `key` (keys are unique): LDS.128 per two keys, one 64-bit compare + predicated add per key.
-__device__ __forceinline__ int rank_of(const unsigned long long *sh_key, int n, unsigned long long key)
-{
-    int r = 0;
-    const ulonglong2 *k2 = reinterpret_cast<const ulonglong2 *>(sh_key);
-    const int n2 = (n + 1) >> 1;
-#pragma unroll 4
-    for (int j = 0; j < n2; ++j) {
-        const ulonglong2 k = k2[j];
-        asm("{\n\t.reg .pred p, q;\n\tsetp.lt.u64 p, %1, %3;\n\tsetp.lt.u64 q, %2, %3;\n\t@p add.s32 %0, %0, 1;\n\t@q add.s32 %0, %0, 1;\n\t}"
-            : "+r"(r) : "l"(k.x), "l"(k.y), "l"(key));
-    }
-    return r;
-}
 
 __device__ __forceinline__ int coord_bin(float v, float lo, float scale)
 {
@@ -224,6 +224,9 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
     __shared__ BinsSmem S;
     const unsigned FULL = 0xFFFFFFFFu;
     const int seg = seg_first + blockIdx.x;
+#ifdef YL_NMS_PROBE
+    long long probe_t = clock64();
+#endif
     pdl_trigger();
     {
         // zero the exclusion tables: independent of the input, so a CTA launched early (PDL) does it while the filter
@@ -231,6 +234,7 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         uint4 *z = reinterpret_cast<uint4 *>(&S.b.tab[0][0][0]);
         constexpr int NZ = (int)(sizeof(S.b.tab) / sizeof(uint4));
         for (int i = threadIdx.x; i < NZ; i += SMALL_THREADS) z[i] = make_uint4(0u, 0u, 0u, 0u);
+        for (int i = threadIdx.x; i < RB; i += SMALL_THREADS) S.a.s.base[i] = 0u;
         if (threadIdx.x < SMALL_WARPS) S.qn[threadIdx.x] = 0u;
         if (threadIdx.x < SMALL_W) S.dirty[threadIdx.x] = 0u;
     }
@@ -246,6 +250,9 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
     const int n = (int)cnt;
     const int nw = (n + 31) >> 5, nwp = (nw + 1) >> 1;
     uint4 *rec = cand + (size_t)seg * cap_seg * 2;
+    NMS_PHASE(0);
+    NMS_COUNT(9, 1);
+    NMS_COUNT(12, n);
 
     // ---- 1. records -> registers; score keys -> shared memory; coordinate range of the segment ----
     uint4 ra[SMALL_EPT];
@@ -257,92 +264,88 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         rb[u] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (e < n) { ra[u] = rec[2 * e]; rb[u] = as_float4(rec[2 * e + 1]); }
     }
-    unsigned key[SMALL_EPT];
+    unsigned long long key[SMALL_EPT];
     bool valid[SMALL_EPT];
     float lo = kInf, hi = -kInf;
+    unsigned kmin = 0xFFFFFFFFu, kmax = 0u;
 #pragma unroll
     for (int u = 0; u < SMALL_EPT; ++u) {
         const int e = tid + u * SMALL_THREADS;
-        key[u] = 0xFFFFFFFFu;
+        key[u] = ~0ull;
         valid[u] = false;
         if (e < n) {
-            key[u] = score_desc_bits(ra[u].x);
-            S.a.s.key[e] = key[u];
+            const unsigned k32 = score_desc_bits(ra[u].x);
+            key[u] = ((unsigned long long)k32 << 32) | (unsigned)(~ra[u].y);
+            kmin = min(kmin, k32);
+            kmax = max(kmax, k32);
             // only boxes with positive extents (hence no NaN) can overlap anything (suppresses_pos: tl < br on both axes)
             valid[u] = rb[u].x < rb[u].z && rb[u].y < rb[u].w;
             if (valid[u]) { lo = fminf(lo, fminf(rb[u].x, rb[u].y)); hi = fmaxf(hi, fmaxf(rb[u].z, rb[u].w)); }
         }
     }
-    if (tid < 4) S.a.s.key[n + tid] = 0xFFFFFFFFu;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         lo = fminf(lo, __shfl_xor_sync(FULL, lo, o));
         hi = fmaxf(hi, __shfl_xor_sync(FULL, hi, o));
     }
-    if (lane == 0) { S.red[0][warp] = lo; S.red[1][warp] = hi; }
+    kmin = __reduce_min_sync(FULL, kmin);
+    kmax = __reduce_max_sync(FULL, kmax);
+    if (lane == 0) { S.red[0][warp] = lo; S.red[1][warp] = hi; S.kred[0][warp] = kmin; S.kred[1][warp] = kmax; }
     __syncthreads();
+    NMS_PHASE(1);
 
-    // ---- 2. rank ----
-    const int wbase = tid & ~31;                                // warp-uniform bounds below
-    int rank[SMALL_EPT];
-#pragma unroll
-    for (int u = 0; u < SMALL_EPT; ++u) rank[u] = 0;
-    if (wbase < n) rank[0] = rank32(S.a.s.key, n, key[0]);
-#if YL_NMS_SPLIT_RANK
-    static_assert(SMALL_EPT == 2, "the split second pass assumes two records per thread");
-    if (n > SMALL_THREADS) {                                    // CTA-uniform
-        // Records SMALL_THREADS.. (a few dozen in the typical segment of ~144) would all sit in warp 0 and make it walk
-        // every key a second time while the other warps wait at the barrier.  Instead every warp ranks them against its own
-        // quarter of the keys and the partial counts are added up in shared memory.
-        const int x = n - SMALL_THREADS;
-        S.bins[tid] = 0u;                                       // S.bins is free until the sorted arrays are built
-        __syncthreads();
-        const int n4 = (n + 3) >> 2;
-        const int g0 = (n4 * warp) / SMALL_WARPS, g1 = (n4 * (warp + 1)) / SMALL_WARPS;
-        for (int c = 0; 32 * c < x; ++c) {
-            const int i = 32 * c + lane;
-            if (i < x) {
-                const int part = rank32(S.a.s.key + 4 * g0, 4 * (g1 - g0), S.a.s.key[SMALL_THREADS + i]);
-                atomicAdd(&S.bins[i], (unsigned)part);
-            }
-        }
-        __syncthreads();
-        if (tid < x) rank[1] = (int)S.bins[tid];
-    }
-#else
-#pragma unroll
-    for (int u = 1; u < SMALL_EPT; ++u)
-        if (wbase + u * SMALL_THREADS < n) rank[u] = rank32(S.a.s.key, n, key[u]);
-#endif
-#pragma unroll
-    for (int u = 0; u < SMALL_EPT; ++u) {
-        const int e = tid + u * SMALL_THREADS;
-        if (e < n) S.owner[rank[u]] = (unsigned char)e;
-    }
-    __syncthreads();
+    // ---- 2. rank: bucket = (score key - smallest key) >> sh, sh such that every key of the segment has a bucket below RB ----
+    int bk[SMALL_EPT], rank[SMALL_EPT];
     {
-        bool coll = false;
+#pragma unroll
+        for (int wq = 1; wq < SMALL_WARPS; ++wq) { kmin = min(kmin, S.kred[0][wq]); kmax = max(kmax, S.kred[1][wq]); }
+        kmin = min(kmin, S.kred[0][0]);                         // kmin / kmax already hold this thread's own warp
+        kmax = max(kmax, S.kred[1][0]);
+        const int sh = max(0, (32 - __clz((int)(kmax - kmin))) - RB_LOG2);
 #pragma unroll
         for (int u = 0; u < SMALL_EPT; ++u) {
-            const int e = tid + u * SMALL_THREADS;
-            if (e < n) coll |= (S.owner[rank[u]] != (unsigned char)e);
-        }
-        if (__syncthreads_or(coll)) {
-            // equal scores inside the segment: the order is (score desc, row desc), decided on the unique 64-bit key
-            unsigned long long k64[SMALL_EPT];
-#pragma unroll
-            for (int u = 0; u < SMALL_EPT; ++u) {
-                const int e = tid + u * SMALL_THREADS;
-                k64[u] = ~0ull;
-                if (e < n) { k64[u] = ((unsigned long long)key[u] << 32) | (unsigned)(~ra[u].y); S.a.s.k64[e] = k64[u]; }
+            bk[u] = 0;
+            rank[u] = 0;
+            if (tid + u * SMALL_THREADS < n) {
+                bk[u] = (int)(((unsigned)(key[u] >> 32) - kmin) >> sh);
+                rank[u] = (int)atomicAdd(&S.a.s.base[bk[u]], 1u);     // position inside the bucket, for the scatter
             }
-            if (tid == 0 && (n & 1)) S.a.s.k64[n] = ~0ull;
-            __syncthreads();
-#pragma unroll
-            for (int u = 0; u < SMALL_EPT; ++u)
-                if (wbase + u * SMALL_THREADS < n) rank[u] = rank_of(S.a.s.k64, n, k64[u]);
         }
     }
+    __syncthreads();
+    if (warp == 0) {
+        // exclusive prefix of the bucket counts, RB / 32 buckets per lane
+        constexpr int BL = RB / 32;
+        unsigned c[BL], sum = 0u;
+#pragma unroll
+        for (int k = 0; k < BL; ++k) { c[k] = S.a.s.base[BL * lane + k]; sum += c[k]; }
+        unsigned incl = sum;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned v = __shfl_up_sync(FULL, incl, o);
+            if (lane >= o) incl += v;
+        }
+        unsigned run = incl - sum;
+#pragma unroll
+        for (int k = 0; k < BL; ++k) { S.a.s.base[BL * lane + k] = run; run += c[k]; }
+        if (lane == 31) S.a.s.base[RB] = incl;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < SMALL_EPT; ++u)
+        if (tid + u * SMALL_THREADS < n) S.a.s.key[S.a.s.base[bk[u]] + rank[u]] = key[u];
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < SMALL_EPT; ++u) {
+        if (tid + u * SMALL_THREADS < n) {
+            const int b0 = (int)S.a.s.base[bk[u]], b1 = (int)S.a.s.base[bk[u] + 1];
+            int r = b0;
+            for (int m = b0; m < b1; ++m) r += (S.a.s.key[m] < key[u]) ? 1 : 0;     // equal scores: ordered by ~row
+            rank[u] = r;
+        }
+    }
+
+    NMS_PHASE(2);
 
     // ---- 3. sorted arrays, bins, table inserts ----
     {
@@ -386,6 +389,7 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         }
     }
     __syncthreads();
+    NMS_PHASE(3);
     // prefix / suffix OR over the bins of 6 tables x nwp word pairs.  Eight lanes share a chain: each ORs its own run of
     // bins (independent loads), a 3-step shuffle scan over the eight run totals gives every lane its carry, and the runs
     // are stored back -- about 15 dependent steps where one lane per chain walked NBIN of them while three warps waited.
@@ -423,8 +427,10 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         }
     }
     __syncthreads();
+    NMS_PHASE(4);
 
     // ---- 4. candidate pairs (i < j) -> this warp's queue ----
+    const int wbase = tid & ~31;
     unsigned qcount = 0u;
     bool overflow = false;
     {
@@ -473,6 +479,8 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
     unsigned qtotal = 0u;
 #pragma unroll
     for (int wq = 0; wq < SMALL_WARPS; ++wq) qtotal += S.qn[wq];
+    NMS_PHASE(5);
+    NMS_COUNT(11, qtotal);
 
     // ---- 5. exact tests on the queued pairs, suppression matrix, resolve ----
     bool any_edges = false;
@@ -481,22 +489,28 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         for (int i = tid; i < n * (SMALL_W / 4); i += SMALL_THREADS) z[i] = make_uint4(0u, 0u, 0u, 0u);
         __syncthreads();
         bool found = false;
-#pragma unroll 1
-        for (int wq = 0; wq < SMALL_WARPS; ++wq) {
-            const unsigned cq = S.qn[wq];
-            for (unsigned q = tid; q < cq; q += SMALL_THREADS) {
-                const unsigned e = S.a.queue[wq][q];
-                const int j = e >> 8, i = e & 255;
-                const float4 bj = S.box[j], bi = S.box[i];
-                if (suppresses_pos<DIOU>(bj, box_area(bj), bi, box_area(bi), thr)) {
-                    atomicOr(&S.b.T[j][i >> 5], 1u << (i & 31));
-                    atomicOr(&S.dirty[j >> 5], 1u << (j & 31));
-                    found = true;
-                }
+        // the queues laid end to end, so that the ~110 pairs of a typical segment take one round of the whole CTA rather
+        // than one round of the first warp per queue
+        for (unsigned p = tid; p < qtotal; p += SMALL_THREADS) {
+            unsigned q = p;
+            int wq = 0;
+#pragma unroll
+            for (int k = 0; k < SMALL_WARPS - 1; ++k) {
+                const unsigned cq = S.qn[k];
+                if (wq == k && q >= cq) { q -= cq; wq = k + 1; }
+            }
+            const unsigned e = S.a.queue[wq][q];
+            const int j = e >> 8, i = e & 255;
+            const float4 bj = S.box[j], bi = S.box[i];
+            if (suppresses_pos<DIOU>(bj, box_area(bj), bi, box_area(bi), thr)) {
+                atomicOr(&S.b.T[j][i >> 5], 1u << (i & 31));
+                atomicOr(&S.dirty[j >> 5], 1u << (j & 31));
+                found = true;
             }
         }
         any_edges = __syncthreads_or(found) != 0;
     }
+    NMS_PHASE(6);
     if (tid < 32) {
         // lane w owns kept word w; only rows with a suppressor are visited, in score order (utils.py:67-84)
         unsigned keptw = 0u;
@@ -522,6 +536,10 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         if (lane == SMALL_W - 1) { S.pref[SMALL_W] = (unsigned)incl; kept_count[seg] = (unsigned)incl; }
     }
     __syncthreads();
+    NMS_PHASE(7);
+    NMS_COUNT(13, __popc(S.dirty[0]) + __popc(S.dirty[1]) + __popc(S.dirty[2]) + __popc(S.dirty[3]) + __popc(S.dirty[4]) +
+                  __popc(S.dirty[5]) + __popc(S.dirty[6]) + __popc(S.dirty[7]));
+    NMS_COUNT(14, S.pref[SMALL_W]);
 
     // ---- 6. finished rows: stage in shared memory (the tables / T are dead), store as one contiguous run ----
     const float fc = (float)(seg % C);                           // utils.py:183 class id stored as float
@@ -542,6 +560,7 @@ k_segment_nms_bins(uint4 *__restrict__ cand, const unsigned *__restrict__ seg_co
         const int tail = nf & ~3;
         if (tid < (nf & 3)) reinterpret_cast<float *>(rec)[tail + tid] = S.b.stage[tail + tid];
     }
+    NMS_PHASE(8);
 }
 
 // ---- big tier ---------------------------------------------------------------------------------------------
